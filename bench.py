@@ -22,6 +22,10 @@ beta2Simple, beta2Cryptic, SSE (what `process` does per sample, SpliSER_v0_1_8.p
             CUDA-event time vs the measured HBM peak.
   parity    the table e2e returned is compared with the oracle's C port of the reference on the SAME full workload
             (every column, floats bit for bit); that oracle run is also the cpu_baseline.
+
+  --dump-outputs DIR   after the timed steps, the site table the last timed step computed (rank 0's; --impl reference:
+            the oracle's table of its last step) goes to DIR/<column>.npy as float64, so that two builds run with the same
+            arguments (seeded, identical inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -175,6 +179,30 @@ def table_digest(t):
     return h.hexdigest()[:32]
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, t, limit=DUMP_BYTES):
+    """Every column of a result table (dict of arrays or SiteTable) -> out_dir/<column>.npy, float64 (exact for the integer
+    columns).  When the columns come to more than `limit` bytes, each keeps the same fixed share of its entries: a seeded
+    sample that depends only on the array's length, so columns of one length keep the same rows and two runs with the same
+    inputs keep the same entries."""
+    from oracle import c_oracle
+    d = t if isinstance(t, dict) else c_oracle.table_dict(t)
+    cols = {k: np.asarray(d[k]) for k in c_oracle.TABLE_FIELDS}
+    keep = min(1.0, (limit - 128 * len(cols)) / max(1, sum(8 * len(a) for a in cols.values())))     # 128 B: the header of a 1-D .npy
+    os.makedirs(out_dir, exist_ok=True)
+    rows = {}
+    for k, a in cols.items():
+        if keep < 1.0:
+            n = len(a)
+            if n not in rows:
+                rows[n] = np.sort(np.random.default_rng([DUMP_SEED, n]).choice(n, int(n * keep), replace=False))
+            a = a[rows[n]]
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float64))
+
+
 def synthetic_gff(w, path):
     """A gene every ~4 kb on both strands (seeded): only the Gene column of the TSV depends on it."""
     rng = np.random.default_rng(20260099)
@@ -253,9 +281,11 @@ def reference_arm(args, ncores):
     times = []
     for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        c_oracle.process(rec, len(w.chroms), junc, w.flags, threads=ncores)
+        res = c_oracle.process(rec, len(w.chroms), junc, w.flags, threads=ncores)
         if i >= args.warmup:
             times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     tot = float(sum(times))
     val = len(rec) * len(times) / tot
     if strong:
@@ -291,7 +321,11 @@ def main():
     ap.add_argument("--profile", action="store_true", help="resident passes only (for ncu): no e2e, no CPU baseline")
     ap.add_argument("--scaling", default="strong", choices=["weak", "strong"],
                     help="N > 1: strong (default) = ONE sample sharded over the GPUs by genomic tile; weak = one sample per GPU (replicas)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the site table of the last timed step to DIR/<column>.npy (float64, at most 64 MB, a seeded sample above that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -302,6 +336,8 @@ def main():
     if args.workload is None:
         args.workload = "c2" if max(world, args.gpus) == 1 else "c3"
     if args.workload == "c4":
+        if args.dump_outputs:
+            ap.error("--dump-outputs: the combine workload (c4) writes .combined.tsv files, not a site table")
         import bench_combine
         return bench_combine.run(args, rank, world, local, emit)
 
@@ -349,6 +385,8 @@ def main():
     ctx.resident_count(args.warmup)
     barrier()
     st = ctx.resident_count(args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.resident_fetch())
     barrier()
     ms_total = max_over_ranks(st["ms_total"])
     reads_rank = st["n_aligned"]

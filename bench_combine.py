@@ -101,7 +101,7 @@ def run(args, rank, world, local, emit):
     outc = os.path.join(out_dir, "combined")
     devices = list(range(n_dev))
     times = []
-    for it in range(1 + max(1, min(args.steps, 5))):                 # first run = warm-up (contexts, page cache)
+    for it in range(1 + args.steps):                                 # first run = warm-up (contexts, page cache)
         a = time.perf_counter()
         cli.combine(sf, outc, isStranded=True, strandedType="rf", devices=devices)
         if it:

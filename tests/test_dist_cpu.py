@@ -114,6 +114,56 @@ def test_bench_reference_arm_prints_the_contract_line(tmp_path):
     assert len(lines) == 1 and json.loads(lines[0])["n_gpus"] == 2
 
 
+def _bench_dump(tmp_path, tag, *args):
+    """Runs bench.py with --dump-outputs (workload cache of its own) -> {column: array}."""
+    import numpy as np
+    out = tmp_path / ("dump_" + tag)
+    env = dict(os.environ, SPLISER_BENCH_CACHE=str(tmp_path / ("cache_" + tag)))
+    res = subprocess.run([sys.executable, "bench.py", "--workload", "small", "--reads", "60000", "--steps", "2", "--warmup", "1",
+                          "--dump-outputs", str(out)] + list(args), capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-2000:]
+    return {p.name[:-4]: np.load(str(p)) for p in out.iterdir()}
+
+
+def test_bench_dump_outputs_of_the_reference_arm(tmp_path):
+    """`bench.py --dump-outputs DIR`: every column of the last step's table as float64 .npy, the same in two runs that each
+    generate the workload afresh, and equal to the oracle's table of that seeded workload."""
+    import numpy as np
+    import bench
+    from oracle import c_oracle
+    from spliser_b200 import synth
+    a = _bench_dump(tmp_path, "a", "--impl", "reference")
+    b = _bench_dump(tmp_path, "b", "--impl", "reference")
+    assert sorted(a) == sorted(c_oracle.TABLE_FIELDS) and sorted(b) == sorted(a)
+    w = synth.generate(bench.workload_config("small", 60000)[0])
+    want = c_oracle.process(w.records, len(w.chroms), w.junctions, w.flags)
+    assert len(want["pos"]) > 500 and want["sse"].any()
+    for k in c_oracle.TABLE_FIELDS:
+        assert a[k].dtype == np.float64 and np.array_equal(a[k], b[k], equal_nan=True), k
+        assert np.array_equal(a[k], want[k].astype(np.float64), equal_nan=True), k
+
+
+def test_bench_dump_outputs_sample_above_the_limit(tmp_path):
+    """A table larger than the limit keeps a seeded sample: under the limit on disk, the same rows in every column of one
+    length, the same entries from call to call."""
+    import numpy as np
+    import bench
+    from oracle import c_oracle
+    n, e = 20000, 30000
+    lens = {"partner_off": n + 1, "comp_off": n + 1, "partner_pos": e, "partner_cnt": e, "comp_pos": e // 2}
+    t = {k: np.arange(lens.get(k, n), dtype=np.int64) * (i + 1) for i, k in enumerate(c_oracle.TABLE_FIELDS)}
+    limit = 400_000
+    for tag in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / tag), t, limit=limit)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= limit
+    got = {k: np.load(str(tmp_path / "a" / (k + ".npy"))) for k in c_oracle.TABLE_FIELDS}
+    for i, k in enumerate(c_oracle.TABLE_FIELDS):
+        assert 0 < len(got[k]) < lens.get(k, n) and np.array_equal(got[k], np.load(str(tmp_path / "b" / (k + ".npy")))), k
+        rows = got[k] / (i + 1)                                      # the sampled row indices
+        ref = {"partner_off": "comp_off", "partner_pos": "partner_cnt"}.get(k, "chrom" if lens.get(k, n) == n else k)
+        assert np.array_equal(rows, got[ref] / (c_oracle.TABLE_FIELDS.index(ref) + 1)), k
+
+
 def test_host_topology_against_a_fake_sysfs(tmp_path):
     """The NUMA report bench.py attaches to every line (and the opt-in binding) reads sysfs only: a fake tree with two
     nodes, the GPU on node 1."""

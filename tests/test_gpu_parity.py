@@ -765,3 +765,16 @@ def test_junction_extraction_from_the_alignments(ctx, tmp_path):
     assert got == [(0, 119, 219, 4, "?"), (0, 310, 400, 1, "?"), (0, 709, 789, 1, "?"), (0, 797, 877, 1, "?")], got
     got = as_rows(ctx.extract_junctions_records(rec, 1, 1 | 2))          # --isStranded -s rf
     assert (0, 119, 219, 1, "+") in got and (0, 119, 219, 3, "-") in got, got       # flags 0, 99, 147 read '-' under rf, flag 16 '+' (S:374-406)
+
+
+def test_bench_dump_outputs_equal_the_reference_arms(tmp_path):
+    """`bench.py --dump-outputs DIR` on the CUDA arm writes the table of its last timed resident pass: column for column the
+    reference arm's (the C oracle's) for the same arguments."""
+    import numpy as np
+    from test_dist_cpu import _bench_dump
+    ours = _bench_dump(tmp_path, "ours", "--no-bam", "--no-variants", "--no-cpu-baseline")
+    ref = _bench_dump(tmp_path, "reference", "--impl", "reference")
+    assert sorted(ours) == sorted(ref)
+    for k in ref:
+        assert ours[k].dtype == np.float64 and np.array_equal(ours[k], ref[k], equal_nan=True), k
+    assert len(ref["pos"]) > 500 and ref["sse"].any()
