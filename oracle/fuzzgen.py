@@ -113,6 +113,130 @@ def _gen_read(rng, grid):
     return (max(1, pos), flag, cigar)
 
 
+LONG_FLAGS = FLAGS + (2048, 2064, 272)
+
+
+def gen_long_case(seed, *, dirty=False, max_long=14, max_short=20):
+    """Long-read shapes in the dict layout of gen_case: reads that walk 5-40 exons whose ends snap to a site grid (junction
+    ends land on hot anchors), small I / D every 5-60 bp inside the blocks, leading and trailing N or D, zero-length M / N / D,
+    back-to-back N N and N D, soft and hard clips, and the flags of gen_case plus 256 and 2048.  Junction rows often come on
+    both strands at the same positions (two sites per position), and some grid sites are hubs with six or more partners, so
+    one (junction, side) is a partner/competitor pair for five sites or more.  Short gen_case reads are mixed in."""
+    rng = random.Random(seed)
+    n_chrom = rng.choice([1, 1, 2])
+    chroms = ["C%d" % i for i in range(n_chrom)] if n_chrom > 1 else ["C"]
+    stranded = rng.random() < 0.6
+    stype = rng.choice(["fr", "rf"]) if stranded else None
+    cryptic = rng.random() < 0.5
+    bed, reads = [], []
+    strands = ["+", "-", "?"] if dirty else ["+", "-"]
+    for chrom in chroms:
+        nsite = rng.randint(10, 40)
+        grid, p = [], rng.randint(200, 400)
+        for _ in range(nsite):
+            grid.append(p)
+            p += rng.randint(12, 90)
+        rows = []
+        for _ in range(rng.randint(10, 60)):
+            a = rng.randrange(len(grid) - 1)
+            b = min(len(grid) - 1, a + rng.randint(1, 4))
+            rows.append((grid[a], grid[b]))
+        if rng.random() < 0.5:                                       # a hub: one site partnered with six or more others
+            h = rng.randrange(len(grid))
+            others = [g for g in grid if g != grid[h]]
+            for o in rng.sample(others, min(len(others), rng.randint(6, 9))):
+                rows.append((min(o, grid[h]), max(o, grid[h])))
+        for l, r in rows:
+            st = rng.choice(strands) if stranded else rng.choice(["+", "-", "?", "."])
+            bed.append(bed_line(chrom, l, r, rng.randint(1, 8), st))
+            if rng.random() < 0.3:                                   # the same junction on the other strand
+                bed.append(bed_line(chrom, l, r, rng.randint(1, 8), {"+": "-", "-": "+"}.get(st, "+")))
+        for _ in range(rng.randint(1, max_long)):
+            reads.append((chrom,) + _gen_long_read(rng, grid))
+        for _ in range(rng.randint(0, max_short)):
+            reads.append((chrom,) + _gen_read(rng, grid))
+    rng.shuffle(bed)
+    reads.sort(key=lambda x: (chroms.index(x[0]), x[1]))
+    return dict(seed=seed, chroms=chroms, bed="".join(bed), reads=reads, stranded=stranded, stype=stype, cryptic=cryptic)
+
+
+def _block_ops(rng, blen, ops, split):
+    """A mapped block of reference length blen (>= 1): M / = / X pieces of 5-60 bp split by small I or D (or one piece)."""
+    if not split:
+        ops.append("%d%s" % (blen, rng.choice("MMMM=X")))
+        return
+    rem = blen
+    while rem > 0:
+        m = min(rem, rng.randint(5, 60))
+        ops.append("%d%s" % (m, rng.choice("MMMM=X")))
+        rem -= m
+        if rem > 1 and rng.random() < 0.4:
+            d = min(rng.randint(1, 3), rem - 1)
+            ops.append("%dD" % d)
+            rem -= d
+        elif rem > 0 and rng.random() < 0.4:
+            ops.append("%dI" % rng.randint(1, 4))
+        if rng.random() < 0.03:
+            ops.append("0%s" % rng.choice("MND"))
+
+
+def _gen_long_read(rng, grid):
+    """One read across 5-40 exons: a block ends on a grid site (its last base, 75 %), the N that follows ends on a grid site
+    (its last base, 85 %) so that the next block starts right after it."""
+    ops = []
+    if rng.random() < 0.1:
+        ops.append("%dH" % rng.randint(1, 20))
+    if rng.random() < 0.3:
+        ops.append("%dS" % rng.randint(1, 40))
+    start = rng.choice(grid) + rng.choice([1, 1, 1, 0, -5, -20])
+    cur = start
+    split = rng.random() < 0.7                                       # else unsplit blocks: often more than two N in five operators
+    if rng.random() < 0.25:                                          # leading N / D: nothing advanced before it
+        n = rng.choice([0, 1, 7, 30])
+        ops.append("%d%s" % (n, rng.choice("ND")))
+        cur += n
+    nblk = rng.randint(5, 40)
+    for b in range(nblk):
+        cands = [g for g in grid if g >= cur]
+        if cands and rng.random() < 0.75:
+            end = rng.choice(cands[:3])
+            blen = max(1, end - cur + 1)
+        else:
+            blen = rng.randint(1, 70)
+        _block_ops(rng, blen, ops, split)
+        cur += blen
+        if b == nblk - 1:
+            break
+        sep = rng.random()
+        cands = [g for g in grid if g > cur]
+        if sep < 0.7 and cands:
+            r = rng.choice(cands[:4]) if rng.random() < 0.85 else cur + rng.randint(0, 40)
+            n = r - cur + 1
+            ops.append("%dN" % n)
+            cur += n
+            if rng.random() < 0.1:                                   # back-to-back N N / N D
+                e = rng.randint(0, 25)
+                ops.append("%d%s" % (e, rng.choice("ND")))
+                cur += e
+        elif sep < 0.78:
+            ops.append("0N")                                         # zero-length N: both ends on one position
+        elif sep < 0.88:
+            d = rng.randint(1, 15)
+            ops.append("%dD" % d)
+            cur += d
+        else:
+            n = rng.randint(1, 15)
+            ops.append("%dN" % n)
+            cur += n
+    if rng.random() < 0.2:                                           # trailing N / D
+        ops.append("%d%s" % (rng.choice([0, 1, 9, 40]), rng.choice("ND")))
+    if rng.random() < 0.3:
+        ops.append("%dS" % rng.randint(1, 40))
+    if rng.random() < 0.1:
+        ops.append("%dH" % rng.randint(1, 20))
+    return (max(1, start), rng.choice(LONG_FLAGS), "".join(ops))
+
+
 def gen_combine_case(seed):
     """Two or three samples over one shared site universe; each sample sees a random subset of
     the junction lines, so the combined table has gaps that need a re-count (S:899-904)."""

@@ -136,22 +136,22 @@ struct ReadWalk {            // any read: every access walks the CIGAR again (lo
     uint32_t c0, nop;
     int32_t pos;
     uint32_t nj, nb, jrel;
-    // x-th operator of the wanted kind (N or mapped): start position, end position, "something advanced before it"
-    __device__ __forceinline__ void find(bool want_n, uint32_t x, int32_t& a, int32_t& b, bool& seen) const {
-        int32_t cur = pos; uint32_t cnt = 0; bool sn = false;
-        a = b = 0; seen = false;
+    // x-th operator of the wanted kind (N or mapped): start position, end position, "it starts at POS"
+    __device__ __forceinline__ void find(bool want_n, uint32_t x, int32_t& a, int32_t& b, bool& at_pos) const {
+        int32_t cur = pos; uint32_t cnt = 0;
+        a = b = 0; at_pos = false;
         for (uint32_t q = 0; q < nop; ++q) {
             const uint32_t w = cw(c0 + q), op = w & 15u;
             const int32_t len = (int32_t)(w >> 4);
             const bool isM = op == 0u || op == 7u || op == 8u, isN = op == 3u;
             if ((want_n && isN) || (!want_n && isM)) {
-                if (cnt == x) { a = cur; b = cur + len; seen = sn; return; }
+                if (cnt == x) { a = cur; b = cur + len; at_pos = cur == pos; return; }
                 ++cnt;
             }
-            if (isM || isN || op == 2u) { cur += len; sn = true; }
+            if (isM || isN || op == 2u) cur += len;
         }
     }
-    __device__ __forceinline__ uint32_t jl(uint32_t x) const { int32_t a, b; bool s; find(true, x, a, b, s); return (uint32_t)(a - 1) | (s ? 0u : 0x80000000u); }
+    __device__ __forceinline__ uint32_t jl(uint32_t x) const { int32_t a, b; bool s; find(true, x, a, b, s); return (uint32_t)(a - 1) | (s ? 0x80000000u : 0u); }
     __device__ __forceinline__ uint32_t jr(uint32_t x) const { int32_t a, b; bool s; find(true, x, a, b, s); return (uint32_t)(b - 1); }
     __device__ __forceinline__ int32_t bs(uint32_t x) const { int32_t a, b; bool s; find(false, x, a, b, s); return a; }
     __device__ __forceinline__ uint32_t be(uint32_t x) const { int32_t a, b; bool s; find(false, x, a, b, s); return (uint32_t)b; }
@@ -180,19 +180,18 @@ __device__ __forceinline__ void hot_item(const DevRecords& rec, const DevGraph& 
     ReadRegs rr;
     rr.nj = rr.nb = rr.jrel = 0;
     int32_t cur = pos;
-    bool seen = false;
     for (uint32_t q = 0; q < nop; ++q) {
         const uint32_t w = cw(c0 + q), op = w & 15u;
         const int32_t len = (int32_t)(w >> 4);
         if (op == 0u || op == 7u || op == 8u) {
             if (rr.nb < (uint32_t)FC_MAXB) { rr.bsv[rr.nb] = cur; rr.bev[rr.nb] = (uint32_t)(cur + len); }
-            ++rr.nb; cur += len; seen = true;
+            ++rr.nb; cur += len;
         } else if (op == 3u) {
             if (q == j) rr.jrel = rr.nj;
-            if (rr.nj < (uint32_t)FC_MAXJ) { rr.jlv[rr.nj] = (uint32_t)(cur - 1) | (seen ? 0u : 0x80000000u); rr.jrv[rr.nj] = (uint32_t)(cur + len - 1); }
-            ++rr.nj; cur += len; seen = true;
+            if (rr.nj < (uint32_t)FC_MAXJ) { rr.jlv[rr.nj] = (uint32_t)(cur - 1) | (cur == pos ? 0x80000000u : 0u); rr.jrv[rr.nj] = (uint32_t)(cur + len - 1); }
+            ++rr.nj; cur += len;
         } else if (op == 2u) {
-            cur += len; seen = true;
+            cur += len;
         }
     }
     if (rr.nj <= (uint32_t)FC_MAXJ && rr.nb <= (uint32_t)FC_MAXB) {

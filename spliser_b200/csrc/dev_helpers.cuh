@@ -173,7 +173,7 @@ __device__ __forceinline__ void agg_add(uint32_t* p, uint32_t w) {
 
 // The read makes compSplicing true for site t through its junction number rd.jrel, unless an earlier junction of the read
 // already did: classify the read at t (S:503-557, first match wins); every counter moves by w.  Rd: nj, nb, jrel, jl(x) (bit 31: the N is the read's
-// first advancing operator -> POS > l, S:435), jr(x), bs(x), be(x) (block start / end; callers may leave flag bits in bit 31).
+// N starts at POS -> l = POS - 1), jr(x), bs(x), be(x) (block start / end; callers may leave flag bits in bit 31).
 template <class Rd>
 __device__ __forceinline__ void k4_classify(const Rd& rd, const DevGraph& g, const DevCounters& cnt, int t, uint32_t k, bool combine,
                                             uint32_t w = 1u /* identical reads this one stands for */) {
@@ -187,7 +187,8 @@ __device__ __forceinline__ void k4_classify(const Rd& rd, const DevGraph& g, con
     for (uint32_t x = 0; x < rd.nj; ++x) {
         const uint32_t lraw = rd.jl(x);
         const int32_t ll = (int32_t)(lraw & POS_MASK), rr = (int32_t)(rd.jr(x) & POS_MASK);
-        if (ll == tp && !(lraw >> 31)) { alpha = true; partner_used = rr; }   // firstN: POS > t, read skipped (S:435)
+        if (ll == tp && (lraw >> 31)) return;                    // POS > t: the read is skipped (S:435), a zero-length N's r = l too
+        if (ll == tp) { alpha = true; partner_used = rr; }
         if (rr == tp) { alpha = true; partner_used = ll; }
         if (ll < tp && tp < rr) kstar = (int)x;
     }

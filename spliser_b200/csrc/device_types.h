@@ -77,7 +77,8 @@ struct DevRecords {
 // word of every element carries the read's strand class (0 = '+' / unstranded, 1 = '-'):
 //   blocks     (start, end | class<<31)            [start, end) of one M/=/X operator
 //   junctions  (l | firstN<<31, r | class<<31)     l = last base before the N, r = last base of the N;
-//                                                  firstN marks a read whose first advancing op is this N
+//                                                  firstN marks an N that starts at POS (l = POS - 1: nothing before it
+//                                                  moved the position, zero-length operators included)
 // Blocks of unspliced reads (stream A, sorted by start) come first, blocks of spliced reads (stream B,
 // contiguous per read) follow in the same arrays.
 struct DevSoA {

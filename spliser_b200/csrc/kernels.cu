@@ -228,7 +228,7 @@ k_expand_scatter(DevRecords rec, const Chunk* chunks, DevSoA soa, uint32_t mode)
             const uint32_t kbit = read_class(rec.flag[i], mode) << 31;
             if (spliced) { soa.sr_boff[run.s + ex.s] = im - soa.bB; soa.sr_joff[run.s + ex.s] = ij; }
             int32_t cur = rec.pos[i];
-            bool seen = false, last_n = false;
+            bool last_n = false;
             int32_t a0 = 0;
             uint32_t nD = 0, first_m = 1;
             const uint32_t ij_first = ij;
@@ -239,14 +239,14 @@ k_expand_scatter(DevRecords rec, const Chunk* chunks, DevSoA soa, uint32_t mode)
                 if (op == 0u || op == 7u || op == 8u) {
                     if (first_m) { a0 = cur; first_m = 0; }
                     soa.m_start[im] = cur; soa.m_endk[im] = (uint32_t)(cur + len) | kbit; ++im;
-                    cur += len; seen = true; last_n = false;
+                    cur += len; last_n = false;
                 } else if (op == 3u) {
-                    soa.jn_l[ij] = (uint32_t)(cur - 1) | (seen ? 0u : 0x80000000u);     // S:482; firstN flag (POS <= t filter, S:435)
+                    soa.jn_l[ij] = (uint32_t)(cur - 1) | (cur == rec.pos[i] ? 0x80000000u : 0u);    // S:482; the N starts at POS (POS <= t filter, S:435)
                     soa.jn_rk[ij] = (uint32_t)(cur + len - 1) | kbit;                   // S:483
                     ++ij;
-                    cur += len; seen = true; last_n = true;
+                    cur += len; last_n = true;
                 } else if (op == 2u) {
-                    cur += len; seen = true; ++nD;
+                    cur += len; ++nD;
                 }
             }
             if (spliced) {

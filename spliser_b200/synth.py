@@ -475,6 +475,112 @@ def generate(cfg: SynthConfig, cache_dir=None, workers=None) -> Workload:
     return Workload(cfg, chroms, [l for _, l in cfg.contigs], rec, j)
 
 
+def config_long_reads(n_records=12_000, seed=20260011) -> SynthConfig:
+    """Long-read RNA-seq (Iso-Seq / ONT shaped) for generate_long_reads: ~25 exons per gene, every gene with alternative sites,
+    skipped exons and extra isoforms (most junction ends have competitors), reads of 1-10 kb, 5 % unspliced pre-mRNA reads."""
+    return SynthConfig(name="long", seed=seed, contigs=(("L1", 1_500_000), ("L2", 1_000_000), ("L3", 1_000_000)), n_records=n_records,
+                       read_len=10_000, stranded=True, genes_per_mb=25.0, exon_median=220.0, intron_median=600.0, intron_min=70,
+                       intron_max=20_000, mean_exons=25.0, frac_alt_site=1.0, frac_exon_skip=1.0, extra_isoforms=3, frac_retained=0.05,
+                       frac_softclip=0.2, frac_odd_flag=0.03)
+
+
+LONG_MAX_OPS = 255          # operators per record: what CompactRecords can carry
+
+
+def _long_block(rng, ops, blen):
+    """One exon's stretch of a read: unsplit (so exons over FC_WALK bases stay one M) or split by small I / D every 10-120 bp."""
+    if rng.random() < 0.4 or len(ops) > LONG_MAX_OPS - 24:
+        ops.append((blen << 4) | OP_M)
+        return
+    rem = blen
+    while rem > 0:
+        m = min(rem, int(rng.integers(10, 121)))
+        if len(ops) > LONG_MAX_OPS - 24:
+            m = rem
+        ops.append((m << 4) | OP_M)
+        rem -= m
+        if rem > 2 and rng.random() < 0.5:
+            d = int(rng.integers(1, 3))
+            ops.append((d << 4) | OP_D)
+            rem -= d
+        elif rem > 0:
+            ops.append((int(rng.integers(1, 4)) << 4) | OP_I)
+
+
+def _long_reads_for_contig(rng, cfg, m, n_rec):
+    """-> pos, flag, per-record operator lists, junction (left, right) -> (count, strand) of one contig."""
+    t_off, ex_start, ex_len = m["t_off"], m["ex_start"], m["ex_len"]
+    t_len = np.add.reduceat(ex_len, t_off[:-1])
+    g_expr = rng.lognormal(0.0, 1.0, size=len(m["g_start"]))
+    w = g_expr[m["t_gene"]] * np.maximum(t_len - 999, 0)
+    cdf = np.cumsum(w / w.sum())
+    pos, flag, reads, junc = [], [], [], {}
+    for _ in range(n_rec):
+        ops = []
+        if rng.random() < cfg.frac_softclip:
+            ops.append((int(rng.integers(5, 60)) << 4) | OP_S)
+        if rng.random() < cfg.frac_retained:                   # unspliced pre-mRNA: one block of 4096 bp or more
+            g = int(rng.integers(0, len(m["g_start"])))
+            L = int(rng.integers(4096, cfg.read_len + 1))
+            p = int(m["g_start"][g]) + int(rng.integers(0, max(1, int(m["g_end"][g] - m["g_start"][g]) - L // 2)))
+            ops.append((L << 4) | OP_M)
+            strand = int(m["g_strand"][g])
+        else:
+            t = min(int(np.searchsorted(cdf, rng.random(), side="right")), len(t_len) - 1)
+            L = min(int(rng.integers(1000, cfg.read_len + 1)), int(t_len[t]))
+            x = int(rng.integers(0, int(t_len[t]) - L + 1))       # transcript coordinate of the first base
+            e, e1 = int(t_off[t]), int(t_off[t + 1])
+            while x >= ex_len[e]:
+                x -= int(ex_len[e]); e += 1
+            p = int(ex_start[e]) + x
+            cur, rem = p, L
+            while rem > 0 and e < e1 and len(ops) <= LONG_MAX_OPS - 3:
+                blen = min(rem, int(ex_start[e] + ex_len[e]) - cur)
+                _long_block(rng, ops, blen)
+                rem -= blen; cur += blen; e += 1
+                if rem > 0 and e < e1 and len(ops) <= LONG_MAX_OPS - 3:      # room for N, a block and a clip
+                    n = int(ex_start[e]) - cur
+                    ops.append((n << 4) | OP_N)
+                    key = (cur - 1, cur + n - 1)                 # last exon base, last intron base (S:482-483)
+                    junc[key] = (junc.get(key, (0, 0))[0] + 1, int(m["t_strand"][t]))
+                    cur += n
+            strand = int(m["t_strand"][t])
+        if rng.random() < cfg.frac_softclip:
+            ops.append((int(rng.integers(5, 60)) << 4) | OP_S)
+        f = 16 if strand else 0                                  # single-end, sense reads map like fr; 30 % antisense (cDNA)
+        if rng.random() < 0.3:
+            f ^= 16
+        if rng.random() < cfg.frac_odd_flag:
+            f |= int(rng.choice([256, 2048]))
+        pos.append(p); flag.append(f); reads.append(ops)
+    return pos, flag, reads, junc
+
+
+def generate_long_reads(cfg: SynthConfig) -> Workload:
+    """A long-read sample on the gene models of _gene_models: reads of 1-10 kb along transcripts (5-40 junctions, ~100-255
+    operators each), unspliced reads of 4096 bp and more, and the junction table of every N in the reads (score = reads,
+    strand = transcript's).  cfg.read_len is the longest read."""
+    rng = np.random.default_rng(cfg.seed)
+    lens = np.array([l for _, l in cfg.contigs], float)
+    n_per = np.floor(lens / lens.sum() * cfg.n_records).astype(np.int64)
+    n_per[0] += cfg.n_records - int(n_per.sum())
+    P, F, O, C, jc, jl, jr, js, jst, seg_off = [], [], [], [], [], [], [], [], [], [0]
+    for ci, (_, clen) in enumerate(cfg.contigs):
+        m = _gene_models(rng, cfg, int(clen))
+        pos, flag, reads, junc = _long_reads_for_contig(rng, cfg, m, int(n_per[ci]))
+        order = np.argsort(np.array(pos), kind="stable")
+        P.append(np.array(pos, np.int32)[order]); F.append(np.array(flag, np.uint16)[order])
+        O.extend(len(reads[i]) for i in order); C.extend(op for i in order for op in reads[i])
+        seg_off.append(seg_off[-1] + len(pos))
+        for (l, r), (cnt, st) in sorted(junc.items()):
+            jc.append(ci); jl.append(l); jr.append(r); js.append(cnt); jst.append(ord("-") if st else ord("+"))
+    cig_off = np.zeros(sum(len(p) for p in P) + 1, np.uint32)
+    np.cumsum(O, out=cig_off[1:])
+    rec = Records(np.concatenate(P), np.concatenate(F), cig_off, np.array(C, np.uint32), np.arange(len(cfg.contigs), dtype=np.int32),
+                  np.array(seg_off, np.int64))
+    return Workload(cfg, [c for c, _ in cfg.contigs], [l for _, l in cfg.contigs], rec, Junctions(jc, jl, jr, js, jst))
+
+
 def reads_as_tuples(w: Workload):
     """(chrom_name, pos, flag, cigar_string) per record -- for text-based consumers on small workloads."""
     rec = w.records
