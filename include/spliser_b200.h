@@ -210,7 +210,33 @@ const int32_t* spl_junctions_left(const spl_junctions* j);      /* j_left / j_ri
 const int32_t* spl_junctions_right(const spl_junctions* j);
 const int64_t* spl_junctions_score(const spl_junctions* j);
 const uint8_t* spl_junctions_strand(const spl_junctions* j);
+/* Anchor extents, what a BED12 of the table carries in chromStart / chromEnd: start = left - the longest flanking stretch in
+ * front of the junction among its supporting records, end = right + the longest one behind it (stretches as above: M/=/X/D
+ * since the previous N or the read start, up to the next N or the read end).  blockSizes = (left - start, end - right), so
+ * that spl_bed_parse gives back left = chromStart + blockSizes[0] and right = chromEnd - blockSizes[1] (S:275-276). */
+const int32_t* spl_junctions_start(const spl_junctions* j);
+const int32_t* spl_junctions_end(const spl_junctions* j);
 void spl_junctions_free(spl_junctions* j);
+
+/* `process` without a BED12 file (the regtools step and process in one call): ingest the BAM once (on the device, or the host
+ * reader as the fallback, as spl_process chooses), extract its junction table (min_anchor / min_intron / max_intron as
+ * above; strands from SPL_FLAG_STRANDED / SPL_FLAG_RF), keep the rows `process` would keep of a BED12 holding that table
+ * -- -c (S:269) and the -g window (S:279-288), the same filter code as spl_bed_parse -- and count those rows against the same
+ * device-resident records as spl_process_records would.  *rows_out is the table after the filters in the order it was
+ * counted (spl_result_first_line indexes it); free it with spl_junctions_free.  Writing *rows_out with
+ * spl_write_junctions_bed and running spl_process on that file gives the same result. */
+typedef struct spl_extract_opts {
+    int32_t min_anchor, min_intron, max_intron;   /* regtools -a / -m / -M (8 / 70 / 500000) */
+    const char* qchrom;                           /* -c: keep the rows of this chromosome name only; NULL = "All" */
+    int32_t use_gene_window;                      /* -g: keep rows with a site in [gene_left - window_max_intron, gene_right + window_max_intron] */
+    int64_t gene_left, gene_right, window_max_intron;
+} spl_extract_opts;
+int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names,
+                            const spl_extract_opts* opts, uint32_t flags, spl_junctions** rows_out, spl_result** out);
+
+/* Reference names of a BAM header in header order (host only, no GPU): written NUL-terminated back to back into
+ * names[0 .. cap) when *bytes (the space they need) <= cap; *n_ref and *bytes are always set. */
+int spl_bam_reference_names(const char* path, char* names, int64_t cap, int64_t* n_ref, int64_t* bytes, char* err, int err_len);
 
 /* ---- result accessors ---------------------------------------------------------------------- */
 /* Sites are in the reference's output order: chrom_index order, then the per-chromosome list
@@ -288,6 +314,9 @@ int spl_resident_fetch(spl_ctx* ctx, spl_result** out);
 #define SPL_STAT_MS_GRAPH_DEV 25   /* spl_resident_count: summed CUDA-event ms of the site table + graph build inside the timed passes */
 #define SPL_STAT_N_HOT_ITEMS  27   /* junction ends on hot sites queued for the exception kernel in the last pass (fused variant) */
 #define SPL_STAT_GRAPH_TIMED  26   /* spl_resident_count: 1 = every pass rebuilt the site table + graph (fused variant, clean regime) */
+#define SPL_STAT_MS_EXTRACT   28   /* junction extraction: CUDA-event ms of its kernels (anchor extents included)           */
+#define SPL_STAT_MS_EXTENTS   29   /* junction extraction: CUDA-event ms of the anchor-extent walk alone                    */
+#define SPL_STAT_N_JUNCTIONS  30   /* junction extraction: rows extracted (before the -c / -g filters of spl_process_bam_extract) */
 int spl_last_stats(const spl_ctx* ctx, double* stats_out);
 
 /* ---- host text layer (no GPU): Gene column, .SpliSER.tsv writer, combine merge driver ------------
@@ -365,6 +394,15 @@ int spl_gene_search(int64_t n_genes, const int32_t* g_left, const int32_t* g_rig
 /* outputBedFile (S:641-664).  strand_texts = the distinct BED column-6 texts, line_strand[j] = id of
  * junction row j's text (the Strand column prints the text of the row that created the site:
  * first_line); site_gene[i] indexes gene_names, < 0 (or site_gene == NULL) prints "NA". */
+/* The BED12 of a junction table in the layout `regtools junctions extract` writes (its documentation; byte parity with
+ * regtools is not pinned), one line per row in table order:
+ *   chrom  start  end  JUNC%08d  score  strand  start  end  255,0,0  2  a,b  0,end-start-b
+ * with a = left - start, b = end - right; names are numbered from 1; chrom_names[chrom[i]] names row i's chromosome; a strand
+ * byte 0 writes an empty column. */
+int spl_write_junctions_bed(const char* path, int64_t n, const int32_t* chrom, const int32_t* left, const int32_t* right,
+                            const int32_t* start, const int32_t* end, const int64_t* score, const uint8_t* strand,
+                            const spl_strtab* chrom_names, char* err, int err_len);
+
 int spl_write_process_tsv(const char* path, const spl_site_columns* table, const spl_strtab* chrom_names,
                           const spl_strtab* strand_texts, const int32_t* line_strand,
                           const spl_strtab* gene_names, const int32_t* site_gene, int cryptic,

@@ -6,6 +6,6 @@ SpliSER-compatible CLI and TSV writers.  Importing the package does not need a G
 Context does, and there is no CPU fallback.
 """
 from .api import (CompactRecords, Context, Junctions, PackedRecords, Records, SiteTable, SpliserError, mode_flags,  # noqa: F401
-                  FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED)
+                  FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names)
 
 __version__ = "0.1.0"

@@ -16,7 +16,7 @@ SPL_FLAG_COMBINE = 8
 SPL_NSTATS = 32
 STAT_NAMES = ("ms_total", "ms_beta1", "ms_spliced", "ms_final", "n_mblocks_a", "n_mblocks_b", "n_junc_ops",
               "n_spliced", "n_sites", "n_edges", "n_aligned", "launches", "ms_expand", "ms_decode",
-              "h2d_bytes", "d2h_bytes", "ms_graph", "ms_upload", "ms_count", "n_distinct_junc", "n_simple_junc", "n_complex_junc", "graph_on_device", "bam_on_device", "n_parts", "ms_graph_dev", "graph_timed", "n_hot_items", "r28", "r29", "r30", "r31")
+              "h2d_bytes", "d2h_bytes", "ms_graph", "ms_upload", "ms_count", "n_distinct_junc", "n_simple_junc", "n_complex_junc", "graph_on_device", "bam_on_device", "n_parts", "ms_graph_dev", "graph_timed", "n_hot_items", "ms_extract", "ms_extents", "n_junctions", "r31")
 
 c_i32p = C.POINTER(C.c_int32)
 c_i64p = C.POINTER(C.c_int64)
@@ -47,6 +47,11 @@ class CompactView(C.Structure):
 
 class StrTab(C.Structure):
     _fields_ = [("n", C.c_int64), ("blob", C.c_char_p), ("off", c_i64p)]
+
+
+class ExtractOpts(C.Structure):
+    _fields_ = [("min_anchor", C.c_int32), ("min_intron", C.c_int32), ("max_intron", C.c_int32), ("qchrom", C.c_char_p),
+                ("use_gene_window", C.c_int32), ("gene_left", C.c_int64), ("gene_right", C.c_int64), ("window_max_intron", C.c_int64)]
 
 
 class SiteColumns(C.Structure):
@@ -83,7 +88,14 @@ SIGNATURES = {
     "spl_junctions_right": (c_i32p, [C.c_void_p]),
     "spl_junctions_score": (c_i64p, [C.c_void_p]),
     "spl_junctions_strand": (c_u8p, [C.c_void_p]),
+    "spl_junctions_start": (c_i32p, [C.c_void_p]),
+    "spl_junctions_end": (c_i32p, [C.c_void_p]),
     "spl_junctions_free": (None, [C.c_void_p]),
+    "spl_process_bam_extract": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp, C.POINTER(ExtractOpts), C.c_uint32,
+                                          C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    "spl_bam_reference_names": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int64, c_i64p, c_i64p, C.c_char_p, C.c_int]),
+    "spl_write_junctions_bed": (C.c_int, [C.c_char_p, C.c_int64, c_i32p, c_i32p, c_i32p, c_i32p, c_i32p, c_i64p, c_u8p,
+                                          C.POINTER(StrTab), C.c_char_p, C.c_int]),
     "spl_recount": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp] + _GAPS + [C.c_uint32, c_i64p, c_i64p]),
     "spl_recount_records": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), C.c_int32] + _GAPS + [C.c_uint32, c_i64p, c_i64p]),
     "spl_build_site_table": (C.c_int, [C.c_int32] + _JUNC + [C.c_uint32, C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),

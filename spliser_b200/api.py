@@ -48,12 +48,16 @@ def _ptr(a, ty):
 
 @dataclass
 class Junctions:
-    """Junction table in BED-line order after the text filters (S:259-288)."""
+    """Junction table in BED-line order after the text filters (S:259-288).  start / end: the BED12 chromStart / chromEnd of
+    every row (left - its longest left anchor, right + its longest right anchor) when the table was extracted from the
+    alignments, else None."""
     chrom: np.ndarray
     left: np.ndarray
     right: np.ndarray
     score: np.ndarray
     strand: np.ndarray
+    start: np.ndarray = None
+    end: np.ndarray = None
 
     def __post_init__(self):
         self.chrom = np.ascontiguousarray(self.chrom, dtype=np.int32)
@@ -64,6 +68,13 @@ class Junctions:
         n = len(self.chrom)
         if not (len(self.left) == len(self.right) == len(self.score) == len(self.strand) == n):
             raise ValueError("junction arrays differ in length")
+        if (self.start is None) != (self.end is None):
+            raise ValueError("start and end come together")
+        if self.start is not None:
+            self.start = np.ascontiguousarray(self.start, dtype=np.int32)
+            self.end = np.ascontiguousarray(self.end, dtype=np.int32)
+            if not (len(self.start) == len(self.end) == n):
+                raise ValueError("junction arrays differ in length")
 
     def __len__(self):
         return len(self.chrom)
@@ -547,7 +558,8 @@ class Context:
             def arr(fn, dt):
                 return np.ctypeslib.as_array(fn(h), shape=(n,)).astype(dt, copy=True) if n else np.zeros(0, dt)
             return Junctions(arr(lib.spl_junctions_chrom, np.int32), arr(lib.spl_junctions_left, np.int32), arr(lib.spl_junctions_right, np.int32),
-                             arr(lib.spl_junctions_score, np.int64), arr(lib.spl_junctions_strand, np.uint8))
+                             arr(lib.spl_junctions_score, np.int64), arr(lib.spl_junctions_strand, np.uint8),
+                             arr(lib.spl_junctions_start, np.int32), arr(lib.spl_junctions_end, np.int32))
         finally:
             lib.spl_junctions_free(h)
 
@@ -566,6 +578,21 @@ class Context:
         rc = self._lib.spl_extract_junctions(self._h, str(bam_path).encode(), len(chrom_names), names, min_anchor, min_intron, max_intron, flags, C.byref(h))
         self._check(rc, "spl_extract_junctions")
         return self._take_junctions(h)
+
+    def process_bam_extract(self, bam_path, chrom_names, flags: int = 0, min_anchor=8, min_intron=70, max_intron=500000,
+                            qchrom="All", gene_bounds=None, window_max_intron=0):
+        """`process` without a BED12 file: the BAM is ingested once, its junction table extracted (as extract_junctions_bam),
+        filtered like a BED12 of it (-c qchrom, -g window gene_bounds = (leftPos, rightPos) widened by window_max_intron,
+        S:269, S:279-288) and counted against the same device-resident records.  Returns (Junctions after the filters, in the
+        order they were counted -- first_line indexes them; SiteTable)."""
+        names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
+        o = L.ExtractOpts(int(min_anchor), int(min_intron), int(max_intron), None if qchrom == "All" else str(qchrom).encode(),
+                          int(gene_bounds is not None), *(int(x) for x in (gene_bounds or (0, 0))), int(window_max_intron))
+        hj, hr = C.c_void_p(), C.c_void_p()
+        rc = self._lib.spl_process_bam_extract(self._h, str(bam_path).encode(), len(chrom_names), names, C.byref(o), flags,
+                                               C.byref(hj), C.byref(hr))
+        self._check(rc, "spl_process_bam_extract")
+        return self._take_junctions(hj), self._take(hr)
 
     # ---- combine re-count ----------------------------------------------------------------------
     @staticmethod
@@ -609,6 +636,23 @@ class Context:
         h = C.c_void_p()
         self._check(self._lib.spl_resident_fetch(self._h, C.byref(h)), "spl_resident_fetch")
         return self._take(h)
+
+
+def bam_reference_names(path):
+    """Reference names of a BAM header in header order (host only)."""
+    lib = L.load()
+    n, need = C.c_int64(), C.c_int64()
+    err = C.create_string_buffer(512)
+    cap = 1 << 16
+    while True:
+        buf = C.create_string_buffer(cap)
+        rc = lib.spl_bam_reference_names(str(path).encode(), buf, cap, C.byref(n), C.byref(need), err, 512)
+        if rc != 0:
+            raise IOError("spl_bam_reference_names(%s): %s" % (path, err.value.decode()))
+        if need.value <= cap:
+            break
+        cap = need.value
+    return [x.decode() for x in buf.raw[:need.value].split(b"\0")[:n.value]]
 
 
 def build_site_table(n_chrom: int, junctions: Junctions, flags: int) -> SiteTable:

@@ -1,4 +1,5 @@
-"""BED12 junction file -> junction table (the text half of findAlphaCounts, SpliSER_v0_1_8.py:255-288).
+"""BED12 junction file -> junction table (the text half of findAlphaCounts, SpliSER_v0_1_8.py:255-288), and the BED12 of a
+junction table extracted from the alignments (what `regtools junctions extract` writes).
 
 Text handling, not counting, so it sits on the host side of the counting ABI; the per-line work is native
 (spl_bed_parse in csrc/host_text.cpp): the 12-column test (S:259), the chromosome index in first-appearance order
@@ -91,3 +92,21 @@ def parse_bed12(lines, chrom_index=None, qchrom="All", qgene_bounds=None, max_in
     finally:
         lib.spl_bed_free(h)
     return chroms, junc, sstr
+
+
+def write_junctions_bed(path, chroms, junc: Junctions):
+    """The BED12 of an extracted junction table in regtools' layout (spl_write_junctions_bed): chromStart / chromEnd from the
+    anchor extents junc.start / junc.end, names JUNC00000001, ... in row order.  parse_bed12 of the file gives back
+    (chrom, left, right, score, strand).  Byte parity with regtools itself is not pinned."""
+    from .hosttext import StrTable
+    if junc.start is None:
+        raise ValueError("the junction table has no anchor extents (start / end)")
+    lib = L.load()
+    tab = StrTable(list(chroms))
+    err = C.create_string_buffer(256)
+    p32 = lambda a: a.ctypes.data_as(L.c_i32p)  # noqa: E731
+    rc = lib.spl_write_junctions_bed(str(path).encode(), len(junc), p32(junc.chrom), p32(junc.left), p32(junc.right), p32(junc.start),
+                                     p32(junc.end), junc.score.ctypes.data_as(L.c_i64p), junc.strand.ctypes.data_as(L.c_u8p), tab.ref(),
+                                     err, 256)
+    if rc != 0:
+        raise (ValueError if rc == -1 else IOError)(err.value.decode())

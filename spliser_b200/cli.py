@@ -5,6 +5,13 @@
                                        [--isStranded -s rf|fr] [--beta2Cryptic]
     python -m spliser_b200.cli combine -S samples.tsv -o out [-g gene] [--isStranded -s rf|fr] [--beta2Cryptic]
 
+Without regtools (not a reference command; regtools' option letters):
+    python -m spliser_b200.cli junctions -B x.bam -o x.bed [-a 8] [-m 70] [-M 500000] [--isStranded -s rf|fr]
+    python -m spliser_b200.cli processBam -B x.bam -o out [process's -A -t -c -g -m --isStranded -s --beta2Cryptic]
+                                          [--minAnchor 8] [--minIntron 70] [--maxIntron 500000]
+`junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
+`junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.
+
 What stays in Python is what the reference does in text: BED12 parsing and its filters (S:255-288), the
 annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) and the lock-step merge of
 `combine` (S:742-917).  The body of `process` (S:710-717) is one spl_process call; every checkBam call of
@@ -19,7 +26,7 @@ import timeit
 import numpy as np
 
 from . import api
-from .bed import parse_bed12
+from .bed import StrandColumn, parse_bed12, write_junctions_bed
 from .dist import samples_of
 from .genes import load_annotation
 from .hosttext import CombineMerge, write_process_tsv as _native_write_process_tsv
@@ -106,6 +113,64 @@ def process(inBAM, inBed, outputPath, qGene="All", qChrom="All", maxIntronSize=0
             ctx.close()
     print("Sites:\t\t\t" + str(len(table)))
     write_process_tsv(outputPath + ".SpliSER.tsv", chroms, table, sstr, annotation=annotation, is_stranded=isStranded,
+                      beta2_cryptic=isbeta2Cryptic)
+
+
+# ------------------------------------------------------------------------------------------------ without regtools
+def junctions(inBAM, outBed, minAnchor=8, minIntron=70, maxIntron=500000, isStranded=False, strandedType=None, ctx=None):
+    """The `regtools junctions extract -a -m -M` step on the GPU: the junction table of every header reference, written as
+    BED12 in regtools' layout (chromStart / chromEnd from the longest anchors).  Strands: '?' unstranded, else the strand
+    check_strand derives from the FLAG (S:374-406); regtools' XS-tag strands are not available."""
+    chroms = api.bam_reference_names(inBAM)
+    flags = api.mode_flags(isStranded, strandedType)
+    own = ctx is None
+    ctx = ctx or api.Context(0)
+    try:
+        junc = ctx.extract_junctions_bam(inBAM, chroms, flags, minAnchor, minIntron, maxIntron)
+    finally:
+        if own:
+            ctx.close()
+    print("Junctions:\t\t" + str(len(junc)))
+    write_junctions_bed(outBed, chroms, junc)
+
+
+def _strand_column(junc):
+    """Column 6 of the BED12 `junctions` writes for these rows, as parse_bed12 would return it."""
+    texts, lut = [], np.zeros(256, dtype=np.int32)
+    for b in dict.fromkeys(junc.strand.tolist()):            # distinct bytes in first-appearance order
+        lut[b] = len(texts)
+        texts.append(chr(b) if b else "")
+    return StrandColumn(texts, lut[junc.strand])
+
+
+def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, annotationFile=None, aType="gene", isStranded=False,
+               strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, ctx=None):
+    """`junctions` + `process -b` in one GPU call that ingests the BAM once (spl_process_bam_extract).  The chromosome list is
+    the annotation's names, then the header's references not among them in header order: the relative order `process` gets
+    from a BED12 written by `junctions`, so the .SpliSER.tsv is the same byte for byte."""
+    print("Processing")
+    print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
+    annotation = load_annotation(annotationFile, qGene) if annotationFile is not None else None
+    bounds = None
+    if qGene != "All":
+        q = annotation.query_gene if annotation is not None else None
+        if q is None:                           # S:283, as in process
+            raise AttributeError("'NoneType' object has no attribute 'getLeftPos'")
+        bounds = (q.left, q.right)
+    chroms = list(annotation.chrom_index) if annotation is not None else []
+    known = set(chroms)
+    chroms += [c for c in api.bam_reference_names(inBAM) if c not in known]
+    flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic)
+    own = ctx is None
+    ctx = ctx or api.Context(0)
+    try:
+        junc, table = ctx.process_bam_extract(inBAM, chroms, flags, minAnchor, minIntron, maxIntron, qchrom=qChrom, gene_bounds=bounds,
+                                              window_max_intron=int(maxIntronSize))
+    finally:
+        if own:
+            ctx.close()
+    print("Sites:\t\t\t" + str(len(table)))
+    write_process_tsv(outputPath + ".SpliSER.tsv", chroms, table, _strand_column(junc), annotation=annotation, is_stranded=isStranded,
                       beta2_cryptic=isbeta2Cryptic)
 
 
@@ -288,13 +353,35 @@ def main(argv=None):
     cs.add_argument("--beta2Cryptic", dest="isbeta2Cryptic", default=False, action="store_true")
     cs.add_argument("--gpus", dest="n_gpus", nargs="?", default=1, type=int,
                     help="re-count the samples on this many GPUs (sharded by sample; not a reference option)")
+    j = sub.add_parser("junctions", help="junction BED12 from the BAM alone (the regtools junctions extract step)")
+    j.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
+    j.add_argument("-o", "--output", dest="outBed", required=True)
+    j.add_argument("-a", "--minAnchor", dest="minAnchor", default=8, type=int)
+    j.add_argument("-m", "--minIntron", dest="minIntron", default=70, type=int)
+    j.add_argument("-M", "--maxIntron", dest="maxIntron", default=500000, type=int)
+    j.add_argument("--isStranded", dest="isStranded", default=False, action="store_true")
+    j.add_argument("-s", "--strandedType", dest="strandedType", nargs="?", type=str)
+    pb = sub.add_parser("processBam", help="process without a BED12: junctions extracted from the BAM in the same pass")
+    pb.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
+    pb.add_argument("-o", "--outputPath", dest="outputPath", required=True)
+    pb.add_argument("-A", "--annotationFile", dest="annotationFile", required=False)
+    pb.add_argument("-t", "--annotationType", dest="aType", nargs="?", default="gene", type=str)
+    pb.add_argument("-c", "--chromosome", dest="qChrom", nargs="?", default="All", type=str)
+    pb.add_argument("-g", "--gene", dest="qGene", nargs="?", default="All", type=str)
+    pb.add_argument("-m", "--maxIntronSize", dest="maxIntronSize", nargs="?", default=0, type=int)
+    pb.add_argument("--isStranded", dest="isStranded", default=False, action="store_true")
+    pb.add_argument("-s", "--strandedType", dest="strandedType", nargs="?", type=str)
+    pb.add_argument("--beta2Cryptic", dest="isbeta2Cryptic", default=False, action="store_true")
+    pb.add_argument("--minAnchor", dest="minAnchor", default=8, type=int)
+    pb.add_argument("--minIntron", dest="minIntron", default=70, type=int)
+    pb.add_argument("--maxIntron", dest="maxIntron", default=500000, type=int)
     kwargs = vars(parser.parse_args(argv))
     command = kwargs.pop("command")
     if command in ("combine", "combineShallow"):
         kwargs["devices"] = list(range(max(1, kwargs.pop("n_gpus") or 1)))
-    if command == "process" and kwargs.get("qGene") != "All" and (kwargs.get("annotationFile") is None or kwargs.get("maxIntronSize") is None):
+    if command in ("process", "processBam") and kwargs.get("qGene") != "All" and (kwargs.get("annotationFile") is None or kwargs.get("maxIntronSize") is None):
         parser.error("--gene requires --annotationFile and --maxIntronSize")                      # S:1350-1353
-    elif command in ("process", "combine", "combineShallow") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
+    elif command in ("process", "combine", "combineShallow", "junctions", "processBam") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
         parser.error("--isStranded requires parameter --strandedType/-s as fr or rf")            # S:1354-1355
     elif command == "process":
         process(**kwargs)
@@ -302,8 +389,12 @@ def main(argv=None):
         combine(**kwargs)
     elif command == "combineShallow":
         combineShallow(**kwargs)
+    elif command == "junctions":
+        junctions(**kwargs)
+    elif command == "processBam":
+        processBam(**kwargs)
     else:
-        parser.error("command must be process, combine or combineShallow (output is unchanged Python in the reference)")
+        parser.error("command must be process, combine, combineShallow, junctions or processBam (output is unchanged Python in the reference)")
     print("Total runtime (s): \t" + str(timeit.default_timer() - start))
 
 

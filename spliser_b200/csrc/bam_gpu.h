@@ -37,9 +37,11 @@ constexpr uint32_t BAMGPU_MAX_SEG = 1u << 16;
 enum : int { BAMGPU_OK = 0, BAMGPU_FALLBACK = 1, BAMGPU_ERROR = 2 };
 
 // Host: BGZF member table of a whole file image + BAM header (names -> caller chromosome indices).
-// first_record = offset of the first alignment record in the inflated stream.  Returns "" or an error.
+// first_record = offset of the first alignment record in the inflated stream; ref_names (may be NULL) receives the header's
+// reference names in header order.  Returns "" or an error.
 std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const char* const* chrom_names, std::vector<BgzfMember>& members,
-                     uint64_t& total_u, uint64_t& first_record, int32_t& n_ref, std::vector<int32_t>& refmap);
+                     uint64_t& total_u, uint64_t& first_record, int32_t& n_ref, std::vector<int32_t>& refmap,
+                     std::vector<std::string>* ref_names = nullptr);
 
 // Device: inflate + parse.  BAMGPU_FALLBACK (err says why) = use the host reader instead; nothing was counted yet.
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,

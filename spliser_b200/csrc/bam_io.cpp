@@ -241,8 +241,10 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
 
 // ---- scan for the device ingest path (bam_gpu.cu) -----------------------------------------------
 std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const char* const* chrom_names, std::vector<BgzfMember>& members,
-                     uint64_t& total_u, uint64_t& first_record, int32_t& n_ref, std::vector<int32_t>& refmap) {
+                     uint64_t& total_u, uint64_t& first_record, int32_t& n_ref, std::vector<int32_t>& refmap,
+                     std::vector<std::string>* ref_names) {
     members.clear();
+    if (ref_names) ref_names->clear();
     size_t off = 0;
     uint64_t utotal = 0;
     while (off + 18 <= fsz) {
@@ -303,6 +305,7 @@ std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const cha
         std::string nm((const char*)hb.data() + q + 4, (size_t)l_name - 1);
         auto it = names.find(nm);
         if (it != names.end()) refmap[(size_t)r] = it->second;
+        if (ref_names) ref_names->push_back(std::move(nm));
         q += 4 + (size_t)l_name + 4;
     }
     first_record = q;
@@ -502,6 +505,39 @@ int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_nam
 }
 
 const spl_records_view* spl_records_get(const spl_records* r) { return r ? &r->v : nullptr; }
+
+int spl_bam_reference_names(const char* path, char* names, int64_t cap, int64_t* n_ref, int64_t* bytes, char* err, int err_len) {
+    if (!path || !n_ref || !bytes || cap < 0 || (cap > 0 && !names)) return SPL_ERR_ARG;
+    auto fail = [&](const std::string& e) {
+        if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
+        return SPL_ERR_IO;
+    };
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) return fail(std::string("cannot open BAM file ") + path);
+    struct stat st;
+    if (fstat(fd, &st) != 0 || st.st_size < 28) { close(fd); return fail(std::string("BAM file too small: ") + path); }
+    const size_t fsz = (size_t)st.st_size;
+    const uint8_t* file = (const uint8_t*)mmap(nullptr, fsz, PROT_READ, MAP_PRIVATE, fd, 0);
+    close(fd);
+    if (file == MAP_FAILED) return fail(std::string("mmap failed for ") + path);
+    std::vector<spl::BgzfMember> members;
+    std::vector<int32_t> refmap;
+    std::vector<std::string> ref;
+    uint64_t total_u = 0, first_record = 0;
+    int32_t nr = 0;
+    const std::string e = spl::bam_scan(file, fsz, 0, nullptr, members, total_u, first_record, nr, refmap, &ref);
+    munmap((void*)file, fsz);
+    if (!e.empty()) return fail(e);
+    int64_t need = 0;
+    for (const auto& s : ref) need += (int64_t)s.size() + 1;
+    *n_ref = (int64_t)ref.size();
+    *bytes = need;
+    if (cap >= need) {
+        char* p = names;
+        for (const auto& s : ref) { memcpy(p, s.c_str(), s.size() + 1); p += s.size() + 1; }
+    }
+    return SPL_OK;
+}
 void spl_records_free(spl_records* r) { delete r; }
 
 }  // extern "C"

@@ -1235,14 +1235,27 @@ __device__ __forceinline__ int je_chrom_of(const JeSeg& sg, uint32_t r) {
     return sg.seg_chrom[lo];
 }
 
-// EMIT = false: count the supporting N operators of every record; true: write their keys at the scanned offsets
-template <bool EMIT>
+// Pass JE_COUNT: count the supporting N operators of every record and the largest l among them (sizes the position field of
+// the key); JE_EMIT: write their keys at the scanned offsets; JE_EXTENT: find each one's row in the sorted unique keys
+// (lower_bound; the table is small and stays in L2) and raise the row's longest left / right flanking stretch -- the anchor
+// extents a BED12 writes as chromStart = l - max_left, chromEnd = r + max_right.
+enum : int { JE_COUNT = 0, JE_EMIT = 1, JE_EXTENT = 2 };
+struct JeOut {
+    uint32_t* cnt;                  // [R] supporting N operators per record (JE_COUNT writes, JE_EMIT reads its scan)
+    uint32_t* max_l;                // JE_COUNT: atomicMax of l over the supporting N operators
+    uint64_t* keys;                 // JE_EMIT
+    const uint64_t* ukeys;          // JE_EXTENT: unique keys, ascending
+    uint32_t n_u;
+    uint32_t* ext_l;                // JE_EXTENT: [n_u] atomicMax of the left / right stretch
+    uint32_t* ext_r;
+};
+template <int PASS>
 __global__ void __launch_bounds__(256) k_je_walk(DevRecords rec, JeSeg sg, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron,
-                                                 int pb, uint32_t* __restrict__ cnt, uint64_t* __restrict__ keys) {
+                                                 int pb, JeOut o) {
     const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= rec.n_rec) return;
-    const int chrom = je_chrom_of(sg, r);
-    uint32_t n = 0, w = EMIT ? cnt[r] : 0u;
+    const bool live = r < rec.n_rec;                                    // every lane reaches the warp reduction of JE_COUNT
+    const int chrom = live ? je_chrom_of(sg, r) : -1;
+    uint32_t n = 0, w = (PASS == JE_EMIT && live) ? o.cnt[r] : 0u, top = 0;
     if (chrom >= 0) {
         const uint32_t c0 = rec.cig_off[r], c1 = rec.cig_off[r + 1];
         const uint32_t flag = rec.flag[r];
@@ -1263,7 +1276,17 @@ __global__ void __launch_bounds__(256) k_je_walk(DevRecords rec, JeSeg sg, uint3
             const int32_t len = (int32_t)(v >> 4);
             if (op == 3u) {
                 if (plen >= 0 && plen >= min_intron && plen <= max_intron && pleft >= min_anchor && left >= min_anchor) {
-                    if (EMIT) keys[w] = ((((uint64_t)(uint32_t)chrom << pb | (uint64_t)(uint32_t)pl) << 20 | (uint64_t)(uint32_t)plen) << 2) | strand;
+                    if (PASS == JE_COUNT) top = max(top, (uint32_t)pl);
+                    if (PASS != JE_COUNT) {
+                        const uint64_t key = ((((uint64_t)(uint32_t)chrom << pb | (uint64_t)(uint32_t)pl) << 20 | (uint64_t)(uint32_t)plen) << 2) | strand;
+                        if (PASS == JE_EMIT) o.keys[w] = key;
+                        if (PASS == JE_EXTENT) {
+                            uint32_t lo = 0, hi = o.n_u;                // first unique key >= key: the key is there
+                            while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (o.ukeys[mid] < key) lo = mid + 1; else hi = mid; }
+                            atomicMax(o.ext_l + lo, (uint32_t)pleft);
+                            atomicMax(o.ext_r + lo, (uint32_t)left);
+                        }
+                    }
                     ++w; ++n;
                 }
                 pl = cur - 1; plen = k < c1 ? len : -1; pleft = left; left = 0;
@@ -1273,7 +1296,11 @@ __global__ void __launch_bounds__(256) k_je_walk(DevRecords rec, JeSeg sg, uint3
             }
         }
     }
-    if (!EMIT) cnt[r] = n;
+    if (PASS == JE_COUNT) {
+        if (live) o.cnt[r] = n;
+        top = __reduce_max_sync(0xffffffffu, top);                      // one atomic per warp
+        if ((threadIdx.x & 31u) == 0 && top) atomicMax(o.max_l, top);
+    }
 }
 
 __global__ void k_je_heads(const uint64_t* __restrict__ k, uint32_t n, uint32_t* __restrict__ flag) {
@@ -1281,7 +1308,8 @@ __global__ void k_je_heads(const uint64_t* __restrict__ k, uint32_t n, uint32_t*
     if (e < n) flag[e] = (e == 0 || k[e] != k[e - 1]) ? 1u : 0u;
 }
 __global__ void k_je_out(const uint64_t* __restrict__ k, const uint32_t* __restrict__ ex, uint32_t n, int pb, int32_t* __restrict__ o_chrom,
-                         int32_t* __restrict__ o_left, int32_t* __restrict__ o_right, uint8_t* __restrict__ o_strand, unsigned long long* __restrict__ o_score) {
+                         int32_t* __restrict__ o_left, int32_t* __restrict__ o_right, uint8_t* __restrict__ o_strand, unsigned long long* __restrict__ o_score,
+                         uint64_t* __restrict__ o_key) {
     const uint32_t e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     const bool head = e == 0 || k[e] != k[e - 1];
@@ -1289,6 +1317,7 @@ __global__ void k_je_out(const uint64_t* __restrict__ k, const uint32_t* __restr
     atomicAdd(o_score + idx, 1ull);
     if (head) {
         const uint64_t key = k[e];
+        o_key[idx] = key;
         const uint32_t st = (uint32_t)(key & 3u);
         const int32_t plen = (int32_t)((key >> 2) & 0xfffffu);
         const int32_t l = (int32_t)((key >> 22) & ((1ull << pb) - 1ull));
@@ -1493,18 +1522,18 @@ bool graph_build_device(GraphBuildMem& m, const int32_t* j_chrom, const int32_t*
     return true;
 }
 
-// Junction table of the device-resident records, sorted by (chromosome, l, r, strand).  Synchronises the stream (sizes).
+// Junction table of the device-resident records, sorted by (chromosome, l, r, strand), with each row's anchor extents.
+// Synchronises the stream (sizes).
 bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int64_t* h_seg_off, const int32_t* h_seg_chrom, int32_t n_seg,
                              int32_t n_chrom, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron, void* stream,
                              std::vector<int32_t>& chrom, std::vector<int32_t>& left, std::vector<int32_t>& right, std::vector<int64_t>& score,
-                             std::vector<uint8_t>& strand, std::string& err) {
+                             std::vector<uint8_t>& strand, std::vector<int32_t>& start, std::vector<int32_t>& end, std::string& err) {
     cudaStream_t st = (cudaStream_t)stream;
-    chrom.clear(); left.clear(); right.clear(); score.clear(); strand.clear();
+    chrom.clear(); left.clear(); right.clear(); score.clear(); strand.clear(); start.clear(); end.clear();
     const uint32_t R = rec.n_rec;
     if (R == 0 || n_seg == 0) return true;
     if (max_intron >= (1 << 20)) { err = "junction extraction: max_intron must be below 2^20"; return false; }
-    const int pb = 31, cb = bits_for_u64((uint64_t)(n_chrom > 1 ? n_chrom - 1 : 1));
-    if (cb + pb + 22 > 64) { err = "junction extraction: too many chromosomes for the packed key"; return false; }
+    const int cb = bits_for_u64((uint64_t)(n_chrom > 1 ? n_chrom - 1 : 1));
     Carve a;
     const size_t a_so = a.take<int64_t>((size_t)n_seg + 1), a_sc = a.take<int32_t>((size_t)n_seg + 1), a_cnt = a.take<uint32_t>((size_t)R + 4);
     const uint32_t lb_tiles0 = cdiv(R + 2u, LB_TILE) + 2;
@@ -1517,17 +1546,28 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     GB_CU(cudaMemsetAsync(ab + a_tot, 0, 64, st));
     const JeSeg sg{(const int64_t*)(ab + a_so), (const int32_t*)(ab + a_sc), n_seg};
     uint32_t* cnt = (uint32_t*)(ab + a_cnt);
-    uint32_t* d_tot = (uint32_t*)(ab + a_tot);
+    uint32_t* d_tot = (uint32_t*)(ab + a_tot);                          // [0] keys, [1] unique keys, [3] largest l, [5] sorter scratch
     uint32_t epoch = 0;
     unsigned long long* desc0 = (unsigned long long*)(ab + a_desc);
     const Scanner sc0{desc0, (uint32_t*)(desc0 + lb_tiles0 + 8), &epoch, st, (uint32_t*)(desc0 + lb_tiles0 + 16)};
-    { SPL_LAUNCH; k_je_walk<false><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, cnt, nullptr); }
+    JeOut jo{};
+    jo.cnt = cnt; jo.max_l = d_tot + 3;
+    for (auto& e : m.ev) if (!e) GB_CU(cudaEventCreate(&e));
+    m.ms_kernels = m.ms_extent = 0;
+    GB_CU(cudaEventRecord(m.ev[0], st));
+    { SPL_LAUNCH; k_je_walk<JE_COUNT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, 0, jo); }
     sc0.scan(cnt, R, nullptr, d_tot);
-    uint32_t h_n = 0;
-    GB_CU(cudaMemcpyAsync(&h_n, d_tot, 4, cudaMemcpyDeviceToHost, st));
+    GB_CU(cudaEventRecord(m.ev[1], st));
+    uint32_t h_tot[4] = {0, 0, 0, 0};
+    GB_CU(cudaMemcpyAsync(h_tot, d_tot, 16, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaStreamSynchronize(st));
-    const uint32_t n = h_n;
+    const uint32_t n = h_tot[0];
+    GB_CU(cudaEventElapsedTime(&m.ms_kernels, m.ev[0], m.ev[1]));
     if (n == 0) return true;
+    // the position field holds the largest l of the data (a real genome needs at most 28 bits), so headers with thousands of
+    // references still fit the 64-bit key
+    const int pb = bits_for_u64((uint64_t)std::max<uint32_t>(h_tot[3], 1u));
+    if (cb + pb + 22 > 64) { err = "junction extraction: too many chromosomes for the packed key"; return false; }
     const uint32_t max_tiles = cdiv(n, RS_TILE) + 1;
     const uint32_t lb_tiles = cdiv(std::max((uint32_t)RS_BINS * max_tiles, n + 2u), LB_TILE) + 2;
     Carve b;
@@ -1535,6 +1575,7 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     const size_t b_hist = b.take<uint32_t>((size_t)RS_BINS * (size_t)max_tiles + 2), b_desc = b.take<unsigned long long>(lb_tiles + SC_EXTRA);
     const size_t b_oc = b.take<int32_t>((size_t)n + 1), b_ol = b.take<int32_t>((size_t)n + 1), b_or = b.take<int32_t>((size_t)n + 1),
                  b_os = b.take<uint8_t>((size_t)n + 8), b_sc = b.take<unsigned long long>((size_t)n + 1);
+    const size_t b_uk = b.take<uint64_t>((size_t)n + 1), b_xl = b.take<uint32_t>((size_t)n + 1), b_xr = b.take<uint32_t>((size_t)n + 1);
     GB_CU(m.b.reserve(b.off + 256));
     char* bb = (char*)m.b.p;
     uint64_t* ka = (uint64_t*)(bb + b_ka); uint64_t* kb = (uint64_t*)(bb + b_kb);
@@ -1545,24 +1586,47 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     uint32_t epoch2 = 0;
     const Scanner sc{desc, (uint32_t*)(desc + lb_tiles + 8), &epoch2, st, (uint32_t*)(desc + lb_tiles + 16)};
     const Sorter sorter{(uint32_t*)(bb + b_hist), sc, d_tot + 5, st};
-    { SPL_LAUNCH; k_je_walk<true><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, cnt, ka); }
+    jo.keys = ka;
+    GB_CU(cudaEventRecord(m.ev[2], st));
+    { SPL_LAUNCH; k_je_walk<JE_EMIT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo); }
     uint64_t* sk = sorter.sort(ka, kb, n, 0, 22 + pb + cb);
     { SPL_LAUNCH; k_je_heads<<<cdiv(n, 256), 256, 0, st>>>(sk, n, flag); }
     sc.scan(flag, n, nullptr, d_tot + 1);
+    uint64_t* ukey = (uint64_t*)(bb + b_uk);
     { SPL_LAUNCH; k_je_out<<<cdiv(n, 256), 256, 0, st>>>(sk, flag, n, pb, (int32_t*)(bb + b_oc), (int32_t*)(bb + b_ol), (int32_t*)(bb + b_or),
-                                                       (uint8_t*)(bb + b_os), (unsigned long long*)(bb + b_sc)); }
+                                                       (uint8_t*)(bb + b_os), (unsigned long long*)(bb + b_sc), ukey); }
     GB_CU(cudaGetLastError());
+    GB_CU(cudaEventRecord(m.ev[3], st));
     uint32_t h_u = 0;
     GB_CU(cudaMemcpyAsync(&h_u, d_tot + 1, 4, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaStreamSynchronize(st));
     const size_t U = h_u;
-    chrom.resize(U); left.resize(U); right.resize(U); strand.resize(U); score.resize(U);
+    // anchor extents of the U rows
+    GB_CU(cudaMemsetAsync(bb + b_xl, 0, U * 4, st));
+    GB_CU(cudaMemsetAsync(bb + b_xr, 0, U * 4, st));
+    jo.ukeys = ukey; jo.n_u = (uint32_t)U; jo.ext_l = (uint32_t*)(bb + b_xl); jo.ext_r = (uint32_t*)(bb + b_xr);
+    GB_CU(cudaEventRecord(m.ev[4], st));
+    { SPL_LAUNCH; k_je_walk<JE_EXTENT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo); }
+    GB_CU(cudaGetLastError());
+    GB_CU(cudaEventRecord(m.ev[5], st));
+    chrom.resize(U); left.resize(U); right.resize(U); strand.resize(U); score.resize(U); start.resize(U); end.resize(U);
+    std::vector<uint32_t> xl(U), xr(U);
     GB_CU(cudaMemcpyAsync(chrom.data(), bb + b_oc, U * 4, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaMemcpyAsync(left.data(), bb + b_ol, U * 4, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaMemcpyAsync(right.data(), bb + b_or, U * 4, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaMemcpyAsync(strand.data(), bb + b_os, U, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaMemcpyAsync(score.data(), bb + b_sc, U * 8, cudaMemcpyDeviceToHost, st));
+    GB_CU(cudaMemcpyAsync(xl.data(), bb + b_xl, U * 4, cudaMemcpyDeviceToHost, st));
+    GB_CU(cudaMemcpyAsync(xr.data(), bb + b_xr, U * 4, cudaMemcpyDeviceToHost, st));
     GB_CU(cudaStreamSynchronize(st));
+    float ms_b = 0;
+    GB_CU(cudaEventElapsedTime(&ms_b, m.ev[2], m.ev[3]));
+    GB_CU(cudaEventElapsedTime(&m.ms_extent, m.ev[4], m.ev[5]));
+    m.ms_kernels += ms_b + m.ms_extent;
+    for (size_t i = 0; i < U; ++i) {
+        start[i] = left[i] - (int32_t)xl[i];
+        end[i] = right[i] + (int32_t)xr[i];
+    }
     return true;
 }
 

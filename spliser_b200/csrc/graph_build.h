@@ -58,12 +58,21 @@ bool graph_build_device(GraphBuildMem& m, const int32_t* j_chrom, const int32_t*
                         const int64_t* j_score, int64_t n_junc, int32_t n_chrom, int32_t max_pos, bool stranded, void* stream,
                         int phase /* 0: allocate + upload the junction table, 1: build + read sizes, 2: build only */, GraphDev& g, GraphCounts& counts, std::string& err);
 
-// junction extraction from device-resident records (graph_build.cu, shares its sort / scan kernels)
-struct JuncExtractMem { GbBuf a, b; };
+// junction extraction from device-resident records (graph_build.cu, shares its sort / scan kernels); start / end: the rows'
+// BED12 chromStart / chromEnd (l - longest left anchor, r + longest right anchor)
+struct JuncExtractMem {
+    GbBuf a, b;
+    cudaEvent_t ev[6] = {};          // bracket the three kernel stretches between the host reads of the sizes
+    float ms_kernels = 0, ms_extent = 0;   // CUDA-event ms of the last call: all extraction kernels / the extents walk alone
+    void release() {
+        a.release(); b.release();
+        for (auto& e : ev) if (e) { cudaEventDestroy(e); e = nullptr; }
+    }
+};
 struct DevRecords;
 bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int64_t* h_seg_off, const int32_t* h_seg_chrom, int32_t n_seg,
                              int32_t n_chrom, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron, void* stream,
                              std::vector<int32_t>& chrom, std::vector<int32_t>& left, std::vector<int32_t>& right, std::vector<int64_t>& score,
-                             std::vector<uint8_t>& strand, std::string& err);
+                             std::vector<uint8_t>& strand, std::vector<int32_t>& start, std::vector<int32_t>& end, std::string& err);
 
 }  // namespace spl

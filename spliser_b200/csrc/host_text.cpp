@@ -28,6 +28,7 @@
 #include <vector>
 
 #include "../../include/spliser_b200.h"
+#include "junction_filter.h"
 
 namespace {
 
@@ -972,17 +973,12 @@ bool bed_int(std::string_view s, long long* out) {
 }  // namespace
 
 namespace {
-struct BedFilter {
-    const char* qchrom;
-    bool window;
-    long long gene_left, gene_right, max_intron;
-};
+using BedFilter = spl::JunctionFilter;
 
 // Parses the lines of text[lo, hi) (hi at a line boundary) into `b` with ids local to `b`; returns SPL_OK or the error
 // of the first bad line (err_line = its 1-based number inside the piece).  n_lines = lines seen.
 int bed_parse_piece(const char* text, int64_t lo, int64_t hi, const BedFilter& f, spl_bed* b, int64_t* n_lines,
                     int64_t* err_line, const char** err_msg) {
-    const std::string_view q = f.qchrom ? std::string_view(f.qchrom) : std::string_view();
     // the line count is kept in a local and stored once per return path: the pieces' counters sit next to each other in
     // one cache line, so a store per line from every worker would bounce that line between the cores
     int64_t at = lo, line_no = 0;
@@ -1007,7 +1003,7 @@ int bed_parse_piece(const char* text, int64_t lo, int64_t hi, const BedFilter& f
         ++line_no;
         if (nc != 12) continue;                                          // S:259
         const int32_t ci = b->chroms.id(col[0]);                         // registered before the -c test (S:265-269)
-        if (f.qchrom && col[0] != q) continue;
+        if (!f.chrom_kept(col[0])) continue;
         std::string_view sizes = col[10];
         size_t comma = sizes.find(',');
         if (comma == std::string_view::npos) { *n_lines = line_no; *err_line = line_no; *err_msg = "blockSizes needs two values"; return SPL_ERR_ARG; }
@@ -1020,11 +1016,7 @@ int bed_parse_piece(const char* text, int64_t lo, int64_t hi, const BedFilter& f
             return SPL_ERR_ARG;
         }
         const long long left = start + a0, right = stop - a1;            // S:275-276
-        if (f.window) {                                                  // S:279-288
-            const bool lin = (left + f.max_intron >= f.gene_left) && (left <= f.gene_right);
-            const bool rin = (right - f.max_intron <= f.gene_right) && (right >= f.gene_left);
-            if (!(lin || rin)) continue;
-        }
+        if (!f.window_kept(left, right)) continue;
         if (left < INT32_MIN || left > INT32_MAX || right < INT32_MIN || right > INT32_MAX) {
             *n_lines = line_no; *err_line = line_no; *err_msg = "position outside 32 bits";
             return SPL_ERR_RANGE;
@@ -1128,6 +1120,46 @@ extern "C" const char* spl_bed_strand_text(const spl_bed* b, int64_t i, int64_t*
     if (!b || i < 0 || i >= (int64_t)b->strand_texts.names.size()) return nullptr;
     if (len) *len = (int64_t)b->strand_texts.names[(size_t)i].size();
     return b->strand_texts.names[(size_t)i].data();
+}
+
+// The BED12 that `regtools junctions extract` writes, one line per row in table order:
+//   chrom  start  end  JUNC%08d  score  strand  start  end  255,0,0  2  a,b  0,end-start-b
+// with a = left - start and b = end - right the longest anchors, so that spl_bed_parse gives back left = start + a and
+// right = end - b (S:275-276).  The layout follows regtools' documentation; byte parity with regtools is not pinned.
+extern "C" int spl_write_junctions_bed(const char* path, int64_t n, const int32_t* chrom, const int32_t* left, const int32_t* right,
+                                       const int32_t* start, const int32_t* end, const int64_t* score, const uint8_t* strand,
+                                       const spl_strtab* chrom_names, char* err, int err_len) {
+    if (!path || n < 0 || !chrom_names || (n > 0 && (!chrom || !left || !right || !start || !end || !score || !strand))) {
+        set_err(err, err_len, "spl_write_junctions_bed: null argument");
+        return SPL_ERR_ARG;
+    }
+    for (int64_t i = 0; i < n; ++i)
+        if (chrom[i] < 0 || chrom[i] >= chrom_names->n || start[i] > left[i] || end[i] < right[i]) {
+            set_err(err, err_len, "spl_write_junctions_bed: row %lld: chromosome out of range or anchor extents inside the junction", (long long)i);
+            return SPL_ERR_ARG;
+        }
+    FILE* f = fopen(path, "w");
+    if (!f) { set_err(err, err_len, "cannot open %s: %s", path, strerror(errno)); return SPL_ERR_IO; }
+    bool bad = false;
+    {
+        Out o(f);
+        char name[32];
+        for (int64_t i = 0; i < n; ++i) {
+            const long long s = start[i], e = end[i], a = left[i] - s, b = e - right[i];
+            o.put(tab_get(chrom_names, chrom[i])); o.ch('\t');
+            o.i64(s); o.ch('\t'); o.i64(e); o.ch('\t');
+            o.put(name, (size_t)snprintf(name, sizeof name, "JUNC%08lld", (long long)(i + 1))); o.ch('\t');
+            o.i64(score[i]); o.ch('\t');
+            if (strand[i]) o.ch((char)strand[i]);
+            o.ch('\t');
+            o.i64(s); o.ch('\t'); o.i64(e); o.put("\t255,0,0\t2\t");
+            o.i64(a); o.ch(','); o.i64(b); o.put("\t0,"); o.i64(e - s - b); o.ch('\n');
+        }
+        o.flush();
+        bad = o.bad;
+    }
+    if (fclose(f) != 0 || bad) { set_err(err, err_len, "write to %s failed", path); return SPL_ERR_IO; }
+    return SPL_OK;
 }
 
 // ========================================================================================================== annotation

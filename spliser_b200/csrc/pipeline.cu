@@ -25,6 +25,7 @@
 #include "bam_io.h"
 #include "device_types.h"
 #include "graph_build.h"
+#include "junction_filter.h"
 #include "site_graph.h"
 
 using namespace spl;
@@ -1461,7 +1462,7 @@ void spl_destroy(spl_ctx* ctx) {
         if (ctx->h_file) cudaFreeHost(ctx->h_file);
         ctx->bgm.comp.release(); ctx->bgm.unc.release(); ctx->bgm.tab.release(); ctx->bgm.rec.release(); ctx->bgm.list.release();
         ctx->gbm.fin.release(); ctx->gbm.fin2.release(); ctx->gbm.work.release(); ctx->gbm.work2.release();
-        ctx->jem.a.release(); ctx->jem.b.release();
+        ctx->jem.release();
         if (ctx->stream2) { cudaStreamSynchronize(ctx->stream2); cudaStreamDestroy(ctx->stream2); }
         if (ctx->ev_graph) cudaEventDestroy(ctx->ev_graph);
         cudaStreamDestroy(ctx->stream);
@@ -1679,6 +1680,7 @@ struct spl_junctions {
     std::vector<int32_t> chrom, left, right;
     std::vector<int64_t> score;
     std::vector<uint8_t> strand;
+    std::vector<int32_t> start, end;    // BED12 chromStart / chromEnd: left - longest left anchor, right + longest right anchor
 };
 
 namespace {
@@ -1697,9 +1699,52 @@ int extract_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, i
     if (!j) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
     std::string e;
     if (!junction_extract_device(ctx->jem, ctx->frec, rec->seg_off, rec->seg_chrom, rec->n_seg, n_chrom, flags & 3u, min_anchor, min_intron,
-                                 max_intron, ctx->stream, j->chrom, j->left, j->right, j->score, j->strand, e))
+                                 max_intron, ctx->stream, j->chrom, j->left, j->right, j->score, j->strand, j->start, j->end, e))
         return drain_on_error(ctx, ctx->fail(SPL_ERR_CUDA, "%s", e.c_str()));
+    ctx->stats[SPL_STAT_MS_EXTRACT] = ctx->jem.ms_kernels;
+    ctx->stats[SPL_STAT_MS_EXTENTS] = ctx->jem.ms_extent;
+    ctx->stats[SPL_STAT_N_JUNCTIONS] = (double)j->chrom.size();
     *out = j.release();
+    return SPL_OK;
+}
+
+// spl_process_bam_extract after the ingest: junction table of the records, the -c / -g row filters, then the count over the
+// same records, which extract_common left on the device (ctx->frec) -- they cross PCIe at most once.
+int extract_and_count(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, const char* const* chrom_names, const spl_extract_opts* o,
+                      uint32_t flags, spl_junctions** rows_out, spl_result** out) {
+    spl_junctions* got = nullptr;
+    int rc = extract_common(ctx, rec, n_chrom, o->min_anchor, o->min_intron, o->max_intron, flags, &got);
+    if (rc) return rc;
+    std::unique_ptr<spl_junctions> all(got);
+    double keep[SPL_NSTATS];
+    memcpy(keep, ctx->stats, sizeof keep);
+    std::unique_ptr<spl_junctions> j(new (std::nothrow) spl_junctions());
+    if (!j) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
+    const JunctionFilter f{o->qchrom, o->use_gene_window != 0, o->gene_left, o->gene_right, o->window_max_intron};
+    for (size_t i = 0; i < all->chrom.size(); ++i) {
+        const int32_t c = all->chrom[i];
+        if (!f.chrom_kept(chrom_names[c]) || !f.window_kept(all->left[i], all->right[i])) continue;
+        j->chrom.push_back(c); j->left.push_back(all->left[i]); j->right.push_back(all->right[i]);
+        j->score.push_back(all->score[i]); j->strand.push_back(all->strand[i]);
+        j->start.push_back(all->start[i]); j->end.push_back(all->end[i]);
+    }
+    // the count reads the records where the extraction left them: device-parsed records are ctx->dev_rec already, records of
+    // the host reader are in the extraction's upload (ctx->d_frec)
+    const DevRecordArrays saved = ctx->dev_rec;
+    const bool saved_dev = ctx->rec_on_device;
+    ctx->dev_rec.pos = const_cast<int32_t*>(ctx->frec.pos); ctx->dev_rec.flag = const_cast<uint16_t*>(ctx->frec.flag);
+    ctx->dev_rec.cig_off = const_cast<uint32_t*>(ctx->frec.cig_off); ctx->dev_rec.cigar = const_cast<uint32_t*>(ctx->frec.cigar);
+    spl_records_view dv{};
+    dv.n_rec = rec->n_rec; dv.n_cigar = rec->n_cigar; dv.n_seg = rec->n_seg; dv.seg_chrom = rec->seg_chrom; dv.seg_off = rec->seg_off;
+    ctx->rec_on_device = true;
+    rc = spl_process_records(ctx, &dv, n_chrom, (int64_t)j->chrom.size(), j->chrom.data(), j->left.data(), j->right.data(),
+                             j->score.data(), j->strand.data(), flags, out);
+    ctx->rec_on_device = saved_dev;
+    ctx->dev_rec = saved;
+    if (rc) return rc;
+    ctx->stats[SPL_STAT_H2D_BYTES] += keep[SPL_STAT_H2D_BYTES];
+    for (int k : {SPL_STAT_MS_EXTRACT, SPL_STAT_MS_EXTENTS, SPL_STAT_N_JUNCTIONS}) ctx->stats[k] = keep[k];
+    *rows_out = j.release();
     return SPL_OK;
 }
 }  // namespace
@@ -1747,6 +1792,48 @@ const int32_t* spl_junctions_left(const spl_junctions* j) { return j->left.data(
 const int32_t* spl_junctions_right(const spl_junctions* j) { return j->right.data(); }
 const int64_t* spl_junctions_score(const spl_junctions* j) { return j->score.data(); }
 const uint8_t* spl_junctions_strand(const spl_junctions* j) { return j->strand.data(); }
+const int32_t* spl_junctions_start(const spl_junctions* j) { return j->start.data(); }
+const int32_t* spl_junctions_end(const spl_junctions* j) { return j->end.data(); }
+
+int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names, const spl_extract_opts* opts,
+                            uint32_t flags, spl_junctions** rows_out, spl_result** out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out || !rows_out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
+    *out = nullptr; *rows_out = nullptr;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!bam_path || !opts) return ctx->fail(SPL_ERR_ARG, "bam_path or opts is NULL");
+    if (n_chrom < 0 || (n_chrom > 0 && !chrom_names)) return ctx->fail(SPL_ERR_ARG, "chrom_names is NULL");
+    for (int32_t c = 0; c < n_chrom; ++c) if (!chrom_names[c]) return ctx->fail(SPL_ERR_ARG, "chromosome name %d is NULL", c);
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    {   // ingest exactly as spl_process chooses: BGZF inflate + record parse on the device, the host reader as the fallback
+        BamGpuCounts cnt;
+        spl_records_view dv{};
+        bool fallback = false;
+        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback);
+        if (rc) return rc;
+        if (!fallback) {
+            const double t1 = now_ms();
+            ctx->rec_on_device = true;
+            rc = extract_and_count(ctx, &dv, n_chrom, chrom_names, opts, flags, rows_out, out);
+            ctx->rec_on_device = false;
+            ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+            ctx->stats[SPL_STAT_H2D_BYTES] += cnt.h2d_bytes;
+            ctx->stats[SPL_STAT_BAM_DEVICE] = 1.0;
+            ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+            return rc;
+        }
+    }
+    BamRecords recs;
+    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs);
+    if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
+    const double t1 = now_ms();
+    spl_records_view v = recs.view();
+    const int rc = extract_and_count(ctx, &v, n_chrom, chrom_names, opts, flags, rows_out, out);
+    ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
+}
 void spl_junctions_free(spl_junctions* j) { delete j; }
 
 int spl_recount_records(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int64_t n_sites, const int32_t* s_chrom,
