@@ -52,6 +52,19 @@ typedef enum spl_status {
 #define SPL_FLAG_RF       2u   /* -s rf (else fr); only read when STRANDED */
 #define SPL_FLAG_CRYPTIC  4u   /* --beta2Cryptic: SSE includes beta2Cryptic_weighted (S:633-635) */
 #define SPL_FLAG_COMBINE  8u   /* checkBam runs under `combine`: flanking reads add beta2Simple (S:531-532) */
+/* Junction extraction only (spl_extract_junctions, spl_extract_junctions_records_xs, spl_process_bam_extract): the table's
+ * strands come from the aligner's XS tag, as `regtools junctions extract` takes them for unstranded libraries; STRANDED / RF
+ * then do not touch the table (spl_process_bam_extract still counts with them).  The rule, one strand per record:
+ *   - walk the aux fields in order from the end of QUAL to the end of the record, sizing each by its type: A c C 1 byte,
+ *     s S 2, i I f 4, Z H up to and including the NUL, B a subtype byte, a u32 count and count x the subtype's size
+ *     (1 for c C, 2 for s S, 4 otherwise);
+ *   - the FIRST field tagged exactly XS decides: XS:A:+ gives '+', XS:A:- gives '-', any other type or character '?'
+ *     (later XS fields are ignored, as htslib's bam_aux_get does);
+ *   - '?' also when there is no XS field, or when an unknown type byte or a field running past the end of the record (a Z
+ *     without its NUL does) comes before it.  A malformed aux block is not an error.
+ * Every junction a record supports takes that record's strand.  Deviation: regtools writes other XS:A characters (such as
+ * '.') through unchanged; here they are '?'. */
+#define SPL_FLAG_XS_STRAND 16u
 
 /* ---- context ------------------------------------------------------------------------------- */
 /* device_ids: CUDA ordinals this context drives (one process per GPU: pass exactly one).
@@ -197,13 +210,18 @@ int spl_build_site_table(int32_t n_chrom,
  * when min_intron <= length(N) <= max_intron and the aligned stretches on both sides of the N (M/=/X/D operators up to the
  * neighbouring N or the end of the read) are at least min_anchor long; regtools' defaults are 8 / 70 / 500000.  regtools is
  * not part of the reference tree: these rules are restated from its documentation (parity unpinned; the tests pin the
- * kernel to synthetic samples whose generator knows the table).  Strand: with SPL_FLAG_STRANDED the strand check_strand
- * derives from the FLAG ('+' / '-'), else '?'.  Rows are sorted by (chromosome, l, r, strand). */
+ * kernel to synthetic samples whose generator knows the table).  Strand: with SPL_FLAG_XS_STRAND the record's XS tag (rule
+ * above), else with SPL_FLAG_STRANDED the strand check_strand derives from the FLAG ('+' / '-'), else '?'.  Rows are sorted by
+ * (chromosome, l, r, strand) with '?' < '+' < '-'.  spl_extract_junctions_records has no tags to read: SPL_FLAG_XS_STRAND is
+ * SPL_ERR_ARG there; spl_extract_junctions_records_xs takes the strands from xs[n_rec] ('+', '-' or '?' per record, e.g.
+ * spl_records_xs) when the flag is set. */
 typedef struct spl_junctions spl_junctions;
 int spl_extract_junctions(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names,
                           int32_t min_anchor, int32_t min_intron, int32_t max_intron, uint32_t flags, spl_junctions** out);
 int spl_extract_junctions_records(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom,
                                   int32_t min_anchor, int32_t min_intron, int32_t max_intron, uint32_t flags, spl_junctions** out);
+int spl_extract_junctions_records_xs(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom,
+                                     int32_t min_anchor, int32_t min_intron, int32_t max_intron, uint32_t flags, spl_junctions** out);
 int64_t        spl_junctions_n(const spl_junctions* j);
 const int32_t* spl_junctions_chrom(const spl_junctions* j);
 const int32_t* spl_junctions_left(const spl_junctions* j);      /* j_left / j_right / j_score / j_strand of spl_process */
@@ -220,7 +238,7 @@ void spl_junctions_free(spl_junctions* j);
 
 /* `process` without a BED12 file (the regtools step and process in one call): ingest the BAM once (on the device, or the host
  * reader as the fallback, as spl_process chooses), extract its junction table (min_anchor / min_intron / max_intron as
- * above; strands from SPL_FLAG_STRANDED / SPL_FLAG_RF), keep the rows `process` would keep of a BED12 holding that table
+ * above; strands from SPL_FLAG_XS_STRAND, else SPL_FLAG_STRANDED / SPL_FLAG_RF), keep the rows `process` would keep of a BED12 holding that table
  * -- -c (S:269) and the -g window (S:279-288), the same filter code as spl_bed_parse -- and count those rows against the same
  * device-resident records as spl_process_records would.  *rows_out is the table after the filters in the order it was
  * counted (spl_result_first_line indexes it); free it with spl_junctions_free.  Writing *rows_out with
@@ -454,12 +472,20 @@ int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names,
  * slowly): a sequencer-shaped file -- members of mostly literals, about 10 x the inflated bytes -- for the ingest benchmark. */
 int spl_write_bam_seq(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                       const spl_records_view* rec, int n_threads);
+/* spl_write_bam (with_seq = 0) or spl_write_bam_seq (with_seq != 0) with aux fields: record i (record order of the view) ends
+ * with the raw bytes aux[aux_off[i] .. aux_off[i + 1]), written as given (aux_off has n_rec + 1 entries). */
+int spl_write_bam_aux(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
+                      const spl_records_view* rec, const int64_t* aux_off, const uint8_t* aux, int with_seq, int n_threads);
 /* Decodes a BAM into library-owned record arrays (host only; no GPU needed).  chrom_names maps
  * BAM reference names to caller chromosome indices; records on other references are dropped. */
 typedef struct spl_records spl_records;
 int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
                  spl_records** out, char* err, int err_len);
+/* The same, and the strand of every kept record from its XS tag (SPL_FLAG_XS_STRAND's rule): spl_records_xs. */
+int spl_read_bam_xs(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
+                    spl_records** out, char* err, int err_len);
 const spl_records_view* spl_records_get(const spl_records* r);
+const uint8_t* spl_records_xs(const spl_records* r);      /* [n_rec] '+', '-' or '?'; NULL for a handle of spl_read_bam */
 void spl_records_free(spl_records* r);
 
 /* Test hook: the raw-DEFLATE decoder the device runs on every BGZF member (csrc/inflate.h), compiled for the host.

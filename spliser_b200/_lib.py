@@ -12,6 +12,7 @@ SPL_FLAG_STRANDED = 1
 SPL_FLAG_RF = 2
 SPL_FLAG_CRYPTIC = 4
 SPL_FLAG_COMBINE = 8
+SPL_FLAG_XS_STRAND = 16
 
 SPL_NSTATS = 32
 STAT_NAMES = ("ms_total", "ms_beta1", "ms_spliced", "ms_final", "n_mblocks_a", "n_mblocks_b", "n_junc_ops",
@@ -82,6 +83,8 @@ SIGNATURES = {
     "spl_process_compact": (C.c_int, [C.c_void_p, C.POINTER(CompactView), C.c_int32] + _JUNC + [C.c_uint32, C.POINTER(C.c_void_p)]),
     "spl_extract_junctions": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(C.c_void_p)]),
     "spl_extract_junctions_records": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(C.c_void_p)]),
+    "spl_extract_junctions_records_xs": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), c_u8p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                                   C.c_uint32, C.POINTER(C.c_void_p)]),
     "spl_junctions_n": (C.c_int64, [C.c_void_p]),
     "spl_junctions_chrom": (c_i32p, [C.c_void_p]),
     "spl_junctions_left": (c_i32p, [C.c_void_p]),
@@ -121,8 +124,11 @@ SIGNATURES = {
     "spl_resident_fetch": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "spl_write_bam": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), C.c_int]),
     "spl_write_bam_seq": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), C.c_int]),
+    "spl_write_bam_aux": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), c_i64p, c_u8p, C.c_int, C.c_int]),
     "spl_read_bam": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),
+    "spl_read_bam_xs": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),
     "spl_records_get": (C.POINTER(RecordsView), [C.c_void_p]),
+    "spl_records_xs": (c_u8p, [C.c_void_p]),
     "spl_records_free": (None, [C.c_void_p]),
     "spl_debug_inflate": (C.c_int, [c_u8p, C.c_uint32, c_u8p, C.c_uint32, c_u32p]),
     "spl_bed_parse": (C.c_int, [C.c_char_p, C.c_int64, C.POINTER(StrTab), C.c_char_p, C.c_int, C.c_int64, C.c_int64, C.c_int64,

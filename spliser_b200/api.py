@@ -16,6 +16,7 @@ import numpy as np
 from . import _lib as L
 
 FLAG_STRANDED, FLAG_RF, FLAG_CRYPTIC, FLAG_COMBINE = 1, 2, 4, 8
+FLAG_XS_STRAND = 16          # junction extraction: strands from the XS tag (include/spliser_b200.h states the rule)
 
 _CIG = re.compile(r"(\d+)([MIDNSHP=X])")
 _OPS = {c: i for i, c in enumerate("MIDNSHP=X")}
@@ -85,9 +86,10 @@ class Junctions:
 
 
 class Records:
-    """Alignment records as flat arrays grouped in chromosome segments (spl_records_view)."""
+    """Alignment records as flat arrays grouped in chromosome segments (spl_records_view).  xs: optional strand of every record
+    from its XS tag (uint8 '+', '-' or '?'), what extraction with FLAG_XS_STRAND reads."""
 
-    def __init__(self, pos, flag, cig_off, cigar, seg_chrom, seg_off, _owner=None):
+    def __init__(self, pos, flag, cig_off, cigar, seg_chrom, seg_off, _owner=None, xs=None):
         self.pos = np.ascontiguousarray(pos, dtype=np.int32)
         self.flag = np.ascontiguousarray(flag, dtype=np.uint16)
         self.cig_off = np.ascontiguousarray(cig_off, dtype=np.uint32)
@@ -95,8 +97,11 @@ class Records:
         self.seg_chrom = np.ascontiguousarray(seg_chrom, dtype=np.int32)
         self.seg_off = np.ascontiguousarray(seg_off, dtype=np.int64)
         self._owner = _owner
+        self.xs = None if xs is None else np.ascontiguousarray(xs, dtype=np.uint8)
         if len(self.cig_off) != len(self.pos) + 1 or len(self.flag) != len(self.pos):
             raise ValueError("record arrays differ in length")
+        if self.xs is not None and len(self.xs) != len(self.pos):
+            raise ValueError("xs must have one entry per record")
         if len(self.seg_off) != len(self.seg_chrom) + 1:
             raise ValueError("seg_off must have n_seg+1 entries")
 
@@ -118,12 +123,16 @@ class Records:
 
     @classmethod
     def from_reads(cls, chrom_names, reads):
-        """reads: iterable of (chrom_name, pos1, flag, cigar_string) in file order.  Reads on unknown
-        chromosomes become segments with chromosome -1 (skipped by the library)."""
+        """reads: iterable of (chrom_name, pos1, flag, cigar_string[, xs]) in file order, xs = '+', '-' or '?' (the strand of
+        the read's XS tag; given for every read or for none).  Reads on unknown chromosomes become segments with chromosome -1
+        (skipped by the library)."""
         index = {c: i for i, c in enumerate(chrom_names)}
-        pos, flag, off, cig, seg_chrom, seg_off = [], [], [0], [], [], []
+        pos, flag, off, cig, seg_chrom, seg_off, xs = [], [], [0], [], [], [], []
         cur = None
-        for chrom, p, f, cg in reads:
+        for r in reads:
+            chrom, p, f, cg = r[:4]
+            if len(r) > 4:
+                xs.append(ord(r[4]))
             ci = index.get(chrom, -1)
             if ci != cur:
                 seg_chrom.append(ci)
@@ -136,15 +145,18 @@ class Records:
         seg_off.append(len(pos))
         if not seg_chrom:
             seg_off = [0]
-        return cls(pos, flag, off, cig, seg_chrom, seg_off)
+        if xs and len(xs) != len(pos):
+            raise ValueError("an xs strand for every read or for none")
+        return cls(pos, flag, off, cig, seg_chrom, seg_off, xs=xs if xs else None)
 
     @classmethod
-    def from_bam(cls, path, chrom_names, threads=0):
+    def from_bam(cls, path, chrom_names, threads=0, xs=False):
+        """xs: also read every record's strand from its XS tag (Records.xs)."""
         lib = L.load()
         names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
         h = C.c_void_p()
         err = C.create_string_buffer(512)
-        rc = lib.spl_read_bam(str(path).encode(), len(chrom_names), names, threads, C.byref(h), err, 512)
+        rc = (lib.spl_read_bam_xs if xs else lib.spl_read_bam)(str(path).encode(), len(chrom_names), names, threads, C.byref(h), err, 512)
         if rc != 0:
             raise IOError("spl_read_bam(%s): %s" % (path, err.value.decode()))
         try:
@@ -156,21 +168,37 @@ class Records:
             out = cls(arr(v.pos, n, np.int32), arr(v.flag, n, np.uint16),
                       np.ctypeslib.as_array(v.cig_off, shape=(n + 1,)).astype(np.uint32, copy=True),
                       arr(v.cigar, nc, np.uint32), arr(v.seg_chrom, ns, np.int32),
-                      np.ctypeslib.as_array(v.seg_off, shape=(ns + 1,)).astype(np.int64, copy=True))
+                      np.ctypeslib.as_array(v.seg_off, shape=(ns + 1,)).astype(np.int64, copy=True),
+                      xs=arr(lib.spl_records_xs(h), n, np.uint8) if xs else None)
         finally:
             lib.spl_records_free(h)
         return out
 
-    def write_bam(self, path, ref_names, ref_len=None, threads=0, with_seq=False):
-        """with_seq: read names, SEQ and QUAL of the CIGAR's query length are written too (a sequencer-shaped file)."""
+    def write_bam(self, path, ref_names, ref_len=None, threads=0, with_seq=False, aux=None):
+        """with_seq: read names, SEQ and QUAL of the CIGAR's query length are written too (a sequencer-shaped file).
+        aux: raw aux bytes per record, a list of bytes (see encode_aux) or (offsets[n_rec + 1], uint8 blob)."""
         lib = L.load()
         names = (C.c_char_p * max(1, len(ref_names)))(*[c.encode() for c in ref_names])
         rl = None
         if ref_len is not None:
             rl = np.ascontiguousarray(ref_len, dtype=np.int32)
         v = self.view()
-        rc = (lib.spl_write_bam_seq if with_seq else lib.spl_write_bam)(str(path).encode(), len(ref_names), names,
-                                                                        _ptr(rl, L.c_i32p) if rl is not None else None, C.byref(v), threads)
+        rlp = _ptr(rl, L.c_i32p) if rl is not None else None
+        if aux is None:
+            rc = (lib.spl_write_bam_seq if with_seq else lib.spl_write_bam)(str(path).encode(), len(ref_names), names, rlp, C.byref(v), threads)
+        else:
+            if isinstance(aux, tuple):
+                off, blob = aux
+            else:
+                off = np.zeros(len(aux) + 1, np.int64)
+                off[1:] = np.cumsum([len(a) for a in aux])
+                blob = np.frombuffer(b"".join(aux), np.uint8)
+            off = np.ascontiguousarray(off, dtype=np.int64)
+            blob = np.ascontiguousarray(blob, dtype=np.uint8)
+            if len(off) != len(self) + 1 or (len(off) and (off[0] != 0 or off[-1] != len(blob) or np.any(np.diff(off) < 0))):
+                raise ValueError("aux offsets must run from 0 to len(blob), one record each")
+            rc = lib.spl_write_bam_aux(str(path).encode(), len(ref_names), names, rlp, C.byref(v), _ptr(off, L.c_i64p),
+                                       _ptr(blob, L.c_u8p) if len(blob) else C.cast(C.c_char_p(b""), L.c_u8p), int(with_seq), threads)
         if rc != 0:
             raise IOError("spl_write_bam(%s) failed with %d" % (path, rc))
 
@@ -565,10 +593,17 @@ class Context:
 
     def extract_junctions_records(self, records: Records, n_chrom: int, flags: int = 0, min_anchor=8, min_intron=70, max_intron=500000) -> Junctions:
         """Junction table (left, right, score, strand) from the alignments: what `regtools junctions extract -a 8 -m 70 -M 500000`
-        feeds the reference with.  flags: FLAG_STRANDED (| FLAG_RF) gives '+' / '-' strands, else '?'."""
+        feeds the reference with.  flags: FLAG_XS_STRAND takes the strands from records.xs, FLAG_STRANDED (| FLAG_RF) gives
+        '+' / '-' strands from the FLAG, else '?'."""
         v = records.view()
         h = C.c_void_p()
-        rc = self._lib.spl_extract_junctions_records(self._h, C.byref(v), n_chrom, min_anchor, min_intron, max_intron, flags, C.byref(h))
+        if flags & FLAG_XS_STRAND:
+            if records.xs is None:
+                raise ValueError("FLAG_XS_STRAND needs records.xs (Records.from_bam(..., xs=True) or from_reads with an xs column)")
+            rc = self._lib.spl_extract_junctions_records_xs(self._h, C.byref(v), _ptr(records.xs, L.c_u8p), n_chrom, min_anchor, min_intron,
+                                                            max_intron, flags, C.byref(h))
+        else:
+            rc = self._lib.spl_extract_junctions_records(self._h, C.byref(v), n_chrom, min_anchor, min_intron, max_intron, flags, C.byref(h))
         self._check(rc, "spl_extract_junctions_records")
         return self._take_junctions(h)
 

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libspliser_b200.so")
 SOURCES = ["kernels.cu", "count_fused.cu", "graph_build.cu", "bam_gpu.cu", "pipeline.cu", "site_graph.cpp", "bam_io.cpp", "host_text.cpp"]
-HEADERS = ["device_types.h", "dev_helpers.cuh", "graph_build.h", "bam_gpu.h", "inflate.h", "site_graph.h", "bam_io.h", "junction_filter.h", os.path.join("..", "..", "include", "spliser_b200.h")]
+HEADERS = ["device_types.h", "dev_helpers.cuh", "graph_build.h", "bam_gpu.h", "inflate.h", "site_graph.h", "bam_io.h", "bam_aux.h", "junction_filter.h", os.path.join("..", "..", "include", "spliser_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-Wall", "-shared"]
 

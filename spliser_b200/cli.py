@@ -6,11 +6,13 @@
     python -m spliser_b200.cli combine -S samples.tsv -o out [-g gene] [--isStranded -s rf|fr] [--beta2Cryptic]
 
 Without regtools (not a reference command; regtools' option letters):
-    python -m spliser_b200.cli junctions -B x.bam -o x.bed [-a 8] [-m 70] [-M 500000] [--isStranded -s rf|fr]
+    python -m spliser_b200.cli junctions -B x.bam -o x.bed [-a 8] [-m 70] [-M 500000] [--isStranded -s rf|fr | --strandFromXS]
     python -m spliser_b200.cli processBam -B x.bam -o out [process's -A -t -c -g -m --isStranded -s --beta2Cryptic]
-                                          [--minAnchor 8] [--minIntron 70] [--maxIntron 500000]
+                                          [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
 `junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
-`junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.
+`junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.  --strandFromXS
+takes the junction strands from the aligner's XS tag, as regtools does for unstranded libraries; processBam still counts
+with --isStranded -s.
 
 What stays in Python is what the reference does in text: BED12 parsing and its filters (S:255-288), the
 annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) and the lock-step merge of
@@ -117,12 +119,14 @@ def process(inBAM, inBed, outputPath, qGene="All", qChrom="All", maxIntronSize=0
 
 
 # ------------------------------------------------------------------------------------------------ without regtools
-def junctions(inBAM, outBed, minAnchor=8, minIntron=70, maxIntron=500000, isStranded=False, strandedType=None, ctx=None):
+def junctions(inBAM, outBed, minAnchor=8, minIntron=70, maxIntron=500000, isStranded=False, strandedType=None, strandFromXS=False,
+              ctx=None):
     """The `regtools junctions extract -a -m -M` step on the GPU: the junction table of every header reference, written as
-    BED12 in regtools' layout (chromStart / chromEnd from the longest anchors).  Strands: '?' unstranded, else the strand
-    check_strand derives from the FLAG (S:374-406); regtools' XS-tag strands are not available."""
+    BED12 in regtools' layout (chromStart / chromEnd from the longest anchors).  Strands: with strandFromXS the record's XS tag
+    ('?' without one; include/spliser_b200.h, SPL_FLAG_XS_STRAND), else '?' unstranded, else the strand check_strand derives
+    from the FLAG (S:374-406)."""
     chroms = api.bam_reference_names(inBAM)
-    flags = api.mode_flags(isStranded, strandedType)
+    flags = api.FLAG_XS_STRAND if strandFromXS else api.mode_flags(isStranded, strandedType)
     own = ctx is None
     ctx = ctx or api.Context(0)
     try:
@@ -144,10 +148,11 @@ def _strand_column(junc):
 
 
 def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, annotationFile=None, aType="gene", isStranded=False,
-               strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, ctx=None):
+               strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False, ctx=None):
     """`junctions` + `process -b` in one GPU call that ingests the BAM once (spl_process_bam_extract).  The chromosome list is
     the annotation's names, then the header's references not among them in header order: the relative order `process` gets
-    from a BED12 written by `junctions`, so the .SpliSER.tsv is the same byte for byte."""
+    from a BED12 written by `junctions`, so the .SpliSER.tsv is the same byte for byte.  strandFromXS: the table's strands come
+    from the XS tag (`junctions --strandFromXS`); the count still follows isStranded / strandedType."""
     print("Processing")
     print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
     annotation = load_annotation(annotationFile, qGene) if annotationFile is not None else None
@@ -160,7 +165,7 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
     chroms = list(annotation.chrom_index) if annotation is not None else []
     known = set(chroms)
     chroms += [c for c in api.bam_reference_names(inBAM) if c not in known]
-    flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic)
+    flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic) | (api.FLAG_XS_STRAND if strandFromXS else 0)
     own = ctx is None
     ctx = ctx or api.Context(0)
     try:
@@ -361,6 +366,8 @@ def main(argv=None):
     j.add_argument("-M", "--maxIntron", dest="maxIntron", default=500000, type=int)
     j.add_argument("--isStranded", dest="isStranded", default=False, action="store_true")
     j.add_argument("-s", "--strandedType", dest="strandedType", nargs="?", type=str)
+    j.add_argument("--strandFromXS", dest="strandFromXS", default=argparse.SUPPRESS, action="store_true",
+                   help="junction strands from the aligner's XS tag ('?' without one), as regtools writes them")
     pb = sub.add_parser("processBam", help="process without a BED12: junctions extracted from the BAM in the same pass")
     pb.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
     pb.add_argument("-o", "--outputPath", dest="outputPath", required=True)
@@ -375,7 +382,9 @@ def main(argv=None):
     pb.add_argument("--minAnchor", dest="minAnchor", default=8, type=int)
     pb.add_argument("--minIntron", dest="minIntron", default=70, type=int)
     pb.add_argument("--maxIntron", dest="maxIntron", default=500000, type=int)
-    kwargs = vars(parser.parse_args(argv))
+    pb.add_argument("--strandFromXS", dest="strandFromXS", default=argparse.SUPPRESS, action="store_true",
+                    help="junction strands from the aligner's XS tag; the count still follows --isStranded -s")
+    kwargs = vars(parser.parse_args(argv))          # --strandFromXS is only passed on when given (SUPPRESS)
     command = kwargs.pop("command")
     if command in ("combine", "combineShallow"):
         kwargs["devices"] = list(range(max(1, kwargs.pop("n_gpus") or 1)))
@@ -383,6 +392,8 @@ def main(argv=None):
         parser.error("--gene requires --annotationFile and --maxIntronSize")                      # S:1350-1353
     elif command in ("process", "combine", "combineShallow", "junctions", "processBam") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
         parser.error("--isStranded requires parameter --strandedType/-s as fr or rf")            # S:1354-1355
+    elif command == "junctions" and kwargs.get("strandFromXS") and kwargs.get("isStranded"):
+        parser.error("--strandFromXS and --isStranded name two strand sources for the junction table")
     elif command == "process":
         process(**kwargs)
     elif command == "combine":

@@ -14,7 +14,8 @@
 //                      Any broken link (or a feature this path does not parse: CG-tag long CIGARs) -> the caller falls
 //                      back to the host reader (bam_io.cpp).
 //   k_bam_fill         one warp per accepted member: the kept records (offsets listed by the counting walk) are written out
-//                      round-robin by the lanes: POS, FLAG, chromosome and CIGAR
+//                      round-robin by the lanes: POS, FLAG, chromosome and CIGAR (k_bam_fill<true>: and the XS strand, from
+//                      a walk of the record's aux fields by the same lane)
 //   k_bam_segments     chromosome boundaries of the record arrays (a coordinate-sorted BAM has one segment per reference)
 // Kept records follow the host reader: mapped to a caller chromosome and with at least one CIGAR operator (bam_io.cpp).
 #include <cuda_runtime.h>
@@ -25,6 +26,7 @@
 #include <string>
 #include <vector>
 
+#include "bam_aux.h"
 #include "bam_gpu.h"
 #include "device_types.h"
 #include "inflate.h"
@@ -158,6 +160,7 @@ __global__ void __launch_bounds__(128) k_bam_walk(const uint8_t* __restrict__ u,
 // second pass, one WARP per accepted member: the lanes take the kept records of the member round-robin from the offset list
 // the counting walk left, so neighbouring lanes write neighbouring records (the per-thread walk wrote with a stride of
 // ~1,000 records between lanes)
+template <bool XS>
 __global__ void __launch_bounds__(256) k_bam_fill(const uint8_t* __restrict__ u, const BgzfMember* __restrict__ mem, uint32_t n_mem,
                                                   const int32_t* __restrict__ refmap, const WalkOut* __restrict__ wo,
                                                   const uint64_t* __restrict__ rec_base, const uint64_t* __restrict__ cig_base,
@@ -188,6 +191,10 @@ __global__ void __launch_bounds__(256) k_bam_fill(const uint8_t* __restrict__ u,
             out.cig_off[ri] = (uint32_t)c0;
             const uint64_t cig = o + 36 + h.l_name;
             for (uint32_t q = 0; q < nc; ++q) out.cigar[c0 + q] = ld32u(u, cig + 4ull * q);
+            if (XS) {                                                  // aux fields: from the end of QUAL to the end of the record
+                const uint64_t aux = cig + 4ull * nc + ((uint64_t)h.l_seq + 1) / 2 + (uint64_t)h.l_seq;
+                out.xs[ri] = aux_xs_strand(u + aux, u + o + 4 + h.bs);  // aux <= the record end: the counting walk checked it
+            }
         }
         ci += tot;
     }
@@ -216,7 +223,7 @@ __global__ void k_set_u32(uint32_t* p, uint32_t v) { *p = v; }
 
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream, bool comp_uploaded,
-                   DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
+                   bool want_xs, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
     cudaStream_t st = (cudaStream_t)stream;
     const uint32_t n_mem = (uint32_t)members.size();
     cnt = BamGpuCounts{};
@@ -284,16 +291,19 @@ int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const
         size_t off = 0;
         auto take = [&](size_t bytes) { off = (off + 255) & ~(size_t)255; const size_t o = off; off += bytes; return o; };
         const size_t o_pos = take((nrec + 4) * 4), o_flag = take((nrec + 4) * 2), o_off = take((nrec + 4) * 4), o_cig = take((ncig + 4) * 4),
-                     o_chr = take((nrec + 4) * 4), o_sf = take(BAMGPU_MAX_SEG * 8), o_sc = take(BAMGPU_MAX_SEG * 4), o_ns = take(16);
+                     o_chr = take((nrec + 4) * 4), o_sf = take(BAMGPU_MAX_SEG * 8), o_sc = take(BAMGPU_MAX_SEG * 4), o_ns = take(16),
+                     o_xs = want_xs ? take(nrec + 4) : 0;
         if (mem.rec.reserve(off + 256) != cudaSuccess) { cudaGetLastError(); err = "not enough device memory for the record arrays"; return BAMGPU_FALLBACK; }
         char* rb = (char*)mem.rec.p;
         out.pos = (int32_t*)(rb + o_pos); out.flag = (uint16_t*)(rb + o_flag); out.cig_off = (uint32_t*)(rb + o_off);
         out.cigar = (uint32_t*)(rb + o_cig); out.chrom = (int32_t*)(rb + o_chr);
+        out.xs = want_xs ? (uint8_t*)(rb + o_xs) : nullptr;
         uint64_t* d_sf = (uint64_t*)(rb + o_sf); int32_t* d_sc = (int32_t*)(rb + o_sc); uint32_t* d_ns = (uint32_t*)(rb + o_ns);
         BG_CU(cudaMemcpyAsync(d_rbase, rbase.data(), (size_t)n_mem * 8, cudaMemcpyHostToDevice, st));
         BG_CU(cudaMemcpyAsync(d_cbase, cbase.data(), (size_t)n_mem * 8, cudaMemcpyHostToDevice, st));
         BG_CU(cudaMemsetAsync(d_ns, 0, 16, st));
-        { SPL_LAUNCH; k_bam_fill<<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out); }
+        if (want_xs) { SPL_LAUNCH; k_bam_fill<true><<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out); }
+        else { SPL_LAUNCH; k_bam_fill<false><<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out); }
         { SPL_LAUNCH; k_set_u32<<<1, 1, 0, st>>>(out.cig_off + nrec, (uint32_t)ncig); }
         if (nrec) { SPL_LAUNCH; k_bam_segments<<<(unsigned)((nrec + 255) / 256), 256, 0, st>>>(out.chrom, nrec, d_ns, d_sf, d_sc, BAMGPU_MAX_SEG); }
         BG_CU(cudaGetLastError());

@@ -22,6 +22,7 @@ struct DevRecordArrays {     // what DevRecords points at, plus the chromosome o
     uint32_t* cig_off = nullptr;
     uint32_t* cigar = nullptr;
     int32_t* chrom = nullptr;
+    uint8_t* xs = nullptr;   // strand of every record from its XS tag ('+', '-', '?'; bam_aux.h), only when the ingest was asked for it
 };
 
 struct BamGpuMem { GbBuf comp, unc, tab, rec, list; };
@@ -47,6 +48,6 @@ std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const cha
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream,
                    bool comp_uploaded /* mem.comp already holds the file image (copy queued on `stream`) */,
-                   DevRecordArrays& out, BamGpuCounts& cnt, std::string& err);
+                   bool want_xs /* fill out.xs */, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err);
 
 }  // namespace spl

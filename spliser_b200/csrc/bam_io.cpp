@@ -1,6 +1,7 @@
 // BGZF / BAM reader and writer over zlib.  Replaces, for this path, the `samtools view` subprocess
 // of SpliSER_v0_1_8.py:422 (one fork per splice site) by one streaming pass over the file.
 #include "bam_io.h"
+#include "bam_aux.h"
 #include "bam_gpu.h"
 
 #include <fcntl.h>
@@ -56,39 +57,18 @@ bool inflate_block(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t isi
 
 // aux walk: find CG:B,I (real CIGAR of reads with > 65535 operators)
 bool find_cg(const uint8_t* p, const uint8_t* end, const uint8_t*& data, uint32_t& n) {
-    while (p + 3 <= end) {
-        const uint8_t t0 = p[0], t1 = p[1], ty = p[2];
-        p += 3;
-        size_t sz = 0;
-        switch (ty) {
-            case 'A': case 'c': case 'C': sz = 1; break;
-            case 's': case 'S': sz = 2; break;
-            case 'i': case 'I': case 'f': sz = 4; break;
-            case 'Z': case 'H': { const uint8_t* q = p; while (q < end && *q) ++q; sz = (size_t)(q - p) + 1; break; }
-            case 'B': {
-                if (p + 5 > end) return false;
-                const uint8_t sub = p[0];
-                const uint32_t cnt = rd32(p + 1);
-                const size_t es = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4;
-                if (t0 == 'C' && t1 == 'G' && sub == 'I') {
-                    if (p + 5 + (size_t)cnt * 4 > end) return false;
-                    data = p + 5; n = cnt;
-                    return true;
-                }
-                sz = 5 + (size_t)cnt * es;
-                break;
-            }
-            default: return false;
-        }
-        if (p + sz > end) return false;
-        p += sz;
+    while (end - p >= 3) {
+        const uint8_t* nx = aux_field_end(p, end);
+        if (!nx) return false;
+        if (p[0] == 'C' && p[1] == 'G' && p[2] == 'B' && p[3] == 'I') { data = p + 8; n = rd32(p + 4); return true; }
+        p = nx;
     }
     return false;
 }
 
 }  // namespace
 
-std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out) {
+std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out, bool want_xs) {
     out = BamRecords();
     const int fd = open(path, O_RDONLY);
     if (fd < 0) return std::string("cannot open BAM file ") + path;
@@ -207,11 +187,13 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             if (32 + (size_t)l_name + (size_t)n_cig * 4 > bs) return "corrupt BAM record (CIGAR overruns record)";
             out.n_total++;
             p += 4 + bs;
+            // end of QUAL = start of the aux fields (l_seq < 0 or past the record: no aux block)
+            const uint8_t* aux = l_seq >= 0 ? cig + 4 * (size_t)n_cig + ((size_t)l_seq + 1) / 2 + (size_t)l_seq : nullptr;
+            if (aux && aux > r + bs) aux = nullptr;
             if (n_cig == 2 && l_seq >= 0 && rd32(cig) == (((uint32_t)l_seq << 4) | 4u) && (rd32(cig + 4) & 15u) == 3u) {
-                const uint8_t* aux = cig + 8 + ((size_t)l_seq + 1) / 2 + (size_t)l_seq;
                 const uint8_t* cg = nullptr;
                 uint32_t n = 0;
-                if (aux <= r + bs && find_cg(aux, r + bs, cg, n)) { cig = cg; n_cig = n; }
+                if (aux && find_cg(aux, r + bs, cg, n)) { cig = cg; n_cig = n; }
             }
             const int32_t chrom = (refid >= 0 && (size_t)refid < refmap.size()) ? refmap[(size_t)refid] : -1;
             if (chrom < 0 || n_cig == 0) { out.n_skipped++; continue; }
@@ -222,6 +204,7 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             }
             out.pos.push_back(pos0 + 1);
             out.flag.push_back(flag);
+            if (want_xs) out.xs.push_back(aux ? aux_xs_strand(aux, r + bs) : (uint8_t)'?');
             const size_t c0 = out.cigar.size();
             out.cigar.resize(c0 + n_cig);
             memcpy(out.cigar.data() + c0, cig, (size_t)n_cig * 4);   // BAM is little-endian, so is every host we build for
@@ -356,8 +339,8 @@ bool deflate_block(const uint8_t* src, uint32_t n, std::vector<uint8_t>& dst) {
 }  // namespace
 
 std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
-                      const spl_records_view* rec, int n_threads, bool with_seq) {
-    if (!path || !rec || n_ref < 0) return "bad argument";
+                      const spl_records_view* rec, int n_threads, bool with_seq, const int64_t* aux_off, const uint8_t* aux) {
+    if (!path || !rec || n_ref < 0 || (aux_off && !aux)) return "bad argument";
     std::vector<uint8_t> u;
     u.reserve((size_t)rec->n_rec * (with_seq ? 300 : 40) + (size_t)rec->n_cigar * 4 + 4096);
     u.insert(u.end(), {'B', 'A', 'M', 1});
@@ -386,8 +369,11 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
                 if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) reflen += rec->cigar[k] >> 4;
             }
             const int32_t pos0 = rec->pos[i] - 1;
+            const int64_t a0 = aux_off ? aux_off[i] : 0, a1 = aux_off ? aux_off[i + 1] : 0;
+            if (a1 < a0 || a1 - a0 > (1 << 24)) return "write_bam: bad aux offsets";
+            const uint32_t n_aux = (uint32_t)(a1 - a0);
             if (!with_seq) {
-                wr32(u, 32 + 2 + n_cig * 4);
+                wr32(u, 32 + 2 + n_cig * 4 + n_aux);
                 wr32(u, (uint32_t)ref);
                 wr32(u, (uint32_t)pos0);
                 u.push_back(2);                       // l_read_name
@@ -399,6 +385,7 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
                 wr32(u, (uint32_t)-1); wr32(u, (uint32_t)-1); wr32(u, 0);   // next_refID, next_pos, tlen
                 u.push_back('r'); u.push_back(0);
                 for (uint32_t k = c0; k < c1; ++k) wr32(u, rec->cigar[k]);
+                u.insert(u.end(), aux + a0, aux + a1);
                 continue;
             }
             // a sequencer-shaped record: read name, SEQ and QUAL of the CIGAR's query length (seeded pseudo-random bases and
@@ -410,7 +397,7 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
             }
             char name[16];
             const int ln = snprintf(name, sizeof name, "r%09lld", (long long)(i % 1000000000LL)) + 1;
-            wr32(u, 32 + (uint32_t)ln + n_cig * 4 + (qlen + 1) / 2 + qlen);
+            wr32(u, 32 + (uint32_t)ln + n_cig * 4 + (qlen + 1) / 2 + qlen + n_aux);
             wr32(u, (uint32_t)ref);
             wr32(u, (uint32_t)pos0);
             u.push_back((uint8_t)ln);
@@ -432,6 +419,7 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
                 if ((v & 7) == 0) ql = 2 + (uint32_t)((v >> 8) % 39);
                 u.push_back((uint8_t)ql);
             }
+            u.insert(u.end(), aux + a0, aux + a1);
         }
     }
     const size_t PIECE = 0xff00;
@@ -469,6 +457,7 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
 struct spl_records {
     spl::BamRecords r;
     spl_records_view v;
+    bool has_xs = false;    // read by spl_read_bam_xs: r.xs holds one strand byte per record
 };
 
 extern "C" {
@@ -480,6 +469,14 @@ int spl_write_bam_seq(const char* path, int32_t n_ref, const char* const* ref_na
     return SPL_OK;
 }
 
+int spl_write_bam_aux(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len, const spl_records_view* rec,
+                      const int64_t* aux_off, const uint8_t* aux, int with_seq, int n_threads) {
+    if (!aux_off) return SPL_ERR_ARG;
+    const std::string e = spl::write_bam(path, n_ref, ref_names, ref_len, rec, n_threads, with_seq != 0, aux_off, aux);
+    if (!e.empty()) { fprintf(stderr, "spl_write_bam_aux: %s\n", e.c_str()); return SPL_ERR_IO; }
+    return SPL_OK;
+}
+
 int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                   const spl_records_view* rec, int n_threads) {
     const std::string e = spl::write_bam(path, n_ref, ref_names, ref_len, rec, n_threads);
@@ -487,24 +484,38 @@ int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names,
     return SPL_OK;
 }
 
-int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, spl_records** out,
-                 char* err, int err_len) {
+namespace {
+int read_bam_handle(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, bool want_xs, spl_records** out,
+                    char* err, int err_len) {
     if (!out || !path) return SPL_ERR_ARG;
     *out = nullptr;
     spl_records* h = new (std::nothrow) spl_records();
     if (!h) return SPL_ERR_NOMEM;
-    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r);
+    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r, want_xs);
     if (!e.empty()) {
         if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
         delete h;
         return SPL_ERR_IO;
     }
     h->v = h->r.view();
+    h->has_xs = want_xs;
     *out = h;
     return SPL_OK;
 }
+}  // namespace
+
+int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, spl_records** out,
+                 char* err, int err_len) {
+    return read_bam_handle(path, n_chrom, chrom_names, n_threads, false, out, err, err_len);
+}
+
+int spl_read_bam_xs(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, spl_records** out,
+                    char* err, int err_len) {
+    return read_bam_handle(path, n_chrom, chrom_names, n_threads, true, out, err, err_len);
+}
 
 const spl_records_view* spl_records_get(const spl_records* r) { return r ? &r->v : nullptr; }
+const uint8_t* spl_records_xs(const spl_records* r) { return r && r->has_xs ? r->r.xs.data() : nullptr; }
 
 int spl_bam_reference_names(const char* path, char* names, int64_t cap, int64_t* n_ref, int64_t* bytes, char* err, int err_len) {
     if (!path || !n_ref || !bytes || cap < 0 || (cap > 0 && !names)) return SPL_ERR_ARG;

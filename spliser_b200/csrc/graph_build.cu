@@ -1249,9 +1249,10 @@ struct JeOut {
     uint32_t* ext_l;                // JE_EXTENT: [n_u] atomicMax of the left / right stretch
     uint32_t* ext_r;
 };
-template <int PASS>
+// XS: every junction of record r takes the strand xs[r] ('+', '-', else '?') instead of the one `mode` derives from the FLAG
+template <int PASS, bool XS>
 __global__ void __launch_bounds__(256) k_je_walk(DevRecords rec, JeSeg sg, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron,
-                                                 int pb, JeOut o) {
+                                                 int pb, JeOut o, const uint8_t* __restrict__ xs) {
     const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = r < rec.n_rec;                                    // every lane reaches the warp reduction of JE_COUNT
     const int chrom = live ? je_chrom_of(sg, r) : -1;
@@ -1260,7 +1261,10 @@ __global__ void __launch_bounds__(256) k_je_walk(DevRecords rec, JeSeg sg, uint3
         const uint32_t c0 = rec.cig_off[r], c1 = rec.cig_off[r + 1];
         const uint32_t flag = rec.flag[r];
         uint32_t strand = 0;                                            // 0 '?', 1 '+', 2 '-'
-        if (mode & FLAG_STRANDED) {
+        if (XS) {
+            const uint8_t x = xs[r];
+            strand = x == '+' ? 1u : x == '-' ? 2u : 0u;
+        } else if (mode & FLAG_STRANDED) {
             const bool first = (flag & 64u) || !(flag & 1u), rev = (flag & 16u) != 0;
             bool plus = first != rev;
             if (mode & FLAG_RF) plus = !plus;
@@ -1525,9 +1529,10 @@ bool graph_build_device(GraphBuildMem& m, const int32_t* j_chrom, const int32_t*
 // Junction table of the device-resident records, sorted by (chromosome, l, r, strand), with each row's anchor extents.
 // Synchronises the stream (sizes).
 bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int64_t* h_seg_off, const int32_t* h_seg_chrom, int32_t n_seg,
-                             int32_t n_chrom, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron, void* stream,
-                             std::vector<int32_t>& chrom, std::vector<int32_t>& left, std::vector<int32_t>& right, std::vector<int64_t>& score,
-                             std::vector<uint8_t>& strand, std::vector<int32_t>& start, std::vector<int32_t>& end, std::string& err) {
+                             int32_t n_chrom, uint32_t mode, const uint8_t* xs, int32_t min_anchor, int32_t min_intron, int32_t max_intron,
+                             void* stream, std::vector<int32_t>& chrom, std::vector<int32_t>& left, std::vector<int32_t>& right,
+                             std::vector<int64_t>& score, std::vector<uint8_t>& strand, std::vector<int32_t>& start, std::vector<int32_t>& end,
+                             std::string& err) {
     cudaStream_t st = (cudaStream_t)stream;
     chrom.clear(); left.clear(); right.clear(); score.clear(); strand.clear(); start.clear(); end.clear();
     const uint32_t R = rec.n_rec;
@@ -1555,7 +1560,8 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     for (auto& e : m.ev) if (!e) GB_CU(cudaEventCreate(&e));
     m.ms_kernels = m.ms_extent = 0;
     GB_CU(cudaEventRecord(m.ev[0], st));
-    { SPL_LAUNCH; k_je_walk<JE_COUNT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, 0, jo); }
+    if (xs) { SPL_LAUNCH; k_je_walk<JE_COUNT, true><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, 0, jo, xs); }
+    else { SPL_LAUNCH; k_je_walk<JE_COUNT, false><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, 0, jo, nullptr); }
     sc0.scan(cnt, R, nullptr, d_tot);
     GB_CU(cudaEventRecord(m.ev[1], st));
     uint32_t h_tot[4] = {0, 0, 0, 0};
@@ -1588,7 +1594,8 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     const Sorter sorter{(uint32_t*)(bb + b_hist), sc, d_tot + 5, st};
     jo.keys = ka;
     GB_CU(cudaEventRecord(m.ev[2], st));
-    { SPL_LAUNCH; k_je_walk<JE_EMIT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo); }
+    if (xs) { SPL_LAUNCH; k_je_walk<JE_EMIT, true><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo, xs); }
+    else { SPL_LAUNCH; k_je_walk<JE_EMIT, false><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo, nullptr); }
     uint64_t* sk = sorter.sort(ka, kb, n, 0, 22 + pb + cb);
     { SPL_LAUNCH; k_je_heads<<<cdiv(n, 256), 256, 0, st>>>(sk, n, flag); }
     sc.scan(flag, n, nullptr, d_tot + 1);
@@ -1606,7 +1613,8 @@ bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int
     GB_CU(cudaMemsetAsync(bb + b_xr, 0, U * 4, st));
     jo.ukeys = ukey; jo.n_u = (uint32_t)U; jo.ext_l = (uint32_t*)(bb + b_xl); jo.ext_r = (uint32_t*)(bb + b_xr);
     GB_CU(cudaEventRecord(m.ev[4], st));
-    { SPL_LAUNCH; k_je_walk<JE_EXTENT><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo); }
+    if (xs) { SPL_LAUNCH; k_je_walk<JE_EXTENT, true><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo, xs); }
+    else { SPL_LAUNCH; k_je_walk<JE_EXTENT, false><<<cdiv(R, 256), 256, 0, st>>>(rec, sg, mode, min_anchor, min_intron, max_intron, pb, jo, nullptr); }
     GB_CU(cudaGetLastError());
     GB_CU(cudaEventRecord(m.ev[5], st));
     chrom.resize(U); left.resize(U); right.resize(U); strand.resize(U); score.resize(U); start.resize(U); end.resize(U);

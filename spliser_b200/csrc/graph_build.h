@@ -59,7 +59,8 @@ bool graph_build_device(GraphBuildMem& m, const int32_t* j_chrom, const int32_t*
                         int phase /* 0: allocate + upload the junction table, 1: build + read sizes, 2: build only */, GraphDev& g, GraphCounts& counts, std::string& err);
 
 // junction extraction from device-resident records (graph_build.cu, shares its sort / scan kernels); start / end: the rows'
-// BED12 chromStart / chromEnd (l - longest left anchor, r + longest right anchor)
+// BED12 chromStart / chromEnd (l - longest left anchor, r + longest right anchor).  xs: NULL (strands from `mode`: FLAG_STRANDED /
+// FLAG_RF) or a device column of one strand byte per record ('+', '-', '?'), which then gives every junction of the record its strand
 struct JuncExtractMem {
     GbBuf a, b;
     cudaEvent_t ev[6] = {};          // bracket the three kernel stretches between the host reads of the sizes
@@ -71,7 +72,7 @@ struct JuncExtractMem {
 };
 struct DevRecords;
 bool junction_extract_device(JuncExtractMem& m, const DevRecords& rec, const int64_t* h_seg_off, const int32_t* h_seg_chrom, int32_t n_seg,
-                             int32_t n_chrom, uint32_t mode, int32_t min_anchor, int32_t min_intron, int32_t max_intron, void* stream,
+                             int32_t n_chrom, uint32_t mode, const uint8_t* xs, int32_t min_anchor, int32_t min_intron, int32_t max_intron, void* stream,
                              std::vector<int32_t>& chrom, std::vector<int32_t>& left, std::vector<int32_t>& right, std::vector<int64_t>& score,
                              std::vector<uint8_t>& strand, std::vector<int32_t>& start, std::vector<int32_t>& end, std::string& err);
 

@@ -197,6 +197,7 @@ struct spl_ctx {
     // fused variant (count_fused.cu)
     DevBuf d_cpk;                                        // the columns of a compact upload (spl_process_compact)
     DevBuf d_frec, d_fchunks, d_hotq, d_fpk, d_unpack;   // d_fpk: packed columns (n_op, flag8) of spl_process_packed; d_unpack: scan descriptors + ticket
+    DevBuf d_xs;                    // XS strand column of host records for the extraction (SPL_FLAG_XS_STRAND)
     uint32_t unpack_epoch = 0;
     uint32_t hot_cap = 0;           // items the global hot queue holds; a pass that needs more is repeated with room
     uint32_t* h_hot = nullptr;      // pinned: hot item count of the last pass
@@ -1319,8 +1320,9 @@ int load_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int6
 
 // BAM file -> record arrays on the device.  SPL_OK: ctx->dev_rec / `cnt` are filled and `view` describes them
 // (array pointers NULL, ctx->rec_on_device must be set by the caller around the load).  *fallback = true: use the host reader.
+// want_xs: ctx->dev_rec.xs receives the XS strand of every record as well.
 int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const char* const* chrom_names, BamGpuCounts& cnt,
-                      spl_records_view& view, bool* fallback) {
+                      spl_records_view& view, bool* fallback, bool want_xs = false) {
     *fallback = false;
     if (const char* f = std::getenv("SPLISER_HOST_BAM")) if (f[0] == '1') { *fallback = true; return SPL_OK; }
     const int fd = open(path, O_RDONLY);
@@ -1378,7 +1380,7 @@ int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const cha
     std::string e = bam_scan((const uint8_t*)ctx->h_file, fsz, n_chrom, chrom_names, members, total_u, first_record, n_ref, refmap);
     if (!e.empty()) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_IO, "%s", e.c_str()); }
     const int rc = bam_gpu_ingest(ctx->bgm, (const uint8_t*)ctx->h_file, fsz, members, total_u, first_record, n_ref, refmap, ctx->stream,
-                                  uploaded, ctx->dev_rec, cnt, e);
+                                  uploaded, want_xs, ctx->dev_rec, cnt, e);
     if (rc != BAMGPU_OK) cudaStreamSynchronize(ctx->stream);           // the pinned image may be re-used by the fallback / next call
     if (rc == BAMGPU_ERROR) return ctx->fail(SPL_ERR_CUDA, "%s", e.c_str());
     if (rc == BAMGPU_FALLBACK) { *fallback = true; return SPL_OK; }
@@ -1453,6 +1455,7 @@ void spl_destroy(spl_ctx* ctx) {
         }
         if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
         ctx->d_frec.release(); ctx->d_fchunks.release(); ctx->d_hotq.release(); ctx->d_fpk.release(); ctx->d_unpack.release(); ctx->d_cpk.release();
+        ctx->d_xs.release();
         if (ctx->h_hot) cudaFreeHost(ctx->h_hot);
         if (ctx->h_fchunks) cudaFreeHost(ctx->h_fchunks);
         for (int p = 0; p < MAX_FPARTS; ++p) if (ctx->fpart[p].ev_up) cudaEventDestroy(ctx->fpart[p].ev_up);
@@ -1684,8 +1687,9 @@ struct spl_junctions {
 };
 
 namespace {
-int extract_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int32_t min_anchor, int32_t min_intron, int32_t max_intron,
-                   uint32_t flags, spl_junctions** out) {
+// xs: the host records' XS strand column (SPL_FLAG_XS_STRAND without records on the device; the device ingest fills ctx->dev_rec.xs)
+int extract_common(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom, int32_t min_anchor, int32_t min_intron,
+                   int32_t max_intron, uint32_t flags, spl_junctions** out) {
     if (min_anchor < 0 || min_intron < 0 || max_intron < min_intron) return ctx->fail(SPL_ERR_ARG, "bad anchor / intron bounds");
     ctx->loaded = false;
     int rc = check_view(ctx, rec, n_chrom);
@@ -1695,11 +1699,23 @@ int extract_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, i
     rc = fused_upload(ctx, rec, n_chrom, false);
     if (rc) return drain_on_error(ctx, rc);
     CU(cudaStreamWaitEvent(ctx->stream, ctx->fpart[0].ev_up, 0));
+    const uint8_t* d_xs = nullptr;
+    if ((flags & SPL_FLAG_XS_STRAND) && rec->n_rec > 0) {
+        if (ctx->rec_on_device) {
+            d_xs = ctx->dev_rec.xs;
+        } else if (xs) {                                                   // 1 B per record, once
+            CU(ctx->d_xs.reserve((size_t)rec->n_rec + 16));
+            CU(cudaMemcpyAsync(ctx->d_xs.p, xs, (size_t)rec->n_rec, cudaMemcpyHostToDevice, ctx->stream));
+            ctx->stats[SPL_STAT_H2D_BYTES] += (double)rec->n_rec;
+            d_xs = (const uint8_t*)ctx->d_xs.p;
+        }
+        if (!d_xs) return drain_on_error(ctx, ctx->fail(SPL_ERR_ARG, "SPL_FLAG_XS_STRAND without an XS strand column"));
+    }
     std::unique_ptr<spl_junctions> j(new (std::nothrow) spl_junctions());
     if (!j) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
     std::string e;
-    if (!junction_extract_device(ctx->jem, ctx->frec, rec->seg_off, rec->seg_chrom, rec->n_seg, n_chrom, flags & 3u, min_anchor, min_intron,
-                                 max_intron, ctx->stream, j->chrom, j->left, j->right, j->score, j->strand, j->start, j->end, e))
+    if (!junction_extract_device(ctx->jem, ctx->frec, rec->seg_off, rec->seg_chrom, rec->n_seg, n_chrom, flags & 3u, d_xs, min_anchor,
+                                 min_intron, max_intron, ctx->stream, j->chrom, j->left, j->right, j->score, j->strand, j->start, j->end, e))
         return drain_on_error(ctx, ctx->fail(SPL_ERR_CUDA, "%s", e.c_str()));
     ctx->stats[SPL_STAT_MS_EXTRACT] = ctx->jem.ms_kernels;
     ctx->stats[SPL_STAT_MS_EXTENTS] = ctx->jem.ms_extent;
@@ -1709,11 +1725,12 @@ int extract_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, i
 }
 
 // spl_process_bam_extract after the ingest: junction table of the records, the -c / -g row filters, then the count over the
-// same records, which extract_common left on the device (ctx->frec) -- they cross PCIe at most once.
-int extract_and_count(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, const char* const* chrom_names, const spl_extract_opts* o,
-                      uint32_t flags, spl_junctions** rows_out, spl_result** out) {
+// same records, which extract_common left on the device (ctx->frec) -- they cross PCIe at most once.  SPL_FLAG_XS_STRAND only
+// chooses the table's strands: the count runs with the remaining flags.
+int extract_and_count(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom, const char* const* chrom_names,
+                      const spl_extract_opts* o, uint32_t flags, spl_junctions** rows_out, spl_result** out) {
     spl_junctions* got = nullptr;
-    int rc = extract_common(ctx, rec, n_chrom, o->min_anchor, o->min_intron, o->max_intron, flags, &got);
+    int rc = extract_common(ctx, rec, xs, n_chrom, o->min_anchor, o->min_intron, o->max_intron, flags, &got);
     if (rc) return rc;
     std::unique_ptr<spl_junctions> all(got);
     double keep[SPL_NSTATS];
@@ -1738,7 +1755,7 @@ int extract_and_count(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom
     dv.n_rec = rec->n_rec; dv.n_cigar = rec->n_cigar; dv.n_seg = rec->n_seg; dv.seg_chrom = rec->seg_chrom; dv.seg_off = rec->seg_off;
     ctx->rec_on_device = true;
     rc = spl_process_records(ctx, &dv, n_chrom, (int64_t)j->chrom.size(), j->chrom.data(), j->left.data(), j->right.data(),
-                             j->score.data(), j->strand.data(), flags, out);
+                             j->score.data(), j->strand.data(), flags & ~SPL_FLAG_XS_STRAND, out);
     ctx->rec_on_device = saved_dev;
     ctx->dev_rec = saved;
     if (rc) return rc;
@@ -1755,7 +1772,18 @@ int spl_extract_junctions_records(spl_ctx* ctx, const spl_records_view* rec, int
     if (!out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
-    return extract_common(ctx, rec, n_chrom, min_anchor, min_intron, max_intron, flags, out);
+    if (flags & SPL_FLAG_XS_STRAND) return ctx->fail(SPL_ERR_ARG, "SPL_FLAG_XS_STRAND needs the strand column of spl_extract_junctions_records_xs");
+    return extract_common(ctx, rec, nullptr, n_chrom, min_anchor, min_intron, max_intron, flags, out);
+}
+
+int spl_extract_junctions_records_xs(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom, int32_t min_anchor,
+                                     int32_t min_intron, int32_t max_intron, uint32_t flags, spl_junctions** out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!xs && rec && rec->n_rec > 0) return ctx->fail(SPL_ERR_ARG, "xs is NULL");
+    return extract_common(ctx, rec, xs, n_chrom, min_anchor, min_intron, max_intron, flags, out);
 }
 
 int spl_extract_junctions(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names, int32_t min_anchor,
@@ -1765,25 +1793,35 @@ int spl_extract_junctions(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, c
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
+    const double t0 = now_ms();
     CU(cudaSetDevice(ctx->device));
     {
         BamGpuCounts cnt;
         spl_records_view dv{};
         bool fallback = false;
-        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback);
+        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback, (flags & SPL_FLAG_XS_STRAND) != 0);
         if (rc) return rc;
         if (!fallback) {
+            const double t1 = now_ms();
             ctx->rec_on_device = true;
-            rc = extract_common(ctx, &dv, n_chrom, min_anchor, min_intron, max_intron, flags, out);
+            rc = extract_common(ctx, &dv, nullptr, n_chrom, min_anchor, min_intron, max_intron, flags, out);
             ctx->rec_on_device = false;
+            ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+            ctx->stats[SPL_STAT_H2D_BYTES] += cnt.h2d_bytes;
+            ctx->stats[SPL_STAT_BAM_DEVICE] = 1.0;
+            ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
             return rc;
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs);
+    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
+    const double t1 = now_ms();
     spl_records_view v = recs.view();
-    return extract_common(ctx, &v, n_chrom, min_anchor, min_intron, max_intron, flags, out);
+    const int rc = extract_common(ctx, &v, recs.xs.data(), n_chrom, min_anchor, min_intron, max_intron, flags, out);
+    ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
 }
 
 int64_t spl_junctions_n(const spl_junctions* j) { return j ? (int64_t)j->chrom.size() : 0; }
@@ -1810,12 +1848,12 @@ int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom,
         BamGpuCounts cnt;
         spl_records_view dv{};
         bool fallback = false;
-        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback);
+        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback, (flags & SPL_FLAG_XS_STRAND) != 0);
         if (rc) return rc;
         if (!fallback) {
             const double t1 = now_ms();
             ctx->rec_on_device = true;
-            rc = extract_and_count(ctx, &dv, n_chrom, chrom_names, opts, flags, rows_out, out);
+            rc = extract_and_count(ctx, &dv, nullptr, n_chrom, chrom_names, opts, flags, rows_out, out);
             ctx->rec_on_device = false;
             ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
             ctx->stats[SPL_STAT_H2D_BYTES] += cnt.h2d_bytes;
@@ -1825,11 +1863,11 @@ int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom,
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs);
+    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
-    const int rc = extract_and_count(ctx, &v, n_chrom, chrom_names, opts, flags, rows_out, out);
+    const int rc = extract_and_count(ctx, &v, recs.xs.data(), n_chrom, chrom_names, opts, flags, rows_out, out);
     ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
     ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
     return rc;
