@@ -252,6 +252,37 @@ typedef struct spl_extract_opts {
 int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names,
                             const spl_extract_opts* opts, uint32_t flags, spl_junctions** rows_out, spl_result** out);
 
+/* ---- device-resident samples ---------------------------------------------------------------------------------------------
+ * One BAM's alignment records held in device memory, so that a multi-sample run (`combine` after `process` per sample) ingests
+ * every BAM once: spl_sample_process_extract is spl_process_bam_extract and spl_sample_recount is spl_recount, each without the
+ * ingest.  Both take the caller's chromosome list and map the header's references to it by name on the host, as every BAM
+ * reader here does (the first index of a name that repeats; a reference that is not in the list is skipped).
+ *
+ * spl_sample_load_bam ingests the file as spl_process chooses (on the device, or the host reader as the fallback), keeps every
+ * record of every header reference and copies POS, FLAG, the CIGAR offsets and operators -- and with SPL_FLAG_XS_STRAND (the
+ * only flag it reads) the XS strand column -- into one device allocation of the sample's own.  The inflate scratch stays with
+ * the context and is re-used by its next load.  spl_last_stats reports the load's SPL_STAT_H2D_BYTES and SPL_STAT_BAM_DEVICE.
+ *
+ * Residency: the load returns SPL_ERR_NOMEM and holds nothing when the allocation fails, or when less than the sample's size
+ * plus 1 GiB would stay free on the device after it (cudaMemGetInfo) -- the context's headroom for the next load's copy of a
+ * sample of the same size and for the counting buffers of the next call.  The context stays usable; the caller takes the path
+ * route (spl_process_bam_extract / spl_recount) for that sample.  SPLISER_SAMPLE_BUDGET_MB caps the bytes all samples of the
+ * process may hold together (a test hook: it chooses which samples stay resident, never a result).
+ *
+ * A sample belongs to the context that loaded it: passing it to another one is SPL_ERR_ARG.  spl_sample_free does not touch
+ * the context (it may already be destroyed); one call at a time per context, as everywhere. */
+typedef struct spl_sample spl_sample;
+int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_sample** out);
+int spl_sample_process_extract(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
+                               const spl_extract_opts* opts, uint32_t flags, spl_junctions** rows_out, spl_result** out);
+int spl_sample_recount(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
+                       int64_t n_sites, const int32_t* s_chrom, const int32_t* s_pos, const uint8_t* s_strand,
+                       const int64_t* p_off, const int32_t* p_pos, const int64_t* c_off, const int32_t* c_pos,
+                       uint32_t flags, int64_t* beta1_out, int64_t* beta2simple_out);
+int64_t spl_sample_n_records(const spl_sample* s);
+int64_t spl_sample_device_bytes(const spl_sample* s);
+void    spl_sample_free(spl_sample* s);
+
 /* Reference names of a BAM header in header order (host only, no GPU): written NUL-terminated back to back into
  * names[0 .. cap) when *bytes (the space they need) <= cap; *n_ref and *bytes are always set. */
 int spl_bam_reference_names(const char* path, char* names, int64_t cap, int64_t* n_ref, int64_t* bytes, char* err, int err_len);

@@ -5,7 +5,7 @@ package is its Python host side: ctypes binding, numpy API, BED12 parsing, gene 
 SpliSER-compatible CLI and TSV writers.  Importing the package does not need a GPU; creating a
 Context does, and there is no CPU fallback.
 """
-from .api import (CompactRecords, Context, Junctions, PackedRecords, Records, SiteTable, SpliserError, mode_flags,  # noqa: F401
-                  FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names)
+from .api import (CompactRecords, Context, DeviceSample, Junctions, PackedRecords, Records, SampleMemoryError, SiteTable,  # noqa: F401
+                  SpliserError, mode_flags, FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names)
 
 __version__ = "0.1.0"

@@ -14,6 +14,8 @@ SPL_FLAG_CRYPTIC = 4
 SPL_FLAG_COMBINE = 8
 SPL_FLAG_XS_STRAND = 16
 
+SPL_ERR_NOMEM = -4
+
 SPL_NSTATS = 32
 STAT_NAMES = ("ms_total", "ms_beta1", "ms_spliced", "ms_final", "n_mblocks_a", "n_mblocks_b", "n_junc_ops",
               "n_spliced", "n_sites", "n_edges", "n_aligned", "launches", "ms_expand", "ms_decode",
@@ -96,6 +98,13 @@ SIGNATURES = {
     "spl_junctions_free": (None, [C.c_void_p]),
     "spl_process_bam_extract": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp, C.POINTER(ExtractOpts), C.c_uint32,
                                           C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    "spl_sample_load_bam": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint32, C.POINTER(C.c_void_p)]),
+    "spl_sample_process_extract": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, c_strp, C.POINTER(ExtractOpts), C.c_uint32,
+                                             C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    "spl_sample_recount": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, c_strp] + _GAPS + [C.c_uint32, c_i64p, c_i64p]),
+    "spl_sample_n_records": (C.c_int64, [C.c_void_p]),
+    "spl_sample_device_bytes": (C.c_int64, [C.c_void_p]),
+    "spl_sample_free": (None, [C.c_void_p]),
     "spl_bam_reference_names": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int64, c_i64p, c_i64p, C.c_char_p, C.c_int]),
     "spl_write_junctions_bed": (C.c_int, [C.c_char_p, C.c_int64, c_i32p, c_i32p, c_i32p, c_i32p, c_i32p, c_i64p, c_u8p,
                                           C.POINTER(StrTab), C.c_char_p, C.c_int]),

@@ -465,6 +465,59 @@ class SpliserError(RuntimeError):
     pass
 
 
+class SampleMemoryError(SpliserError):
+    """Context.load_bam refused to hold a sample on the device (SPL_ERR_NOMEM); the context stays usable."""
+
+
+def _names(chrom_names):
+    return (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
+
+
+class DeviceSample:
+    """One BAM's alignment records in device memory (Context.load_bam): the extraction + count of process_bam_extract and the
+    re-count of recount_bam without reading the file again.  Calls go through the context that loaded it.  A context manager;
+    close() frees the device memory."""
+
+    def __init__(self, ctx: "Context", h):
+        self._ctx, self._h = ctx, h
+
+    @property
+    def n_records(self) -> int:
+        return int(self._ctx._lib.spl_sample_n_records(self._h))
+
+    @property
+    def device_bytes(self) -> int:
+        return int(self._ctx._lib.spl_sample_device_bytes(self._h))
+
+    def process_extract(self, chrom_names, flags: int = 0, min_anchor=8, min_intron=70, max_intron=500000, qchrom="All",
+                        gene_bounds=None, window_max_intron=0):
+        """Context.process_bam_extract of the loaded BAM: (Junctions after the filters, SiteTable)."""
+        c = self._ctx
+        return c._extract_and_count(c._lib.spl_sample_process_extract, self._h, chrom_names, flags, min_anchor, min_intron, max_intron,
+                                    qchrom, gene_bounds, window_max_intron)
+
+    def recount(self, chrom_names, gaps, flags: int):
+        """Context.recount_bam of the loaded BAM: (beta1, beta2simple)."""
+        return self._ctx._recount(self._ctx._lib.spl_sample_recount, self._h, chrom_names, gaps, flags)
+
+    def close(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            self._ctx._lib.spl_sample_free(h)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Context:
     """One spl_ctx = one GPU (one process per GPU)."""
 
@@ -620,14 +673,30 @@ class Context:
         filtered like a BED12 of it (-c qchrom, -g window gene_bounds = (leftPos, rightPos) widened by window_max_intron,
         S:269, S:279-288) and counted against the same device-resident records.  Returns (Junctions after the filters, in the
         order they were counted -- first_line indexes them; SiteTable)."""
-        names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
+        return self._extract_and_count(self._lib.spl_process_bam_extract, str(bam_path).encode(), chrom_names, flags, min_anchor,
+                                       min_intron, max_intron, qchrom, gene_bounds, window_max_intron)
+
+    def _extract_and_count(self, fn, source, chrom_names, flags, min_anchor, min_intron, max_intron, qchrom, gene_bounds,
+                           window_max_intron):
+        names = _names(chrom_names)
         o = L.ExtractOpts(int(min_anchor), int(min_intron), int(max_intron), None if qchrom == "All" else str(qchrom).encode(),
                           int(gene_bounds is not None), *(int(x) for x in (gene_bounds or (0, 0))), int(window_max_intron))
         hj, hr = C.c_void_p(), C.c_void_p()
-        rc = self._lib.spl_process_bam_extract(self._h, str(bam_path).encode(), len(chrom_names), names, C.byref(o), flags,
-                                               C.byref(hj), C.byref(hr))
-        self._check(rc, "spl_process_bam_extract")
+        self._check(fn(self._h, source, len(chrom_names), names, C.byref(o), flags, C.byref(hj), C.byref(hr)), fn.__name__)
         return self._take_junctions(hj), self._take(hr)
+
+    # ---- device-resident samples -----------------------------------------------------------------
+    def load_bam(self, bam_path, xs=False) -> "DeviceSample":
+        """Ingests a BAM once and keeps its records in device memory owned by the returned DeviceSample (every header reference,
+        in header order; with xs=True the XS strand column too, for FLAG_XS_STRAND).  Raises SampleMemoryError when the sample
+        does not fit next to this context's working memory (include/spliser_b200.h states the rule): the caller then takes
+        the path route, process_bam_extract / recount_bam, for that sample."""
+        h = C.c_void_p()
+        rc = self._lib.spl_sample_load_bam(self._h, str(bam_path).encode(), FLAG_XS_STRAND if xs else 0, C.byref(h))
+        if rc == L.SPL_ERR_NOMEM:
+            raise SampleMemoryError("spl_sample_load_bam(%s): %s" % (bam_path, self._lib.spl_last_error(self._h).decode()))
+        self._check(rc, "spl_sample_load_bam")
+        return DeviceSample(self, h)
 
     # ---- combine re-count ----------------------------------------------------------------------
     @staticmethod
@@ -648,13 +717,14 @@ class Context:
         return b1, b2
 
     def recount_bam(self, bam_path, chrom_names, gaps, flags: int):
+        return self._recount(self._lib.spl_recount, str(bam_path).encode(), chrom_names, gaps, flags)
+
+    def _recount(self, fn, source, chrom_names, gaps, flags):
         keep, args = self._gap_args(gaps)
         b1 = np.zeros(len(gaps), dtype=np.int64)
         b2 = np.zeros(len(gaps), dtype=np.int64)
-        names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
-        rc = self._lib.spl_recount(self._h, str(bam_path).encode(), len(chrom_names), names, *args, flags,
-                                   _ptr(b1, L.c_i64p), _ptr(b2, L.c_i64p))
-        self._check(rc, "spl_recount")
+        rc = fn(self._h, source, len(chrom_names), _names(chrom_names), *args, flags, _ptr(b1, L.c_i64p), _ptr(b2, L.c_i64p))
+        self._check(rc, fn.__name__)
         return b1, b2
 
     # ---- resident (benchmark) path -------------------------------------------------------------

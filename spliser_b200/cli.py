@@ -9,10 +9,14 @@ Without regtools (not a reference command; regtools' option letters):
     python -m spliser_b200.cli junctions -B x.bam -o x.bed [-a 8] [-m 70] [-M 500000] [--isStranded -s rf|fr | --strandFromXS]
     python -m spliser_b200.cli processBam -B x.bam -o out [process's -A -t -c -g -m --isStranded -s --beta2Cryptic]
                                           [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
+    python -m spliser_b200.cli combineBam -S samples.tsv -o out [-A genes.gff] [-t gene] [-g gene] [--isStranded -s rf|fr]
+                                          [--beta2Cryptic] [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
+                                          [--shallow [-m 0] [-r 10] [-e 0.0]] [--gpus N]
 `junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
 `junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.  --strandFromXS
 takes the junction strands from the aligner's XS tag, as regtools does for unstranded libraries; processBam still counts
-with --isStranded -s.
+with --isStranded -s.  `combineBam` is `processBam` for every sample of a samples file (writing its column 2) followed by
+`combine` (`combineShallow` with --shallow), with every BAM read once: the records stay in GPU memory for the re-count.
 
 What stays in Python is what the reference does in text: BED12 parsing and its filters (S:255-288), the
 annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) and the lock-step merge of
@@ -22,6 +26,7 @@ annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) an
 from __future__ import annotations
 
 import argparse
+import functools
 import sys
 import timeit
 
@@ -162,20 +167,29 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
         if q is None:                           # S:283, as in process
             raise AttributeError("'NoneType' object has no attribute 'getLeftPos'")
         bounds = (q.left, q.right)
+    own = ctx is None
+    ctx = ctx or api.Context(0)
+    try:
+        extract = functools.partial(ctx.process_bam_extract, inBAM)
+        _process_bam_sample(extract, inBAM, outputPath + ".SpliSER.tsv", annotation, bounds, qChrom, maxIntronSize, isStranded,
+                            strandedType, isbeta2Cryptic, minAnchor, minIntron, maxIntron, strandFromXS)
+    finally:
+        if own:
+            ctx.close()
+
+
+def _process_bam_sample(extract, inBAM, tsv_path, annotation, bounds, qChrom, maxIntronSize, isStranded, strandedType, isbeta2Cryptic,
+                        minAnchor, minIntron, maxIntron, strandFromXS):
+    """processBam after the annotation load.  extract(chrom_names, flags, min_anchor, min_intron, max_intron, qchrom=, gene_bounds=,
+    window_max_intron=) answers like Context.process_bam_extract of this BAM (or DeviceSample.process_extract of it loaded)."""
     chroms = list(annotation.chrom_index) if annotation is not None else []
     known = set(chroms)
     chroms += [c for c in api.bam_reference_names(inBAM) if c not in known]
     flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic) | (api.FLAG_XS_STRAND if strandFromXS else 0)
-    own = ctx is None
-    ctx = ctx or api.Context(0)
-    try:
-        junc, table = ctx.process_bam_extract(inBAM, chroms, flags, minAnchor, minIntron, maxIntron, qchrom=qChrom, gene_bounds=bounds,
-                                              window_max_intron=int(maxIntronSize))
-    finally:
-        if own:
-            ctx.close()
+    junc, table = extract(chroms, flags, minAnchor, minIntron, maxIntron, qchrom=qChrom, gene_bounds=bounds,
+                          window_max_intron=int(maxIntronSize))
     print("Sites:\t\t\t" + str(len(table)))
-    write_process_tsv(outputPath + ".SpliSER.tsv", chroms, table, _strand_column(junc), annotation=annotation, is_stranded=isStranded,
+    write_process_tsv(tsv_path, chroms, table, _strand_column(junc), annotation=annotation, is_stranded=isStranded,
                       beta2_cryptic=isbeta2Cryptic)
 
 
@@ -220,8 +234,9 @@ def _chrom_order(runs_per_file):
     return stack[1:]
 
 
-def _recount_sample(ctx, cm, k, regions, bam_path, flags, records_by_bam):
-    """Every S:903 call of sample k in one spl_recount call; returns False when the sample has no gaps."""
+def _recount_sample(ctx, cm, k, regions, recount):
+    """Every S:903 call of sample k in one recount(ctx, k, chrom_names, gaps) -> (beta1, beta2simple) call (one spl_recount);
+    returns False when the sample has no gaps."""
     gaps = cm.gaps(k)
     if not len(gaps):
         return False
@@ -231,12 +246,63 @@ def _recount_sample(ctx, cm, k, regions, bam_path, flags, records_by_bam):
     remap = np.full(len(regions), -1, dtype=np.int32)
     remap[local] = np.arange(len(local), dtype=np.int32)
     gaps.chrom = np.ascontiguousarray(remap[gaps.chrom])
-    if records_by_bam is not None:
-        b1, b2 = ctx.recount_records(records_by_bam(bam_path, names), len(names), gaps, flags)
-    else:
-        b1, b2 = ctx.recount_bam(bam_path, names, gaps, flags)
+    b1, b2 = recount(ctx, k, names, gaps)
     cm.set_recount(k, b1, b2)
     return True
+
+
+def _read_samples_file(samplesFile, shallow):
+    """(titles, tsv paths, BAM paths) of a samples file: a line without exactly three columns raises in `combine` and is
+    skipped by `combineShallow` (S:930-935)."""
+    titles, bed_paths, bam_paths = [], [], []
+    with open(samplesFile) as fh:
+        for line in fh:
+            values = line.split("\t")
+            if len(values) == 3:
+                titles.append(values[0]); bed_paths.append(values[1]); bam_paths.append(values[2].rstrip())
+            elif not shallow:
+                print(str(titles), str(bed_paths), str(bam_paths))
+                raise Exception("Samples File contains lines that do not have exactly 3 tab-separated columns")
+    return titles, bed_paths, bam_paths
+
+
+def _on_ranks(n_ranks, work):
+    """work(rank) for every rank, each on a host thread of its own (the calling thread when there is one rank)."""
+    if n_ranks == 1:
+        work(0)
+        return
+    from concurrent.futures import ThreadPoolExecutor
+    with ThreadPoolExecutor(max_workers=n_ranks) as pool:
+        list(pool.map(work, range(n_ranks)))
+
+
+def _merge_recount_write(titles, tsv_paths, outputPath, qGene, isStranded, isbeta2Cryptic, shallow, n_ranks, rank_ctx, recount):
+    """The merge of `combine` (or combineShallow's, shallow = (minSamples, minReads, minSSE)) over the sample tables in
+    samples-file order, the re-count of every sample's gaps, the .combined.tsv.  The re-count shards by sample: rank r takes
+    dist.samples_of(r, n_ranks, n) on a host thread of its own (the calling thread when n_ranks == 1) with the context
+    rank_ctx(r), asked for once the rank meets its first sample with gaps; recount(ctx, k, chrom_names, gaps) -> (beta1,
+    beta2simple) counts sample k."""
+    n = len(titles)
+    with CombineMerge() as cm:
+        cm.add_samples(titles, tsv_paths)
+        regions = cm.region_names()
+        order = _chrom_order([[regions[r] for r in cm.sample_runs(k)] for k in range(n)])
+        region_id = {name: i for i, name in enumerate(regions)}
+        if shallow is None:
+            cm.merge([region_id[name] for name in order], qGene, isStranded)
+        else:
+            cm.merge_shallow([region_id[name] for name in order], qGene, isStranded, *shallow)
+
+        def rank_work(rank):
+            ctx = None
+            for k in samples_of(rank, n_ranks, n):
+                if cm.n_gaps(k):
+                    ctx = ctx or rank_ctx(rank)
+                    _recount_sample(ctx, cm, k, regions, recount)
+        _on_ranks(n_ranks, rank_work)
+        cm.write(outputPath + ".combined.tsv", isbeta2Cryptic)
+        filled = cm.n_filled()
+    print("Filled in Beta read counts for {} Sites not detected in some samples".format(filled))
 
 
 def combineShallow(samplesFile, outputPath, qGene="All", isStranded=False, minSamples=0, minReads=10, minSSE=0.0, strandedType=None,
@@ -265,58 +331,85 @@ def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType
     nothing but its own BAM and gap list, so the host only collects the count arrays.  `ctx` (one existing context) takes
     precedence; `context_factory(device)` replaces api.Context (tests)."""
     print("Combining samples...")
-    titles, bed_paths, bam_paths = [], [], []
-    with open(samplesFile) as fh:
-        for line in fh:
-            values = line.split("\t")
-            if len(values) == 3:
-                titles.append(values[0]); bed_paths.append(values[1]); bam_paths.append(values[2].rstrip())
-            elif _shallow is None:
-                print(str(titles), str(bed_paths), str(bam_paths))
-                raise Exception("Samples File contains lines that do not have exactly 3 tab-separated columns")
-    n = len(titles)
+    titles, bed_paths, bam_paths = _read_samples_file(samplesFile, _shallow is not None)
     flags = api.mode_flags(isStranded, strandedType, False, combine=True)
-    with CombineMerge() as cm:
-        cm.add_samples(titles, bed_paths)
-        regions = cm.region_names()
-        order = _chrom_order([[regions[r] for r in cm.sample_runs(k)] for k in range(n)])
-        region_id = {name: i for i, name in enumerate(regions)}
-        if _shallow is None:
-            cm.merge([region_id[name] for name in order], qGene, isStranded)
-        else:
-            cm.merge_shallow([region_id[name] for name in order], qGene, isStranded, *_shallow)
-        make = context_factory or api.Context
-        devs = [0] if not devices else list(devices)
-        if ctx is not None or len(devs) == 1:
-            own = None
-            try:
-                for k in range(n):
-                    if ctx is None and cm.n_gaps(k):
-                        ctx = own = make(devs[0])
-                    if cm.n_gaps(k):
-                        _recount_sample(ctx, cm, k, regions, bam_paths[k], flags, records_by_bam)
-            finally:
-                if own is not None:
-                    own.close()
-        else:
-            from concurrent.futures import ThreadPoolExecutor
 
-            def rank_work(rank):                    # one context per device, samples dealt round-robin
-                mine = [k for k in samples_of(rank, len(devs), n) if cm.n_gaps(k)]
-                if not mine:
-                    return 0
-                c = make(devs[rank])
-                try:
-                    for k in mine:
-                        _recount_sample(c, cm, k, regions, bam_paths[k], flags, records_by_bam)
-                finally:
-                    c.close()
-                return len(mine)
-            with ThreadPoolExecutor(max_workers=len(devs)) as pool:
-                list(pool.map(rank_work, range(len(devs))))
-        cm.write(outputPath + ".combined.tsv", isbeta2Cryptic)
-        filled = cm.n_filled()
-    print("Filled in Beta read counts for {} Sites not detected in some samples".format(filled))
+    def recount(c, k, names, gaps):
+        if records_by_bam is not None:
+            return c.recount_records(records_by_bam(bam_paths[k], names), len(names), gaps, flags)
+        return c.recount_bam(bam_paths[k], names, gaps, flags)
+    make = context_factory or api.Context
+    devs = [0] if not devices else list(devices)
+    n_ranks = 1 if ctx is not None else len(devs)
+    made = []
+
+    def rank_ctx(rank):                             # one context per device, made when its rank first needs it
+        if ctx is not None:
+            return ctx
+        made.append(make(devs[rank]))
+        return made[-1]
+    try:
+        _merge_recount_write(titles, bed_paths, outputPath, qGene, isStranded, isbeta2Cryptic, _shallow, n_ranks, rank_ctx, recount)
+    finally:
+        for c in made:
+            c.close()
+
+
+def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene="All", isStranded=False, strandedType=None,
+               isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False, shallow=False, minSamples=0,
+               minReads=10, minSSE=0.0, devices=None, context_factory=None):
+    """`processBam` for every sample of a samples file, then `combine` (or, with shallow, `combineShallow -m -r -e`) over them,
+    reading every BAM once.  Column 2 of the samples file is where the sample's .SpliSER.tsv is written: the file `processBam -B
+    <column 3>` writes with the same -A / --isStranded -s / --beta2Cryptic / --minAnchor --minIntron --maxIntron / --strandFromXS
+    and without -c / -g.  The .combined.tsv is the one `combine -g qGene` (`combineShallow`) writes from those files.
+
+    One context per device in `devices` (context_factory(device) replaces api.Context), each on a host thread of its own with the
+    samples dist.samples_of(rank, n_devices, n_samples) in both GPU phases: a sample is loaded into its rank's GPU memory
+    (Context.load_bam), its table extracted and counted from there, and after the merge its gaps are re-counted from there.  A
+    sample the device cannot hold (SampleMemoryError) takes the path route -- process_bam_extract, then recount_bam -- with the
+    same output."""
+    print("Combining samples from their BAMs...")
+    titles, tsv_paths, bam_paths = _read_samples_file(samplesFile, shallow)
+    n = len(titles)
+    annotation = load_annotation(annotationFile, "All") if annotationFile is not None else None
+    make = context_factory or api.Context
+    devs = [0] if not devices else list(devices)
+    n_ranks = len(devs)
+    ctxs = [None] * n_ranks
+    resident = [None] * n                           # DeviceSample, or None: the path route
+    flags = api.mode_flags(isStranded, strandedType, False, combine=True)
+
+    def process_rank(rank):
+        mine = samples_of(rank, n_ranks, n)
+        if not mine:
+            return
+        ctxs[rank] = c = make(devs[rank])
+        for k in mine:
+            try:
+                resident[k] = c.load_bam(bam_paths[k], xs=strandFromXS)
+                extract = resident[k].process_extract
+            except api.SampleMemoryError:
+                extract = functools.partial(c.process_bam_extract, bam_paths[k])
+            _process_bam_sample(extract, bam_paths[k], tsv_paths[k], annotation, None, "All", 0, isStranded, strandedType,
+                                isbeta2Cryptic, minAnchor, minIntron, maxIntron, strandFromXS)
+
+    def recount(c, k, names, gaps):
+        s, resident[k] = resident[k], None
+        if s is None:
+            return c.recount_bam(bam_paths[k], names, gaps, flags)
+        with s:
+            return s.recount(names, gaps, flags)
+    try:
+        _on_ranks(n_ranks, process_rank)
+        _merge_recount_write(titles, tsv_paths, outputPath, qGene, isStranded, isbeta2Cryptic,
+                             (minSamples, minReads, minSSE) if shallow else None, n_ranks, lambda rank: ctxs[rank], recount)
+    finally:
+        for s in resident:
+            if s is not None:
+                s.close()
+        for c in ctxs:
+            if c is not None:
+                c.close()
 
 
 # ------------------------------------------------------------------------------------------------ main
@@ -384,13 +477,36 @@ def main(argv=None):
     pb.add_argument("--maxIntron", dest="maxIntron", default=500000, type=int)
     pb.add_argument("--strandFromXS", dest="strandFromXS", default=argparse.SUPPRESS, action="store_true",
                     help="junction strands from the aligner's XS tag; the count still follows --isStranded -s")
+    cb = sub.add_parser("combineBam", help="processBam for every sample, then combine, reading every BAM once")
+    cb.add_argument("-S", "--samplesFile", dest="samplesFile", required=True,
+                    help="title <TAB> .SpliSER.tsv to write <TAB> BAM, one sample per line (combine's samples file)")
+    cb.add_argument("-o", "--outputPath", dest="outputPath", required=True)
+    cb.add_argument("-A", "--annotationFile", dest="annotationFile", required=False)
+    cb.add_argument("-t", "--annotationType", dest="aType", nargs="?", default="gene", type=str)
+    cb.add_argument("-g", "--gene", dest="qGene", nargs="?", default="All", type=str)
+    cb.add_argument("--isStranded", dest="isStranded", default=False, action="store_true")
+    cb.add_argument("-s", "--strandedType", dest="strandedType", nargs="?", type=str)
+    cb.add_argument("--beta2Cryptic", dest="isbeta2Cryptic", default=False, action="store_true")
+    cb.add_argument("--minAnchor", dest="minAnchor", default=8, type=int)
+    cb.add_argument("--minIntron", dest="minIntron", default=70, type=int)
+    cb.add_argument("--maxIntron", dest="maxIntron", default=500000, type=int)
+    cb.add_argument("--strandFromXS", dest="strandFromXS", default=False, action="store_true",
+                    help="junction strands from the aligner's XS tag; the count still follows --isStranded -s")
+    cb.add_argument("--shallow", dest="shallow", default=False, action="store_true", help="merge as combineShallow")
+    cb.add_argument("-m", "--minSamples", dest="minSamples", nargs="?", default=0, type=int)
+    cb.add_argument("-r", "--minReads", dest="minReads", nargs="?", default=10, type=int)
+    cb.add_argument("-e", "--minSSE", dest="minSSE", nargs="?", default=0.00, type=float)
+    cb.add_argument("--gpus", dest="n_gpus", nargs="?", default=1, type=int,
+                    help="hold and count the samples on this many GPUs (sharded by sample)")
     kwargs = vars(parser.parse_args(argv))          # --strandFromXS is only passed on when given (SUPPRESS)
     command = kwargs.pop("command")
-    if command in ("combine", "combineShallow"):
+    if command in ("combine", "combineShallow", "combineBam"):
         kwargs["devices"] = list(range(max(1, kwargs.pop("n_gpus") or 1)))
     if command in ("process", "processBam") and kwargs.get("qGene") != "All" and (kwargs.get("annotationFile") is None or kwargs.get("maxIntronSize") is None):
         parser.error("--gene requires --annotationFile and --maxIntronSize")                      # S:1350-1353
-    elif command in ("process", "combine", "combineShallow", "junctions", "processBam") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
+    elif command == "combineBam" and kwargs.get("qGene") != "All" and kwargs.get("annotationFile") is None:
+        parser.error("--gene requires --annotationFile (the Gene column comes from it)")
+    elif command in ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
         parser.error("--isStranded requires parameter --strandedType/-s as fr or rf")            # S:1354-1355
     elif command == "junctions" and kwargs.get("strandFromXS") and kwargs.get("isStranded"):
         parser.error("--strandFromXS and --isStranded name two strand sources for the junction table")
@@ -404,8 +520,10 @@ def main(argv=None):
         junctions(**kwargs)
     elif command == "processBam":
         processBam(**kwargs)
+    elif command == "combineBam":
+        combineBam(**kwargs)
     else:
-        parser.error("command must be process, combine, combineShallow, junctions or processBam (output is unchanged Python in the reference)")
+        parser.error("command must be process, combine, combineShallow, junctions, processBam or combineBam (output is unchanged Python in the reference)")
     print("Total runtime (s): \t" + str(timeit.default_timer() - start))
 
 

@@ -68,8 +68,22 @@ bool find_cg(const uint8_t* p, const uint8_t* end, const uint8_t*& data, uint32_
 
 }  // namespace
 
-std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out, bool want_xs) {
+std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, int32_t n_chrom, const char* const* chrom_names) {
+    std::unordered_map<std::string, int32_t> names;
+    for (int32_t c = 0; c < n_chrom; ++c)
+        if (chrom_names && chrom_names[c]) names.emplace(chrom_names[c], c);
+    std::vector<int32_t> refmap(ref_names.size(), -1);
+    for (size_t r = 0; r < ref_names.size(); ++r) {
+        auto it = names.find(ref_names[r]);
+        if (it != names.end()) refmap[r] = it->second;
+    }
+    return refmap;
+}
+
+std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out, bool want_xs,
+                     std::vector<std::string>* header_order) {
     out = BamRecords();
+    if (header_order) header_order->clear();
     const int fd = open(path, O_RDONLY);
     if (fd < 0) return std::string("cannot open BAM file ") + path;
     struct stat st;
@@ -157,18 +171,20 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             const uint8_t* q = p + 8 + l_text;
             const int32_t n_ref = rdi32(q);
             q += 4;
-            std::unordered_map<std::string, int32_t> names;
-            for (int32_t c = 0; c < n_chrom; ++c)
-                if (chrom_names && chrom_names[c]) names.emplace(chrom_names[c], c);
-            refmap.assign((size_t)std::max(n_ref, 0), -1);
+            std::vector<std::string> ref_names;
             for (int32_t r = 0; r < n_ref; ++r) {
                 if (q + 4 > end) return "truncated BAM reference list";
                 const int32_t l_name = rdi32(q);
                 if (l_name < 1 || q + 4 + l_name + 4 > end) return "truncated BAM reference list";
-                std::string nm((const char*)q + 4, (size_t)l_name - 1);
-                auto it = names.find(nm);
-                if (it != names.end()) refmap[(size_t)r] = it->second;
+                ref_names.emplace_back((const char*)q + 4, (size_t)l_name - 1);
                 q += 4 + l_name + 4;
+            }
+            if (header_order) {
+                refmap.resize(ref_names.size());
+                for (size_t r = 0; r < refmap.size(); ++r) refmap[r] = (int32_t)r;
+                *header_order = std::move(ref_names);
+            } else {
+                refmap = map_references(ref_names, n_chrom, chrom_names);
             }
             p = q;
             header_done = true;
@@ -277,20 +293,16 @@ std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const cha
     n_ref = rdi32(hb.data() + q);
     q += 4;
     if (n_ref < 0) return "corrupt BAM header (n_ref < 0)";
-    std::unordered_map<std::string, int32_t> names;
-    for (int32_t c = 0; c < n_chrom; ++c)
-        if (chrom_names && chrom_names[c]) names.emplace(chrom_names[c], c);
-    refmap.assign((size_t)n_ref, -1);
+    std::vector<std::string> names;
     for (int32_t r = 0; r < n_ref; ++r) {
         if (!need(q + 4)) return "truncated BAM reference list";
         const int32_t l_name = rdi32(hb.data() + q);
         if (l_name < 1 || !need(q + 4 + (size_t)l_name + 4)) return "truncated BAM reference list";
-        std::string nm((const char*)hb.data() + q + 4, (size_t)l_name - 1);
-        auto it = names.find(nm);
-        if (it != names.end()) refmap[(size_t)r] = it->second;
-        if (ref_names) ref_names->push_back(std::move(nm));
+        names.emplace_back((const char*)hb.data() + q + 4, (size_t)l_name - 1);
         q += 4 + (size_t)l_name + 4;
     }
+    refmap = map_references(names, n_chrom, chrom_names);
+    if (ref_names) *ref_names = std::move(names);
     first_record = q;
     return "";
 }

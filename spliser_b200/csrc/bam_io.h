@@ -23,9 +23,14 @@ struct BamRecords {
     spl_records_view view() const;
 };
 
-// Returns "" or an error message.  chrom_names maps BAM reference names to caller indices.
+// The caller's chromosome index of every header reference: the index of the same name in chrom_names (the first one when a
+// name repeats there), else -1.  Every reader and the device-resident samples map references with this one rule.
+std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, int32_t n_chrom, const char* const* chrom_names);
+
+// Returns "" or an error message.  chrom_names maps BAM reference names to caller indices.  header_order != NULL: chrom_names
+// is ignored, every record keeps its header reference index (seg_chrom) and *header_order receives the reference names.
 std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out,
-                     bool want_xs = false);
+                     bool want_xs = false, std::vector<std::string>* header_order = nullptr);
 
 std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                       const spl_records_view* rec, int n_threads, bool with_seq = false,

@@ -1320,9 +1320,10 @@ int load_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int6
 
 // BAM file -> record arrays on the device.  SPL_OK: ctx->dev_rec / `cnt` are filled and `view` describes them
 // (array pointers NULL, ctx->rec_on_device must be set by the caller around the load).  *fallback = true: use the host reader.
-// want_xs: ctx->dev_rec.xs receives the XS strand of every record as well.
+// want_xs: ctx->dev_rec.xs receives the XS strand of every record as well.  header_order != NULL: chrom_names is ignored, every
+// record keeps its header reference index (no reference is dropped) and *header_order receives the reference names.
 int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const char* const* chrom_names, BamGpuCounts& cnt,
-                      spl_records_view& view, bool* fallback, bool want_xs = false) {
+                      spl_records_view& view, bool* fallback, bool want_xs = false, std::vector<std::string>* header_order = nullptr) {
     *fallback = false;
     if (const char* f = std::getenv("SPLISER_HOST_BAM")) if (f[0] == '1') { *fallback = true; return SPL_OK; }
     const int fd = open(path, O_RDONLY);
@@ -1377,8 +1378,10 @@ int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const cha
     std::vector<int32_t> refmap;
     uint64_t total_u = 0, first_record = 0;
     int32_t n_ref = 0;
-    std::string e = bam_scan((const uint8_t*)ctx->h_file, fsz, n_chrom, chrom_names, members, total_u, first_record, n_ref, refmap);
+    std::string e = bam_scan((const uint8_t*)ctx->h_file, fsz, n_chrom, chrom_names, members, total_u, first_record, n_ref, refmap,
+                             header_order);
     if (!e.empty()) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_IO, "%s", e.c_str()); }
+    if (header_order) for (int32_t r = 0; r < n_ref; ++r) refmap[(size_t)r] = r;
     const int rc = bam_gpu_ingest(ctx->bgm, (const uint8_t*)ctx->h_file, fsz, members, total_u, first_record, n_ref, refmap, ctx->stream,
                                   uploaded, want_xs, ctx->dev_rec, cnt, e);
     if (rc != BAMGPU_OK) cudaStreamSynchronize(ctx->stream);           // the pinned image may be re-used by the fallback / next call
@@ -1971,6 +1974,198 @@ int spl_recount(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
     ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
     ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
     return rc;
+}
+
+// ---- device-resident samples ----------------------------------------------------------------------------------------------
+struct spl_sample {
+    const spl_ctx* ctx = nullptr;         // the context that loaded it (compared, never dereferenced)
+    int device = 0;
+    void* mem = nullptr;                  // the one device allocation that holds every column
+    size_t bytes = 0;
+    DevRecordArrays rec{};                // pos / flag / cig_off / cigar (/ xs) inside mem; no per-record chromosome
+    int64_t n_rec = 0, n_cigar = 0;
+    std::vector<std::string> ref_names;   // the header's references, in header order
+    std::vector<int32_t> seg_ref;         // header reference index of every segment
+    std::vector<int64_t> seg_off;         // [n_seg + 1]
+};
+
+namespace {
+std::atomic<int64_t> g_resident_bytes(0);          // what the samples of this process hold (SPLISER_SAMPLE_BUDGET_MB caps it)
+constexpr size_t SAMPLE_HEADROOM = (size_t)1 << 30;
+
+// Takes `bytes` of device memory for a sample under the residency policy of spl_sample_load_bam; SPL_ERR_NOMEM holds nothing.
+int sample_reserve(spl_ctx* ctx, size_t bytes, void** p) {
+    *p = nullptr;
+    const int64_t b = (int64_t)bytes;
+    const int64_t held = g_resident_bytes.fetch_add(b) + b;
+    auto refuse = [&](int code, const char* why) {
+        g_resident_bytes -= b;
+        return ctx->fail(code, "a resident sample of %zu bytes is not held: %s", bytes, why);
+    };
+    if (const char* cap = std::getenv("SPLISER_SAMPLE_BUDGET_MB"))
+        if (held > std::max<int64_t>(0, atoll(cap)) * ((int64_t)1 << 20)) return refuse(SPL_ERR_NOMEM, "over SPLISER_SAMPLE_BUDGET_MB");
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); return refuse(SPL_ERR_CUDA, "cudaMemGetInfo failed"); }
+    if (free_b < 2 * bytes + SAMPLE_HEADROOM) return refuse(SPL_ERR_NOMEM, "it would leave the context less free device memory than its headroom");
+    if (cudaMalloc(p, bytes) != cudaSuccess) { cudaGetLastError(); *p = nullptr; return refuse(SPL_ERR_NOMEM, "cudaMalloc failed"); }
+    return SPL_OK;
+}
+
+int check_sample(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names) {
+    if (!s) return ctx->fail(SPL_ERR_ARG, "sample is NULL");
+    if (s->ctx != ctx) return ctx->fail(SPL_ERR_ARG, "the sample was loaded by another context");
+    if (n_chrom < 0 || (n_chrom > 0 && !chrom_names)) return ctx->fail(SPL_ERR_ARG, "chrom_names is NULL");
+    for (int32_t c = 0; c < n_chrom; ++c) if (!chrom_names[c]) return ctx->fail(SPL_ERR_ARG, "chromosome name %d is NULL", c);
+    return SPL_OK;
+}
+
+// The sample's segments under the caller's chromosome list, by the rule the readers map references with (map_references): a
+// reference that is not in the list becomes -1 and its records are skipped.  `seg_chrom` must outlive the view.
+spl_records_view sample_view(const spl_sample* s, int32_t n_chrom, const char* const* chrom_names, std::vector<int32_t>& seg_chrom) {
+    const std::vector<int32_t> refmap = map_references(s->ref_names, n_chrom, chrom_names);
+    seg_chrom.resize(s->seg_ref.size());
+    for (size_t k = 0; k < seg_chrom.size(); ++k) seg_chrom[k] = refmap[(size_t)s->seg_ref[k]];
+    spl_records_view v{};
+    v.n_rec = s->n_rec; v.n_cigar = s->n_cigar;
+    v.n_seg = (int32_t)seg_chrom.size(); v.seg_chrom = seg_chrom.data(); v.seg_off = s->seg_off.data();
+    return v;
+}
+
+// ctx->dev_rec is the sample's columns for the duration of one call (records on the device, no upload)
+struct SampleBinding {
+    spl_ctx* ctx;
+    DevRecordArrays saved;
+    bool saved_dev;
+    SampleBinding(spl_ctx* c, const spl_sample* s) : ctx(c), saved(c->dev_rec), saved_dev(c->rec_on_device) {
+        ctx->dev_rec = s->rec;
+        ctx->rec_on_device = true;
+    }
+    ~SampleBinding() { ctx->dev_rec = saved; ctx->rec_on_device = saved_dev; }
+};
+}  // namespace
+
+int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_sample** out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
+    if (flags & ~SPL_FLAG_XS_STRAND) return ctx->fail(SPL_ERR_ARG, "spl_sample_load_bam takes SPL_FLAG_XS_STRAND only");
+    const bool want_xs = (flags & SPL_FLAG_XS_STRAND) != 0;
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    reset_stats(ctx);
+    std::unique_ptr<spl_sample> s(new (std::nothrow) spl_sample());
+    if (!s) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
+    s->ctx = ctx;
+    s->device = ctx->device;
+    // ingest exactly as spl_process chooses, every reference kept in header order
+    BamGpuCounts cnt;
+    spl_records_view dv{};
+    bool fallback = false;
+    int rc = ingest_bam_device(ctx, bam_path, 0, nullptr, cnt, dv, &fallback, want_xs, &s->ref_names);
+    if (rc) return rc;
+    BamRecords recs;
+    if (fallback) {
+        std::string e = read_bam(bam_path, 0, nullptr, ctx->n_threads, recs, want_xs, &s->ref_names);
+        if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
+        s->n_rec = (int64_t)recs.pos.size(); s->n_cigar = (int64_t)recs.cigar.size();
+        s->seg_ref = recs.seg_chrom; s->seg_off = recs.seg_off;
+    } else {
+        s->n_rec = (int64_t)cnt.n_rec; s->n_cigar = (int64_t)cnt.n_cigar;
+        s->seg_ref = cnt.seg_chrom; s->seg_off = cnt.seg_off;
+    }
+    if (s->seg_off.empty()) s->seg_off.assign(1, 0);
+    const double t1 = now_ms();
+    const size_t n = (size_t)s->n_rec, nc = (size_t)s->n_cigar;
+    Carver c;
+    const size_t o_pos = c.take<int32_t>(n + 4), o_flag = c.take<uint16_t>(n + 4), o_off = c.take<uint32_t>(n + 4),
+                 o_cig = c.take<uint32_t>(nc + 4), o_xs = want_xs ? c.take<uint8_t>(n + 4) : 0;
+    rc = sample_reserve(ctx, c.off, &s->mem);
+    if (rc) return rc;
+    s->bytes = c.off;
+    char* m = (char*)s->mem;
+    s->rec.pos = (int32_t*)(m + o_pos); s->rec.flag = (uint16_t*)(m + o_flag);
+    s->rec.cig_off = (uint32_t*)(m + o_off); s->rec.cigar = (uint32_t*)(m + o_cig);
+    s->rec.xs = want_xs ? (uint8_t*)(m + o_xs) : nullptr;
+    // device ingest: one copy out of the context's scratch (which the next ingest re-uses); host reader: the upload itself
+    const cudaMemcpyKind kind = fallback ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    const DevRecordArrays& src = ctx->dev_rec;
+    cudaError_t ce = cudaSuccess;
+    auto copy = [&](void* dst, const void* from, size_t bytes) {
+        if (bytes && ce == cudaSuccess) ce = cudaMemcpyAsync(dst, from, bytes, kind, ctx->stream);
+    };
+    if (n) {
+        copy(s->rec.pos, fallback ? (const void*)recs.pos.data() : src.pos, n * 4);
+        copy(s->rec.flag, fallback ? (const void*)recs.flag.data() : src.flag, n * 2);
+        copy(s->rec.cig_off, fallback ? (const void*)recs.cig_off.data() : src.cig_off, (n + 1) * 4);
+        copy(s->rec.cigar, fallback ? (const void*)recs.cigar.data() : src.cigar, nc * 4);
+        if (want_xs) copy(s->rec.xs, fallback ? (const void*)recs.xs.data() : src.xs, n);
+    } else if (cudaMemsetAsync(s->rec.cig_off, 0, 4, ctx->stream) != cudaSuccess) {
+        ce = cudaGetLastError();
+    }
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
+    if (ce != cudaSuccess) {
+        cudaStreamSynchronize(ctx->stream);
+        cudaGetLastError();
+        spl_sample_free(s.release());
+        return ctx->fail(SPL_ERR_CUDA, "copy of the sample's records failed: %s", cudaGetErrorString(ce));
+    }
+    ctx->stats[SPL_STAT_H2D_BYTES] = fallback ? (double)(n * 10 + 4 + nc * 4 + (want_xs ? n : 0)) : cnt.h2d_bytes;
+    ctx->stats[SPL_STAT_BAM_DEVICE] = fallback ? 0.0 : 1.0;
+    ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    *out = s.release();
+    return SPL_OK;
+}
+
+int spl_sample_process_extract(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
+                               const spl_extract_opts* opts, uint32_t flags, spl_junctions** rows_out, spl_result** out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out || !rows_out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
+    *out = nullptr; *rows_out = nullptr;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!opts) return ctx->fail(SPL_ERR_ARG, "opts is NULL");
+    int rc = check_sample(ctx, s, n_chrom, chrom_names);
+    if (rc) return rc;
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    std::vector<int32_t> seg_chrom;
+    const spl_records_view dv = sample_view(s, n_chrom, chrom_names, seg_chrom);
+    {
+        SampleBinding bind(ctx, s);
+        rc = extract_and_count(ctx, &dv, nullptr, n_chrom, chrom_names, opts, flags, rows_out, out);
+    }
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
+}
+
+int spl_sample_recount(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names, int64_t n_sites,
+                       const int32_t* s_chrom, const int32_t* s_pos, const uint8_t* s_strand, const int64_t* p_off, const int32_t* p_pos,
+                       const int64_t* c_off, const int32_t* c_pos, uint32_t flags, int64_t* beta1_out, int64_t* beta2simple_out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    int rc = check_sample(ctx, s, n_chrom, chrom_names);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    std::vector<int32_t> seg_chrom;
+    const spl_records_view dv = sample_view(s, n_chrom, chrom_names, seg_chrom);
+    SampleBinding bind(ctx, s);
+    return spl_recount_records(ctx, &dv, n_chrom, n_sites, s_chrom, s_pos, s_strand, p_off, p_pos, c_off, c_pos, flags, beta1_out,
+                               beta2simple_out);
+}
+
+int64_t spl_sample_n_records(const spl_sample* s) { return s ? s->n_rec : 0; }
+int64_t spl_sample_device_bytes(const spl_sample* s) { return s ? (int64_t)s->bytes : 0; }
+
+void spl_sample_free(spl_sample* s) {
+    if (!s) return;
+    if (s->mem) {
+        cudaSetDevice(s->device);
+        cudaFree(s->mem);
+        g_resident_bytes -= (int64_t)s->bytes;
+    }
+    delete s;
 }
 
 int spl_resident_load(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int64_t n_junc, const int32_t* j_chrom,
