@@ -283,6 +283,54 @@ int64_t spl_sample_n_records(const spl_sample* s);
 int64_t spl_sample_device_bytes(const spl_sample* s);
 void    spl_sample_free(spl_sample* s);
 
+/* ---- library strandedness ------------------------------------------------------------------------------------------------
+ * Which protocol (`--isStranded -s fr`, `-s rf`, or unstranded) a library was made with, from its records: one vote per record.
+ *   - records: those an ingest keeps -- mapped to a caller chromosome, with at least one CIGAR operator; no FLAG filter (as
+ *     checkBam, S:422);
+ *   - read strand under fr (check_strand, S:374-406): first = FLAG & 64 or !(FLAG & 1), rev = FLAG & 16, strand =
+ *     first ? (rev ? '-' : '+') : (rev ? '+' : '-'); under rf it is always the opposite, so the fr strand alone is compared;
+ *   - reference strand, annotation source (genes != NULL): the record spans the 1-based bases POS .. POS + L - 1, L = the sum of
+ *     its M D N = X lengths, 1 when that sum is 0; a gene (left = GFF start - 1, right = GFF end) overlaps it when
+ *     POS - 1 < right and POS - 1 + L > left.  Only genes whose strand byte is '+' or '-' count, and a gene with an empty span
+ *     (right <= left, GFF end < start) has none to give.  The reference strand is the common strand of the overlapping genes;
+ *     no gene, or genes of both strands: no vote;
+ *   - reference strand, XS source (genes == NULL): the record's XS strand (SPL_FLAG_XS_STRAND's rule); '?' is no vote;
+ *   - counts[SPL_VOTE_AGREE_FR] = votes whose fr read strand equals the reference strand, counts[SPL_VOTE_OPPOSITE] = the
+ *     others, counts[SPL_VOTE_NONE] = records without a vote.
+ * The verdict is the caller's (spliser_b200.api.library_type).
+ *
+ * spl_gene_strands: the genes of caller chromosome c (c < n_chrom) are [chrom_off[c], chrom_off[c + 1]) in any order; caller
+ * chromosomes from n_chrom on have none (n_chrom may be below the call's n_chrom).  The call indexes them on the host
+ * (O(G log G): the elementary intervals between gene boundaries with a 2-bit strand mask each, and a sparse table for range-OR)
+ * and uploads the index; a record's query is then two binary searches and two table reads, however many genes overlap it.
+ *
+ * spl_infer_strand_records takes host records (with the XS source xs[n_rec] is required, e.g. spl_records_xs); spl_infer_strand
+ * ingests the BAM as spl_extract_junctions does (the XS column only for the XS source); spl_sample_infer_strand votes over a
+ * resident sample (references mapped to chrom_names by name, as spl_sample_process_extract maps them) -- the XS source needs a
+ * sample loaded with SPL_FLAG_XS_STRAND, else SPL_ERR_ARG.  The records are never copied back; SPL_STAT_MS_STRAND_VOTES is the
+ * CUDA-event time of the vote kernel. */
+typedef struct spl_gene_strands {
+    int32_t n_chrom;
+    const int64_t* chrom_off;     /* [n_chrom + 1], chrom_off[0] == 0 */
+    const int32_t* left;          /* [chrom_off[n_chrom]] GFF start - 1 */
+    const int32_t* right;         /* GFF end */
+    const uint8_t* strand;        /* '+', '-'; any other byte: the gene is ignored */
+} spl_gene_strands;
+#define SPL_VOTE_AGREE_FR 0
+#define SPL_VOTE_OPPOSITE 1
+#define SPL_VOTE_NONE     2
+int spl_infer_strand_records(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom,
+                             const spl_gene_strands* genes, int64_t counts[3]);
+int spl_infer_strand(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names,
+                     const spl_gene_strands* genes, int64_t counts[3]);
+int spl_sample_infer_strand(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
+                            const spl_gene_strands* genes, int64_t counts[3]);
+/* Test hook (host only, no GPU): the index spl_infer_strand builds from `genes`, queried with the device's code: mask_out[i] =
+ * bit 0 '+', bit 1 '-' over the genes of caller chromosome chrom[i] (< n_chrom) that overlap the 0-based span
+ * [start[i], start[i] + len[i]).  Returns 0, or SPL_ERR_ARG with the reason in err. */
+int spl_debug_gene_strand_mask(int32_t n_chrom, const spl_gene_strands* genes, int64_t n, const int32_t* chrom, const int64_t* start,
+                               const int64_t* len, uint8_t* mask_out, char* err, int err_len);
+
 /* Reference names of a BAM header in header order (host only, no GPU): written NUL-terminated back to back into
  * names[0 .. cap) when *bytes (the space they need) <= cap; *n_ref and *bytes are always set. */
 int spl_bam_reference_names(const char* path, char* names, int64_t cap, int64_t* n_ref, int64_t* bytes, char* err, int err_len);
@@ -366,6 +414,7 @@ int spl_resident_fetch(spl_ctx* ctx, spl_result** out);
 #define SPL_STAT_MS_EXTRACT   28   /* junction extraction: CUDA-event ms of its kernels (anchor extents included)           */
 #define SPL_STAT_MS_EXTENTS   29   /* junction extraction: CUDA-event ms of the anchor-extent walk alone                    */
 #define SPL_STAT_N_JUNCTIONS  30   /* junction extraction: rows extracted (before the -c / -g filters of spl_process_bam_extract) */
+#define SPL_STAT_MS_STRAND_VOTES 31   /* spl_infer_strand*: CUDA-event ms of the vote kernel                                */
 int spl_last_stats(const spl_ctx* ctx, double* stats_out);
 
 /* ---- host text layer (no GPU): Gene column, .SpliSER.tsv writer, combine merge driver ------------

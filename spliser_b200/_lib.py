@@ -19,7 +19,7 @@ SPL_ERR_NOMEM = -4
 SPL_NSTATS = 32
 STAT_NAMES = ("ms_total", "ms_beta1", "ms_spliced", "ms_final", "n_mblocks_a", "n_mblocks_b", "n_junc_ops",
               "n_spliced", "n_sites", "n_edges", "n_aligned", "launches", "ms_expand", "ms_decode",
-              "h2d_bytes", "d2h_bytes", "ms_graph", "ms_upload", "ms_count", "n_distinct_junc", "n_simple_junc", "n_complex_junc", "graph_on_device", "bam_on_device", "n_parts", "ms_graph_dev", "graph_timed", "n_hot_items", "ms_extract", "ms_extents", "n_junctions", "r31")
+              "h2d_bytes", "d2h_bytes", "ms_graph", "ms_upload", "ms_count", "n_distinct_junc", "n_simple_junc", "n_complex_junc", "graph_on_device", "bam_on_device", "n_parts", "ms_graph_dev", "graph_timed", "n_hot_items", "ms_extract", "ms_extents", "n_junctions", "ms_strand_votes")
 
 c_i32p = C.POINTER(C.c_int32)
 c_i64p = C.POINTER(C.c_int64)
@@ -55,6 +55,10 @@ class StrTab(C.Structure):
 class ExtractOpts(C.Structure):
     _fields_ = [("min_anchor", C.c_int32), ("min_intron", C.c_int32), ("max_intron", C.c_int32), ("qchrom", C.c_char_p),
                 ("use_gene_window", C.c_int32), ("gene_left", C.c_int64), ("gene_right", C.c_int64), ("window_max_intron", C.c_int64)]
+
+
+class GeneStrandsView(C.Structure):
+    _fields_ = [("n_chrom", C.c_int32), ("chrom_off", c_i64p), ("left", c_i32p), ("right", c_i32p), ("strand", c_u8p)]
 
 
 class SiteColumns(C.Structure):
@@ -105,6 +109,11 @@ SIGNATURES = {
     "spl_sample_n_records": (C.c_int64, [C.c_void_p]),
     "spl_sample_device_bytes": (C.c_int64, [C.c_void_p]),
     "spl_sample_free": (None, [C.c_void_p]),
+    "spl_infer_strand_records": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), c_u8p, C.c_int32, C.POINTER(GeneStrandsView), c_i64p]),
+    "spl_infer_strand": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp, C.POINTER(GeneStrandsView), c_i64p]),
+    "spl_sample_infer_strand": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, c_strp, C.POINTER(GeneStrandsView), c_i64p]),
+    "spl_debug_gene_strand_mask": (C.c_int, [C.c_int32, C.POINTER(GeneStrandsView), C.c_int64, c_i32p, c_i64p, c_i64p, c_u8p,
+                                             C.c_char_p, C.c_int]),
     "spl_bam_reference_names": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int64, c_i64p, c_i64p, C.c_char_p, C.c_int]),
     "spl_write_junctions_bed": (C.c_int, [C.c_char_p, C.c_int64, c_i32p, c_i32p, c_i32p, c_i32p, c_i32p, c_i64p, c_u8p,
                                           C.POINTER(StrTab), C.c_char_p, C.c_int]),

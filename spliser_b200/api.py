@@ -469,6 +469,82 @@ class SampleMemoryError(SpliserError):
     """Context.load_bam refused to hold a sample on the device (SPL_ERR_NOMEM); the context stays usable."""
 
 
+@dataclass
+class StrandVotes:
+    """One vote per record on the library's protocol (include/spliser_b200.h, spl_gene_strands, states the rule): agree_fr =
+    records whose read strand under fr equals the reference strand, opposite = the others, no_vote = records without one."""
+    agree_fr: int
+    opposite: int
+    no_vote: int
+
+
+# library_type's thresholds: constants of the verdict, printed with it by every command that infers
+MIN_VOTES = 100
+FR_MIN, RF_MAX = 0.8, 0.2
+UNSTRANDED_RANGE = (0.35, 0.65)
+
+
+def library_type(votes: StrandVotes):
+    """The verdict on the votes: 'fr', 'rf', 'unstranded', or None (undecided).  With v = agree_fr + opposite and
+    f = agree_fr / v: fewer than MIN_VOTES votes is undecided; f >= 0.8 is fr, f <= 0.2 rf, 0.35 <= f <= 0.65 unstranded,
+    anything else undecided.  Compared in integers, so a boundary is exactly on its side."""
+    a, v = int(votes.agree_fr), int(votes.agree_fr) + int(votes.opposite)
+    if v < MIN_VOTES:
+        return None
+    if 5 * a >= 4 * v:
+        return "fr"
+    if 5 * a <= v:
+        return "rf"
+    if 20 * a >= 7 * v and 20 * a <= 13 * v:
+        return "unstranded"
+    return None
+
+
+class GeneStrands:
+    """The genes of an annotation over a caller's chromosome list (spl_gene_strands): genes of chromosome c are rows
+    chrom_off[c] .. chrom_off[c + 1] of left / right / strand ('+', '-', or 0 for any other strand text)."""
+
+    def __init__(self, chrom_off, left, right, strand):
+        self.chrom_off = np.ascontiguousarray(chrom_off, dtype=np.int64)
+        self.left = np.ascontiguousarray(left, dtype=np.int32)
+        self.right = np.ascontiguousarray(right, dtype=np.int32)
+        self.strand = np.ascontiguousarray(strand, dtype=np.uint8)
+        n = int(self.chrom_off[-1]) if len(self.chrom_off) else 0
+        if not len(self.chrom_off) or self.chrom_off[0] != 0 or not (len(self.left) == len(self.right) == len(self.strand) == n):
+            raise ValueError("gene arrays do not match chrom_off")
+
+    @property
+    def n_chrom(self):
+        return len(self.chrom_off) - 1
+
+    def view(self) -> L.GeneStrandsView:
+        v = L.GeneStrandsView()
+        v.n_chrom = self.n_chrom
+        v.chrom_off = _ptr(self.chrom_off, L.c_i64p)
+        v.left = _ptr(self.left, L.c_i32p)
+        v.right = _ptr(self.right, L.c_i32p)
+        v.strand = _ptr(self.strand, L.c_u8p)
+        return v
+
+
+def gene_strands(annotation, chrom_names) -> GeneStrands:
+    """The gene columns of an Annotation (genes.load_annotation) over chrom_names: a name takes the genes of the annotation's
+    chromosome of that name (its first index when the list repeats it, as records are mapped); a strand text other than
+    exactly '+' or '-' becomes 0 (ignored by the vote)."""
+    cols = annotation.columns
+    at = {c: i for i, c in enumerate(annotation.chrom_index)}
+    lut = np.array([ord(t) if t in ("+", "-") else 0 for t in cols.strand_texts] + [0], np.uint8)
+    rows, offs, seen = [], [0], set()
+    for c in chrom_names:
+        k = at.get(c) if c not in seen else None
+        seen.add(c)
+        if k is not None:
+            rows.append(np.arange(int(cols.chrom_off[k]), int(cols.chrom_off[k + 1]), dtype=np.int64))
+        offs.append(offs[-1] + (len(rows[-1]) if k is not None else 0))
+    sel = np.concatenate(rows) if rows else np.zeros(0, np.int64)
+    return GeneStrands(np.array(offs, np.int64), cols.left[sel], cols.right[sel], lut[cols.strand_id[sel]])
+
+
 def _names(chrom_names):
     return (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
 
@@ -499,6 +575,10 @@ class DeviceSample:
     def recount(self, chrom_names, gaps, flags: int):
         """Context.recount_bam of the loaded BAM: (beta1, beta2simple)."""
         return self._ctx._recount(self._ctx._lib.spl_sample_recount, self._h, chrom_names, gaps, flags)
+
+    def infer_strand(self, chrom_names, genes: "GeneStrands" = None) -> StrandVotes:
+        """Context.infer_strand_bam of the loaded BAM.  The XS source (genes=None) needs a sample loaded with xs=True."""
+        return self._ctx._infer(self._ctx._lib.spl_sample_infer_strand, self._h, chrom_names, genes)
 
     def close(self):
         h, self._h = getattr(self, "_h", None), None
@@ -684,6 +764,30 @@ class Context:
         hj, hr = C.c_void_p(), C.c_void_p()
         self._check(fn(self._h, source, len(chrom_names), names, C.byref(o), flags, C.byref(hj), C.byref(hr)), fn.__name__)
         return self._take_junctions(hj), self._take(hr)
+
+    # ---- library strandedness ------------------------------------------------------------------------
+    def infer_strand_records(self, records: Records, n_chrom: int, genes: GeneStrands = None) -> StrandVotes:
+        """The votes on the library's protocol (spl_gene_strands states the rule): the reference strand of a record from the
+        genes (gene_strands) that overlap it, or with genes=None from its XS tag (records.xs)."""
+        if genes is None and records.xs is None:
+            raise ValueError("the XS source needs records.xs (Records.from_bam(..., xs=True) or from_reads with an xs column)")
+        v = records.view()
+        out = np.zeros(3, np.int64)
+        xs = _ptr(records.xs, L.c_u8p) if records.xs is not None else None
+        gv = C.byref(genes.view()) if genes is not None else None
+        self._check(self._lib.spl_infer_strand_records(self._h, C.byref(v), xs, n_chrom, gv, _ptr(out, L.c_i64p)),
+                    "spl_infer_strand_records")
+        return StrandVotes(*(int(x) for x in out))
+
+    def infer_strand_bam(self, bam_path, chrom_names, genes: GeneStrands = None) -> StrandVotes:
+        """infer_strand_records of a BAM, ingested as extract_junctions_bam ingests it (the XS column only for genes=None)."""
+        return self._infer(self._lib.spl_infer_strand, str(bam_path).encode(), chrom_names, genes)
+
+    def _infer(self, fn, source, chrom_names, genes):
+        out = np.zeros(3, np.int64)
+        gv = C.byref(genes.view()) if genes is not None else None
+        self._check(fn(self._h, source, len(chrom_names), _names(chrom_names), gv, _ptr(out, L.c_i64p)), fn.__name__)
+        return StrandVotes(*(int(x) for x in out))
 
     # ---- device-resident samples -----------------------------------------------------------------
     def load_bam(self, bam_path, xs=False) -> "DeviceSample":

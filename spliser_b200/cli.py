@@ -7,16 +7,20 @@
 
 Without regtools (not a reference command; regtools' option letters):
     python -m spliser_b200.cli junctions -B x.bam -o x.bed [-a 8] [-m 70] [-M 500000] [--isStranded -s rf|fr | --strandFromXS]
-    python -m spliser_b200.cli processBam -B x.bam -o out [process's -A -t -c -g -m --isStranded -s --beta2Cryptic]
+    python -m spliser_b200.cli processBam -B x.bam -o out [process's -A -t -c -g -m --isStranded -s rf|fr|auto --beta2Cryptic]
                                           [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
-    python -m spliser_b200.cli combineBam -S samples.tsv -o out [-A genes.gff] [-t gene] [-g gene] [--isStranded -s rf|fr]
+    python -m spliser_b200.cli combineBam -S samples.tsv -o out [-A genes.gff] [-t gene] [-g gene] [--isStranded -s rf|fr|auto]
                                           [--beta2Cryptic] [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
                                           [--shallow [-m 0] [-r 10] [-e 0.0]] [--gpus N]
+    python -m spliser_b200.cli inferStrandedness -B x.bam [-A genes.gff]
 `junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
 `junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.  --strandFromXS
 takes the junction strands from the aligner's XS tag, as regtools does for unstranded libraries; processBam still counts
 with --isStranded -s.  `combineBam` is `processBam` for every sample of a samples file (writing its column 2) followed by
 `combine` (`combineShallow` with --shallow), with every BAM read once: the records stay in GPU memory for the re-count.
+`inferStrandedness` tells which of --isStranded -s fr, -s rf or an unstranded run fits the library (one vote per record,
+against the annotation's genes or the XS tag); `processBam` and `combineBam` take --isStranded -s auto to infer it over the
+same ingest and run with its verdict.
 
 What stays in Python is what the reference does in text: BED12 parsing and its filters (S:255-288), the
 annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) and the lock-step merge of
@@ -157,9 +161,16 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
     """`junctions` + `process -b` in one GPU call that ingests the BAM once (spl_process_bam_extract).  The chromosome list is
     the annotation's names, then the header's references not among them in header order: the relative order `process` gets
     from a BED12 written by `junctions`, so the .SpliSER.tsv is the same byte for byte.  strandFromXS: the table's strands come
-    from the XS tag (`junctions --strandFromXS`); the count still follows isStranded / strandedType."""
+    from the XS tag (`junctions --strandFromXS`); the count still follows isStranded / strandedType.
+
+    isStranded with strandedType 'auto': the library type is inferred first (inferStrandedness: votes from every gene of the
+    annotation, or from the XS tag without one) over the same ingest -- the BAM is loaded into GPU memory once, voted on and
+    counted from there (a BAM the device cannot hold is read twice: votes, then the count) -- and the run is the one the verdict's
+    flags give.  An undecided verdict raises StrandednessError before anything is written."""
     print("Processing")
-    print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
+    auto = isStranded and strandedType == "auto"
+    if not auto:
+        print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
     annotation = load_annotation(annotationFile, qGene) if annotationFile is not None else None
     bounds = None
     if qGene != "All":
@@ -169,28 +180,97 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
         bounds = (q.left, q.right)
     own = ctx is None
     ctx = ctx or api.Context(0)
+    sample = None
     try:
         extract = functools.partial(ctx.process_bam_extract, inBAM)
+        if auto:
+            chroms = _chrom_list(annotation, inBAM)
+            genes = None
+            if annotationFile is not None:
+                genes = api.gene_strands(annotation if qGene == "All" else load_annotation(annotationFile, "All"), chroms)
+            try:
+                sample = ctx.load_bam(inBAM, xs=genes is None or strandFromXS)
+                extract = sample.process_extract
+                votes = sample.infer_strand(chroms, genes)
+            except api.SampleMemoryError:
+                votes = ctx.infer_strand_bam(inBAM, chroms, genes)
+            isStranded, strandedType = _verdict_flags(votes, inBAM)
+            print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
         _process_bam_sample(extract, inBAM, outputPath + ".SpliSER.tsv", annotation, bounds, qChrom, maxIntronSize, isStranded,
                             strandedType, isbeta2Cryptic, minAnchor, minIntron, maxIntron, strandFromXS)
     finally:
+        if sample is not None:
+            sample.close()
         if own:
             ctx.close()
+
+
+def _chrom_list(annotation, inBAM):
+    """processBam's chromosome list: the annotation's names, then the header's references not among them in header order."""
+    chroms = list(annotation.chrom_index) if annotation is not None else []
+    known = set(chroms)
+    return chroms + [c for c in api.bam_reference_names(inBAM) if c not in known]
 
 
 def _process_bam_sample(extract, inBAM, tsv_path, annotation, bounds, qChrom, maxIntronSize, isStranded, strandedType, isbeta2Cryptic,
                         minAnchor, minIntron, maxIntron, strandFromXS):
     """processBam after the annotation load.  extract(chrom_names, flags, min_anchor, min_intron, max_intron, qchrom=, gene_bounds=,
     window_max_intron=) answers like Context.process_bam_extract of this BAM (or DeviceSample.process_extract of it loaded)."""
-    chroms = list(annotation.chrom_index) if annotation is not None else []
-    known = set(chroms)
-    chroms += [c for c in api.bam_reference_names(inBAM) if c not in known]
+    chroms = _chrom_list(annotation, inBAM)
     flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic) | (api.FLAG_XS_STRAND if strandFromXS else 0)
     junc, table = extract(chroms, flags, minAnchor, minIntron, maxIntron, qchrom=qChrom, gene_bounds=bounds,
                           window_max_intron=int(maxIntronSize))
     print("Sites:\t\t\t" + str(len(table)))
     write_process_tsv(tsv_path, chroms, table, _strand_column(junc), annotation=annotation, is_stranded=isStranded,
                       beta2_cryptic=isbeta2Cryptic)
+
+
+# ------------------------------------------------------------------------------------------------ library strandedness
+class StrandednessError(ValueError):
+    """-s auto could not settle the library type: too few votes, a share between the thresholds, or samples that disagree."""
+
+
+_FLAGS_OF = {"fr": "--isStranded -s fr", "rf": "--isStranded -s rf", "unstranded": "no --isStranded (unstranded)"}
+
+
+def _strand_report(votes):
+    """The lines every command that infers prints: the counts, f, the thresholds and the verdict as the flags to pass."""
+    v = votes.agree_fr + votes.opposite
+    verdict = api.library_type(votes)
+    return verdict, [
+        "Strand votes (one per record):\tagree with fr {}\topposite {}\tno vote {}".format(votes.agree_fr, votes.opposite, votes.no_vote),
+        "f = agree / (agree + opposite):\t" + ("{:.4f}".format(votes.agree_fr / v) if v else "n/a"),
+        "Thresholds:\t\t\tat least {} votes; fr when f >= {}, rf when f <= {}, unstranded when {} <= f <= {}".format(
+            api.MIN_VOTES, api.FR_MIN, api.RF_MAX, *api.UNSTRANDED_RANGE),
+        "Library type:\t\t\t" + (verdict + ": " + _FLAGS_OF[verdict] if verdict else "undecided")]
+
+
+def _verdict_flags(votes, what):
+    """Prints the report; (isStranded, strandedType) of the verdict, or StrandednessError when it is undecided."""
+    verdict, lines = _strand_report(votes)
+    print("\n".join(lines))
+    if verdict is None:
+        raise StrandednessError("the library type of %s is undecided: pass --isStranded -s fr|rf, or nothing for an unstranded run"
+                                % what)
+    return (False, None) if verdict == "unstranded" else (True, verdict)
+
+
+def inferStrandedness(inBAM, annotationFile=None, ctx=None):
+    """The library's protocol from the BAM (one vote per record; include/spliser_b200.h, spl_gene_strands, states the rule): the
+    reference strand from every gene of the annotation, or from the aligner's XS tag without one.  Prints the counts, f, the
+    thresholds and the verdict as the flags to pass; returns (verdict, StrandVotes) and raises StrandednessError when it is
+    undecided."""
+    chroms = api.bam_reference_names(inBAM)
+    genes = api.gene_strands(load_annotation(annotationFile, "All"), chroms) if annotationFile is not None else None
+    own = ctx is None
+    ctx = ctx or api.Context(0)
+    try:
+        votes = ctx.infer_strand_bam(inBAM, chroms, genes)
+    finally:
+        if own:
+            ctx.close()
+    _verdict_flags(votes, inBAM)
+    return api.library_type(votes), votes
 
 
 # ------------------------------------------------------------------------------------------------ combine
@@ -367,7 +447,11 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
     samples dist.samples_of(rank, n_devices, n_samples) in both GPU phases: a sample is loaded into its rank's GPU memory
     (Context.load_bam), its table extracted and counted from there, and after the merge its gaps are re-counted from there.  A
     sample the device cannot hold (SampleMemoryError) takes the path route -- process_bam_extract, then recount_bam -- with the
-    same output."""
+    same output.
+
+    isStranded with strandedType 'auto': every rank loads its samples and votes on each (inferStrandedness's rule) before any
+    extraction; the verdict is taken on the pooled votes and is refused (StrandednessError, nothing written) when it is undecided
+    or when a sample's own decided verdict differs from it.  The run is then the one the verdict's flags give."""
     print("Combining samples from their BAMs...")
     titles, tsv_paths, bam_paths = _read_samples_file(samplesFile, shallow)
     n = len(titles)
@@ -377,7 +461,15 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
     n_ranks = len(devs)
     ctxs = [None] * n_ranks
     resident = [None] * n                           # DeviceSample, or None: the path route
-    flags = api.mode_flags(isStranded, strandedType, False, combine=True)
+    auto = isStranded and strandedType == "auto"
+    votes = [None] * n
+    flags = None if auto else api.mode_flags(isStranded, strandedType, False, combine=True)
+
+    def extract(rank, k):
+        c = ctxs[rank]
+        ex = resident[k].process_extract if resident[k] is not None else functools.partial(c.process_bam_extract, bam_paths[k])
+        _process_bam_sample(ex, bam_paths[k], tsv_paths[k], annotation, None, "All", 0, isStranded, strandedType, isbeta2Cryptic,
+                            minAnchor, minIntron, maxIntron, strandFromXS)
 
     def process_rank(rank):
         mine = samples_of(rank, n_ranks, n)
@@ -385,13 +477,24 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
             return
         ctxs[rank] = c = make(devs[rank])
         for k in mine:
+            genes = None
+            if auto:
+                chroms = _chrom_list(annotation, bam_paths[k])
+                genes = api.gene_strands(annotation, chroms) if annotation is not None else None
             try:
-                resident[k] = c.load_bam(bam_paths[k], xs=strandFromXS)
-                extract = resident[k].process_extract
+                resident[k] = c.load_bam(bam_paths[k], xs=strandFromXS or (auto and genes is None))
             except api.SampleMemoryError:
-                extract = functools.partial(c.process_bam_extract, bam_paths[k])
-            _process_bam_sample(extract, bam_paths[k], tsv_paths[k], annotation, None, "All", 0, isStranded, strandedType,
-                                isbeta2Cryptic, minAnchor, minIntron, maxIntron, strandFromXS)
+                pass
+            if not auto:
+                extract(rank, k)
+            elif resident[k] is not None:
+                votes[k] = resident[k].infer_strand(chroms, genes)
+            else:
+                votes[k] = c.infer_strand_bam(bam_paths[k], chroms, genes)
+
+    def extract_rank(rank):
+        for k in samples_of(rank, n_ranks, n):
+            extract(rank, k)
 
     def recount(c, k, names, gaps):
         s, resident[k] = resident[k], None
@@ -401,6 +504,11 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
             return s.recount(names, gaps, flags)
     try:
         _on_ranks(n_ranks, process_rank)
+        if auto:
+            # with -s auto every sample is loaded and voted on first; the extraction then runs with the pooled verdict's flags
+            isStranded, strandedType = _pooled_verdict(titles, votes)
+            flags = api.mode_flags(isStranded, strandedType, False, combine=True)
+            _on_ranks(n_ranks, extract_rank)
         _merge_recount_write(titles, tsv_paths, outputPath, qGene, isStranded, isbeta2Cryptic,
                              (minSamples, minReads, minSSE) if shallow else None, n_ranks, lambda rank: ctxs[rank], recount)
     finally:
@@ -410,6 +518,19 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
         for c in ctxs:
             if c is not None:
                 c.close()
+
+
+def _pooled_verdict(titles, votes):
+    """combineBam -s auto: the verdict on the votes of all samples together; StrandednessError when it is undecided or when a
+    sample's own decided verdict differs from it (the error names those samples and their counts)."""
+    pooled = api.StrandVotes(*(sum(getattr(v, f) for v in votes) for f in ("agree_fr", "opposite", "no_vote")))
+    verdict = api.library_type(pooled)
+    odd = [(t, v, api.library_type(v)) for t, v in zip(titles, votes) if api.library_type(v) not in (None, verdict)]
+    if odd and verdict is not None:
+        print("\n".join(_strand_report(pooled)[1]))
+        raise StrandednessError("samples disagree with the pooled library type %s: %s" % (verdict, "; ".join(
+            "%s is %s (agree with fr %d, opposite %d, no vote %d)" % (t, lt, v.agree_fr, v.opposite, v.no_vote) for t, v, lt in odd)))
+    return _verdict_flags(pooled, "the pooled samples")
 
 
 # ------------------------------------------------------------------------------------------------ main
@@ -498,6 +619,10 @@ def main(argv=None):
     cb.add_argument("-e", "--minSSE", dest="minSSE", nargs="?", default=0.00, type=float)
     cb.add_argument("--gpus", dest="n_gpus", nargs="?", default=1, type=int,
                     help="hold and count the samples on this many GPUs (sharded by sample)")
+    inf = sub.add_parser("inferStrandedness", help="the library type (--isStranded -s fr|rf, or unstranded) from the BAM")
+    inf.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
+    inf.add_argument("-A", "--annotationFile", dest="annotationFile", required=False,
+                     help="reference strands from the genes of this GFF / GTF (default: from the aligner's XS tag)")
     kwargs = vars(parser.parse_args(argv))          # --strandFromXS is only passed on when given (SUPPRESS)
     command = kwargs.pop("command")
     if command in ("combine", "combineShallow", "combineBam"):
@@ -518,12 +643,14 @@ def main(argv=None):
         combineShallow(**kwargs)
     elif command == "junctions":
         junctions(**kwargs)
-    elif command == "processBam":
-        processBam(**kwargs)
-    elif command == "combineBam":
-        combineBam(**kwargs)
+    elif command in ("processBam", "combineBam", "inferStrandedness"):
+        try:
+            {"processBam": processBam, "combineBam": combineBam, "inferStrandedness": inferStrandedness}[command](**kwargs)
+        except StrandednessError as e:
+            parser.error(str(e))
     else:
-        parser.error("command must be process, combine, combineShallow, junctions, processBam or combineBam (output is unchanged Python in the reference)")
+        parser.error("command must be process, combine, combineShallow, junctions, processBam, combineBam or inferStrandedness "
+                     "(output is unchanged Python in the reference)")
     print("Total runtime (s): \t" + str(timeit.default_timer() - start))
 
 

@@ -27,6 +27,7 @@
 #include "graph_build.h"
 #include "junction_filter.h"
 #include "site_graph.h"
+#include "strand_votes.h"
 
 using namespace spl;
 
@@ -198,6 +199,7 @@ struct spl_ctx {
     DevBuf d_cpk;                                        // the columns of a compact upload (spl_process_compact)
     DevBuf d_frec, d_fchunks, d_hotq, d_fpk, d_unpack;   // d_fpk: packed columns (n_op, flag8) of spl_process_packed; d_unpack: scan descriptors + ticket
     DevBuf d_xs;                    // XS strand column of host records for the extraction (SPL_FLAG_XS_STRAND)
+    DevBuf d_votes;                 // strand votes: the three counters and the gene-strand index (spl_infer_strand*)
     uint32_t unpack_epoch = 0;
     uint32_t hot_cap = 0;           // items the global hot queue holds; a pass that needs more is repeated with room
     uint32_t* h_hot = nullptr;      // pinned: hot item count of the last pass
@@ -1458,7 +1460,7 @@ void spl_destroy(spl_ctx* ctx) {
         }
         if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
         ctx->d_frec.release(); ctx->d_fchunks.release(); ctx->d_hotq.release(); ctx->d_fpk.release(); ctx->d_unpack.release(); ctx->d_cpk.release();
-        ctx->d_xs.release();
+        ctx->d_xs.release(); ctx->d_votes.release();
         if (ctx->h_hot) cudaFreeHost(ctx->h_hot);
         if (ctx->h_fchunks) cudaFreeHost(ctx->h_fchunks);
         for (int p = 0; p < MAX_FPARTS; ++p) if (ctx->fpart[p].ev_up) cudaEventDestroy(ctx->fpart[p].ev_up);
@@ -2153,6 +2155,137 @@ int spl_sample_recount(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const
     SampleBinding bind(ctx, s);
     return spl_recount_records(ctx, &dv, n_chrom, n_sites, s_chrom, s_pos, s_strand, p_off, p_pos, c_off, c_pos, flags, beta1_out,
                                beta2simple_out);
+}
+
+namespace {
+// The one routine behind spl_infer_strand*: the records are where fused_upload finds them (host arrays, or ctx->dev_rec when
+// ctx->rec_on_device); xs = the host records' XS column (XS source with host records).  Only the three counters come back.
+int infer_common(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom, const spl_gene_strands* genes,
+                 int64_t counts[3]) {
+    if (!counts) return ctx->fail(SPL_ERR_ARG, "counts is NULL");
+    ctx->loaded = false;
+    int rc = check_view(ctx, rec, n_chrom);
+    if (rc) return rc;
+    GeneIndexHost gh;
+    if (genes) {
+        const std::string e = build_gene_index(genes, n_chrom, gh);
+        if (!e.empty()) return ctx->fail(SPL_ERR_ARG, "%s", e.c_str());
+    } else if (rec->n_rec > 0 && !(ctx->rec_on_device ? (const uint8_t*)ctx->dev_rec.xs : xs)) {
+        return ctx->fail(SPL_ERR_ARG, "the XS source needs the records' XS strand column");
+    }
+    CU(cudaSetDevice(ctx->device));
+    reset_stats(ctx);
+    while (ctx->events.size() < 2) {
+        cudaEvent_t e;
+        CU(cudaEventCreate(&e));
+        ctx->events.push_back(e);
+    }
+    rc = fused_upload(ctx, rec, n_chrom, false);
+    if (rc) return drain_on_error(ctx, rc);
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->fpart[0].ev_up, 0));
+    const uint8_t* d_xs = ctx->rec_on_device ? ctx->dev_rec.xs : nullptr;
+    if (!genes && !ctx->rec_on_device && rec->n_rec > 0) {             // 1 B per record, once
+        CU(ctx->d_xs.reserve((size_t)rec->n_rec + 16));
+        CU(cudaMemcpyAsync(ctx->d_xs.p, xs, (size_t)rec->n_rec, cudaMemcpyHostToDevice, ctx->stream));
+        ctx->stats[SPL_STAT_H2D_BYTES] += (double)rec->n_rec;
+        d_xs = (const uint8_t*)ctx->d_xs.p;
+    }
+    Carver c;
+    const size_t o_cnt = c.take<unsigned long long>(4), o_bnd = c.take<int32_t>(gh.bnd.size() + 1),
+                 o_off = c.take<int32_t>(gh.bnd_off.size() + 1), o_tab = c.take<uint8_t>(gh.table.size() + 1);
+    CU(ctx->d_votes.reserve(c.off + 256));
+    char* vb = (char*)ctx->d_votes.p;
+    unsigned long long* d_cnt = (unsigned long long*)(vb + o_cnt);
+    CU(cudaMemsetAsync(d_cnt, 0, 3 * sizeof(unsigned long long), ctx->stream));
+    GeneIndexDev gd{(const int32_t*)(vb + o_bnd), (const int32_t*)(vb + o_off), (const uint8_t*)(vb + o_tab), gh.m, n_chrom};
+    if (genes) {
+        if (!gh.bnd.empty()) CU(cudaMemcpyAsync(vb + o_bnd, gh.bnd.data(), gh.bnd.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(vb + o_off, gh.bnd_off.data(), gh.bnd_off.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+        if (!gh.table.empty()) CU(cudaMemcpyAsync(vb + o_tab, gh.table.data(), gh.table.size(), cudaMemcpyHostToDevice, ctx->stream));
+        ctx->stats[SPL_STAT_H2D_BYTES] += (double)(gh.bnd.size() * 4 + gh.bnd_off.size() * 4 + gh.table.size());
+    }
+    CU(cudaEventRecord(ctx->events[0], ctx->stream));
+    launch_strand_votes(ctx->frec, d_xs, ctx->fchunks, ctx->n_fchunks, genes ? &gd : nullptr, d_cnt, ctx->stream);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(ctx->events[1], ctx->stream));
+    unsigned long long h_cnt[3] = {0, 0, 0};
+    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof h_cnt, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, ctx->events[0], ctx->events[1]));
+    ctx->stats[SPL_STAT_MS_STRAND_VOTES] = ms;
+    ctx->stats[SPL_STAT_D2H_BYTES] += (double)sizeof h_cnt;
+    for (int k = 0; k < 3; ++k) counts[k] = (int64_t)h_cnt[k];
+    return SPL_OK;
+}
+}  // namespace
+
+int spl_infer_strand_records(spl_ctx* ctx, const spl_records_view* rec, const uint8_t* xs, int32_t n_chrom,
+                             const spl_gene_strands* genes, int64_t counts[3]) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    const double t0 = now_ms();
+    const int rc = infer_common(ctx, rec, xs, n_chrom, genes, counts);
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
+}
+
+int spl_infer_strand(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char* const* chrom_names,
+                     const spl_gene_strands* genes, int64_t counts[3]) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
+    if (n_chrom < 0 || (n_chrom > 0 && !chrom_names)) return ctx->fail(SPL_ERR_ARG, "chrom_names is NULL");
+    for (int32_t c = 0; c < n_chrom; ++c) if (!chrom_names[c]) return ctx->fail(SPL_ERR_ARG, "chromosome name %d is NULL", c);
+    const bool want_xs = genes == nullptr;
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    {   // ingest as spl_extract_junctions chooses: on the device, the host reader as the fallback
+        BamGpuCounts cnt;
+        spl_records_view dv{};
+        bool fallback = false;
+        int rc = ingest_bam_device(ctx, bam_path, n_chrom, chrom_names, cnt, dv, &fallback, want_xs);
+        if (rc) return rc;
+        if (!fallback) {
+            const double t1 = now_ms();
+            ctx->rec_on_device = true;
+            rc = infer_common(ctx, &dv, nullptr, n_chrom, genes, counts);
+            ctx->rec_on_device = false;
+            ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+            ctx->stats[SPL_STAT_H2D_BYTES] += cnt.h2d_bytes;
+            ctx->stats[SPL_STAT_BAM_DEVICE] = 1.0;
+            ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+            return rc;
+        }
+    }
+    BamRecords recs;
+    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, want_xs);
+    if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
+    const double t1 = now_ms();
+    spl_records_view v = recs.view();
+    const int rc = infer_common(ctx, &v, recs.xs.data(), n_chrom, genes, counts);
+    ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
+}
+
+int spl_sample_infer_strand(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
+                            const spl_gene_strands* genes, int64_t counts[3]) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    int rc = check_sample(ctx, s, n_chrom, chrom_names);
+    if (rc) return rc;
+    if (!genes && !s->rec.xs) return ctx->fail(SPL_ERR_ARG, "the XS source needs a sample loaded with SPL_FLAG_XS_STRAND");
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    std::vector<int32_t> seg_chrom;
+    const spl_records_view dv = sample_view(s, n_chrom, chrom_names, seg_chrom);
+    {
+        SampleBinding bind(ctx, s);
+        rc = infer_common(ctx, &dv, nullptr, n_chrom, genes, counts);
+    }
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return rc;
 }
 
 int64_t spl_sample_n_records(const spl_sample* s) { return s ? s->n_rec : 0; }
