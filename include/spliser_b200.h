@@ -88,6 +88,31 @@ int  spl_set_threads(spl_ctx* ctx, int n_host_threads);   /* BGZF inflate / reco
 #define SPL_VARIANT_FUSED 0
 #define SPL_VARIANT_STAB  1
 int  spl_set_variant(spl_ctx* ctx, int variant);
+
+/* ---- read filter (samtools view -q / -F / -f at ingest) ------------------------------------------------------------------
+ * Every ingest keeps a record when it is mapped to a caller chromosome and has at least one CIGAR operator (the keep rule of
+ * both BAM readers; the reference itself filters nothing, S:422).  With a read filter set on the context, a record that passes
+ * that rule is kept only if also
+ *   MAPQ >= min_mapq                                 (samtools -q: MAPQ 255, "unavailable", passes any threshold)
+ *   (FLAG & exclude_flags) == 0                      (samtools -F)
+ *   (FLAG & require_flags) == require_flags          (samtools -f)
+ * "Dropped by the filter" counts the records the keep rule keeps and these three conditions remove.  The filter applies
+ * wherever a BAM becomes records, on the device ingest and on the host reader alike: spl_process, spl_recount,
+ * spl_extract_junctions, spl_process_bam_extract, spl_infer_strand and spl_sample_load_bam.  A resident sample keeps the filter
+ * it was loaded under: spl_sample_process_extract / spl_sample_recount / spl_sample_infer_strand are SPL_ERR_ARG while the
+ * context's filter differs from it.  Host record arrays carry no MAPQ, so the record-array entry points (spl_*_records,
+ * spl_process_packed / _compact, spl_resident_load) are SPL_ERR_ARG while a filter is set -- it is never silently ignored.
+ * spl_set_read_filter(ctx, NULL) removes the filter; {0, 0, 0} keeps every record and counts as none.  MAPQ outside 0..255 or
+ * flags above 0xFFFF are SPL_ERR_ARG. */
+typedef struct spl_read_filter {
+    int32_t min_mapq;
+    uint32_t exclude_flags, require_flags;
+} spl_read_filter;
+int  spl_set_read_filter(spl_ctx* ctx, const spl_read_filter* filter /* NULL = none */);
+/* counts[0] = records kept, counts[1] = records dropped by the filter, in the last ingest of this context (zeros before the
+ * first; dropped is 0 without a filter).  Not part of spl_last_stats, whose SPL_NSTATS slots are all taken. */
+int  spl_last_read_filter(const spl_ctx* ctx, int64_t counts[2]);
+
 const char* spl_version(void);
 unsigned long long spl_kernel_launches(void);   /* kernels this library has launched in this process so far (every launch is counted) */
 
@@ -285,8 +310,8 @@ void    spl_sample_free(spl_sample* s);
 
 /* ---- library strandedness ------------------------------------------------------------------------------------------------
  * Which protocol (`--isStranded -s fr`, `-s rf`, or unstranded) a library was made with, from its records: one vote per record.
- *   - records: those an ingest keeps -- mapped to a caller chromosome, with at least one CIGAR operator; no FLAG filter (as
- *     checkBam, S:422);
+ *   - records: those an ingest keeps -- mapped to a caller chromosome, with at least one CIGAR operator, and through the
+ *     context's read filter (spl_read_filter; none by default, as checkBam, S:422);
  *   - read strand under fr (check_strand, S:374-406): first = FLAG & 64 or !(FLAG & 1), rev = FLAG & 16, strand =
  *     first ? (rev ? '-' : '+') : (rev ? '+' : '-'); under rf it is always the opposite, so the fr strand alone is compared;
  *   - reference strand, annotation source (genes != NULL): the record spans the 1-based bases POS .. POS + L - 1, L = the sum of
@@ -556,6 +581,11 @@ int spl_write_bam_seq(const char* path, int32_t n_ref, const char* const* ref_na
  * with the raw bytes aux[aux_off[i] .. aux_off[i + 1]), written as given (aux_off has n_rec + 1 entries). */
 int spl_write_bam_aux(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                       const spl_records_view* rec, const int64_t* aux_off, const uint8_t* aux, int with_seq, int n_threads);
+/* spl_write_bam_aux with a MAPQ per record (record order of the view); mapq == NULL writes 255, as the writers above do, and
+ * aux_off == NULL writes no aux fields.  The three writers above are this routine with mapq == NULL. */
+int spl_write_bam_mapq(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
+                       const spl_records_view* rec, const int64_t* aux_off, const uint8_t* aux, const uint8_t* mapq, int with_seq,
+                       int n_threads);
 /* Decodes a BAM into library-owned record arrays (host only; no GPU needed).  chrom_names maps
  * BAM reference names to caller chromosome indices; records on other references are dropped. */
 typedef struct spl_records spl_records;
@@ -564,6 +594,11 @@ int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_nam
 /* The same, and the strand of every kept record from its XS tag (SPL_FLAG_XS_STRAND's rule): spl_records_xs. */
 int spl_read_bam_xs(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
                     spl_records** out, char* err, int err_len);
+/* The same reader under a read filter (spl_read_filter's rule; NULL = none), with the XS column when want_xs != 0: the routine
+ * the context's host-reader fallback runs.  spl_records_filter_counts gives its kept / dropped counts. */
+int spl_read_bam_filtered(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
+                          const spl_read_filter* filter, int want_xs, spl_records** out, char* err, int err_len);
+int spl_records_filter_counts(const spl_records* r, int64_t counts[2]);
 const spl_records_view* spl_records_get(const spl_records* r);
 const uint8_t* spl_records_xs(const spl_records* r);      /* [n_rec] '+', '-' or '?'; NULL for a handle of spl_read_bam */
 void spl_records_free(spl_records* r);

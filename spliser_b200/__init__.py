@@ -5,8 +5,8 @@ package is its Python host side: ctypes binding, numpy API, BED12 parsing, gene 
 SpliSER-compatible CLI and TSV writers.  Importing the package does not need a GPU; creating a
 Context does, and there is no CPU fallback.
 """
-from .api import (CompactRecords, Context, DeviceSample, Junctions, PackedRecords, Records, SampleMemoryError, SiteTable,  # noqa: F401
-                  SpliserError, StrandVotes, mode_flags, FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names,
+from .api import (CompactRecords, Context, DeviceSample, Junctions, PackedRecords, ReadFilter, Records, SampleMemoryError,  # noqa: F401
+                  SiteTable, SpliserError, StrandVotes, mode_flags, FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names,
                   gene_strands, library_type)
 
 __version__ = "0.1.0"

@@ -61,6 +61,10 @@ class GeneStrandsView(C.Structure):
     _fields_ = [("n_chrom", C.c_int32), ("chrom_off", c_i64p), ("left", c_i32p), ("right", c_i32p), ("strand", c_u8p)]
 
 
+class ReadFilterC(C.Structure):
+    _fields_ = [("min_mapq", C.c_int32), ("exclude_flags", C.c_uint32), ("require_flags", C.c_uint32)]
+
+
 class SiteColumns(C.Structure):
     _fields_ = [("n_sites", C.c_int64), ("chrom", c_i32p), ("pos", c_i32p), ("first_line", c_i64p),
                 ("alpha", c_i64p), ("beta1", c_i64p), ("beta2simple", c_i64p), ("beta2cryptic", c_i64p),
@@ -83,6 +87,8 @@ SIGNATURES = {
     "spl_set_threads": (C.c_int, [C.c_void_p, C.c_int]),
     "spl_set_variant": (C.c_int, [C.c_void_p, C.c_int]),
     "spl_last_stats": (C.c_int, [C.c_void_p, c_f64p]),
+    "spl_set_read_filter": (C.c_int, [C.c_void_p, C.POINTER(ReadFilterC)]),
+    "spl_last_read_filter": (C.c_int, [C.c_void_p, c_i64p]),
     "spl_process": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp] + _JUNC + [C.c_uint32, C.POINTER(C.c_void_p)]),
     "spl_process_records": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), C.c_int32] + _JUNC + [C.c_uint32, C.POINTER(C.c_void_p)]),
     "spl_process_packed": (C.c_int, [C.c_void_p, C.POINTER(PackedView), C.c_int32] + _JUNC + [C.c_uint32, C.POINTER(C.c_void_p)]),
@@ -143,8 +149,13 @@ SIGNATURES = {
     "spl_write_bam": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), C.c_int]),
     "spl_write_bam_seq": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), C.c_int]),
     "spl_write_bam_aux": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), c_i64p, c_u8p, C.c_int, C.c_int]),
+    "spl_write_bam_mapq": (C.c_int, [C.c_char_p, C.c_int32, c_strp, c_i32p, C.POINTER(RecordsView), c_i64p, c_u8p, c_u8p, C.c_int,
+                                     C.c_int]),
     "spl_read_bam": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),
     "spl_read_bam_xs": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),
+    "spl_read_bam_filtered": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(ReadFilterC), C.c_int, C.POINTER(C.c_void_p),
+                                        C.c_char_p, C.c_int]),
+    "spl_records_filter_counts": (C.c_int, [C.c_void_p, c_i64p]),
     "spl_records_get": (C.POINTER(RecordsView), [C.c_void_p]),
     "spl_records_xs": (c_u8p, [C.c_void_p]),
     "spl_records_free": (None, [C.c_void_p]),

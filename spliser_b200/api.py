@@ -37,6 +37,30 @@ def mode_flags(is_stranded=False, stranded_type=None, beta2_cryptic=False, combi
     return f
 
 
+@dataclass(frozen=True)
+class ReadFilter:
+    """samtools view -q / -F / -f at ingest (include/spliser_b200.h, spl_read_filter, states the rule): a record the ingest keeps
+    (mapped to a caller chromosome, at least one CIGAR operator) is kept only if MAPQ >= min_mapq (255, "unavailable", passes
+    any threshold), FLAG & exclude_flags == 0 and FLAG & require_flags == require_flags.  ReadFilter() keeps every record."""
+    min_mapq: int = 0
+    exclude_flags: int = 0
+    require_flags: int = 0
+
+    def __post_init__(self):
+        if not 0 <= int(self.min_mapq) <= 255:
+            raise ValueError("min_mapq must be in 0..255, got %r" % (self.min_mapq,))
+        for name in ("exclude_flags", "require_flags"):
+            if not 0 <= int(getattr(self, name)) <= 0xFFFF:
+                raise ValueError("%s must be in 0..0xFFFF, got %r" % (name, getattr(self, name)))
+
+    @property
+    def is_none(self) -> bool:
+        return self.min_mapq == 0 and self.exclude_flags == 0 and self.require_flags == 0
+
+    def _c(self):
+        return L.ReadFilterC(int(self.min_mapq), int(self.exclude_flags), int(self.require_flags))
+
+
 def encode_cigar(cigar: str):
     if cigar == "*" or not cigar:
         return []
@@ -150,13 +174,19 @@ class Records:
         return cls(pos, flag, off, cig, seg_chrom, seg_off, xs=xs if xs else None)
 
     @classmethod
-    def from_bam(cls, path, chrom_names, threads=0, xs=False):
-        """xs: also read every record's strand from its XS tag (Records.xs)."""
+    def from_bam(cls, path, chrom_names, threads=0, xs=False, read_filter: "ReadFilter" = None):
+        """xs: also read every record's strand from its XS tag (Records.xs).  read_filter: keep only the records it passes
+        (spl_read_bam_filtered, the reader a context falls back to); the result's filter_counts is then (kept, dropped)."""
         lib = L.load()
         names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
         h = C.c_void_p()
         err = C.create_string_buffer(512)
-        rc = (lib.spl_read_bam_xs if xs else lib.spl_read_bam)(str(path).encode(), len(chrom_names), names, threads, C.byref(h), err, 512)
+        if read_filter is not None:
+            rf = read_filter._c()
+            rc = lib.spl_read_bam_filtered(str(path).encode(), len(chrom_names), names, threads, C.byref(rf), int(bool(xs)), C.byref(h),
+                                           err, 512)
+        else:
+            rc = (lib.spl_read_bam_xs if xs else lib.spl_read_bam)(str(path).encode(), len(chrom_names), names, threads, C.byref(h), err, 512)
         if rc != 0:
             raise IOError("spl_read_bam(%s): %s" % (path, err.value.decode()))
         try:
@@ -170,13 +200,18 @@ class Records:
                       arr(v.cigar, nc, np.uint32), arr(v.seg_chrom, ns, np.int32),
                       np.ctypeslib.as_array(v.seg_off, shape=(ns + 1,)).astype(np.int64, copy=True),
                       xs=arr(lib.spl_records_xs(h), n, np.uint8) if xs else None)
+            if read_filter is not None:
+                fc = np.zeros(2, np.int64)
+                lib.spl_records_filter_counts(h, _ptr(fc, L.c_i64p))
+                out.filter_counts = (int(fc[0]), int(fc[1]))
         finally:
             lib.spl_records_free(h)
         return out
 
-    def write_bam(self, path, ref_names, ref_len=None, threads=0, with_seq=False, aux=None):
+    def write_bam(self, path, ref_names, ref_len=None, threads=0, with_seq=False, aux=None, mapq=None):
         """with_seq: read names, SEQ and QUAL of the CIGAR's query length are written too (a sequencer-shaped file).
-        aux: raw aux bytes per record, a list of bytes (see encode_aux) or (offsets[n_rec + 1], uint8 blob)."""
+        aux: raw aux bytes per record, a list of bytes (see encode_aux) or (offsets[n_rec + 1], uint8 blob).
+        mapq: MAPQ of every record (uint8, record order); None writes 255."""
         lib = L.load()
         names = (C.c_char_p * max(1, len(ref_names)))(*[c.encode() for c in ref_names])
         rl = None
@@ -184,8 +219,16 @@ class Records:
             rl = np.ascontiguousarray(ref_len, dtype=np.int32)
         v = self.view()
         rlp = _ptr(rl, L.c_i32p) if rl is not None else None
-        if aux is None:
+        mq = None
+        if mapq is not None:
+            mq = np.ascontiguousarray(mapq, dtype=np.uint8)
+            if len(mq) != len(self):
+                raise ValueError("mapq must have one entry per record")
+        if aux is None and mq is None:
             rc = (lib.spl_write_bam_seq if with_seq else lib.spl_write_bam)(str(path).encode(), len(ref_names), names, rlp, C.byref(v), threads)
+        elif aux is None:
+            rc = lib.spl_write_bam_mapq(str(path).encode(), len(ref_names), names, rlp, C.byref(v), None, None,
+                                        _ptr(mq, L.c_u8p) if len(mq) else None, int(with_seq), threads)
         else:
             if isinstance(aux, tuple):
                 off, blob = aux
@@ -197,8 +240,13 @@ class Records:
             blob = np.ascontiguousarray(blob, dtype=np.uint8)
             if len(off) != len(self) + 1 or (len(off) and (off[0] != 0 or off[-1] != len(blob) or np.any(np.diff(off) < 0))):
                 raise ValueError("aux offsets must run from 0 to len(blob), one record each")
-            rc = lib.spl_write_bam_aux(str(path).encode(), len(ref_names), names, rlp, C.byref(v), _ptr(off, L.c_i64p),
-                                       _ptr(blob, L.c_u8p) if len(blob) else C.cast(C.c_char_p(b""), L.c_u8p), int(with_seq), threads)
+            blob_p = _ptr(blob, L.c_u8p) if len(blob) else C.cast(C.c_char_p(b""), L.c_u8p)
+            if mq is None:
+                rc = lib.spl_write_bam_aux(str(path).encode(), len(ref_names), names, rlp, C.byref(v), _ptr(off, L.c_i64p), blob_p,
+                                           int(with_seq), threads)
+            else:
+                rc = lib.spl_write_bam_mapq(str(path).encode(), len(ref_names), names, rlp, C.byref(v), _ptr(off, L.c_i64p), blob_p,
+                                            _ptr(mq, L.c_u8p) if len(mq) else None, int(with_seq), threads)
         if rc != 0:
             raise IOError("spl_write_bam(%s) failed with %d" % (path, rc))
 
@@ -552,10 +600,12 @@ def _names(chrom_names):
 class DeviceSample:
     """One BAM's alignment records in device memory (Context.load_bam): the extraction + count of process_bam_extract and the
     re-count of recount_bam without reading the file again.  Calls go through the context that loaded it.  A context manager;
-    close() frees the device memory."""
+    close() frees the device memory.  read_filter: the context's read filter at the load (None = none); a call while the context
+    has another one raises SpliserError, since the sample's records would not be the ones a path call reads."""
 
-    def __init__(self, ctx: "Context", h):
+    def __init__(self, ctx: "Context", h, read_filter: "ReadFilter" = None):
         self._ctx, self._h = ctx, h
+        self.read_filter = read_filter
 
     @property
     def n_records(self) -> int:
@@ -648,6 +698,23 @@ class Context:
         bin-partitioned block stream; the cross-check)."""
         v = {"fused": 0, "stab": 1}[variant] if isinstance(variant, str) else int(variant)
         self._check(self._lib.spl_set_variant(self._h, v), "spl_set_variant")
+
+    def set_read_filter(self, min_mapq=0, exclude_flags=0, require_flags=0):
+        """samtools view -q / -F / -f for every following ingest of this context (ReadFilter states the rule); the defaults
+        remove the filter.  Record-array calls refuse to run while a filter is set (their arrays carry no MAPQ), and a
+        DeviceSample loaded under another filter refuses its calls."""
+        f = min_mapq if isinstance(min_mapq, ReadFilter) else ReadFilter(min_mapq, exclude_flags, require_flags)
+        rf = f._c()
+        self._check(self._lib.spl_set_read_filter(self._h, None if f.is_none else C.byref(rf)), "spl_set_read_filter")
+        self.read_filter = None if f.is_none else f
+
+    read_filter = None                              # the filter set_read_filter set, None = none
+
+    def last_read_filter(self):
+        """(records kept, records dropped by the read filter) in the last ingest of this context."""
+        out = np.zeros(2, np.int64)
+        self._check(self._lib.spl_last_read_filter(self._h, _ptr(out, L.c_i64p)), "spl_last_read_filter")
+        return int(out[0]), int(out[1])
 
     def stats(self):
         buf = (C.c_double * L.SPL_NSTATS)()
@@ -800,7 +867,7 @@ class Context:
         if rc == L.SPL_ERR_NOMEM:
             raise SampleMemoryError("spl_sample_load_bam(%s): %s" % (bam_path, self._lib.spl_last_error(self._h).decode()))
         self._check(rc, "spl_sample_load_bam")
-        return DeviceSample(self, h)
+        return DeviceSample(self, h, self.read_filter)
 
     # ---- combine re-count ----------------------------------------------------------------------
     @staticmethod
@@ -845,6 +912,12 @@ class Context:
         h = C.c_void_p()
         self._check(self._lib.spl_resident_fetch(self._h, C.byref(h)), "spl_resident_fetch")
         return self._take(h)
+
+
+def read_bam(path, chrom_names, threads=0, xs=False, read_filter: ReadFilter = None) -> Records:
+    """The host BAM reader (no GPU): Records.from_bam, under read_filter when given (the result's filter_counts is then
+    (kept, dropped))."""
+    return Records.from_bam(path, chrom_names, threads=threads, xs=xs, read_filter=read_filter)
 
 
 def bam_reference_names(path):

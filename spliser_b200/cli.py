@@ -13,6 +13,8 @@ Without regtools (not a reference command; regtools' option letters):
                                           [--beta2Cryptic] [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
                                           [--shallow [-m 0] [-r 10] [-e 0.0]] [--gpus N]
     python -m spliser_b200.cli inferStrandedness -B x.bam [-A genes.gff]
+Every command that reads a BAM also takes [--minMAPQ N] [--excludeFlags F] [--requireFlags F], samtools view's -q / -F / -f
+applied as the BAM is ingested (flags in decimal or 0x hex; include/spliser_b200.h, spl_read_filter, states the rule).
 `junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
 `junctions` followed by `process -b` in one call that reads the BAM once, and writes the same .SpliSER.tsv.  --strandFromXS
 takes the junction strands from the aligner's XS tag, as regtools does for unstranded libraries; processBam still counts
@@ -43,6 +45,21 @@ from .genes import load_annotation
 from .hosttext import CombineMerge, write_process_tsv as _native_write_process_tsv
 
 VERSION = "v0.1.8 (spliser_b200)"
+
+
+# ------------------------------------------------------------------------------------------------ read filter
+def _with_filter(ctx, read_filter):
+    """ctx under the command's read filter (api.ReadFilter, or None: the context is left as it is)."""
+    if read_filter is not None:
+        ctx.set_read_filter(read_filter)
+    return ctx
+
+
+def _report_filter(ctx, bam, read_filter):
+    """With a read filter, the one line per BAM: the records its ingest kept and the records the filter dropped."""
+    if read_filter is not None:
+        kept, dropped = ctx.last_read_filter()
+        print("Read filter {}:\tkept {}\tdropped {}".format(bam, kept, dropped))
 
 
 # ------------------------------------------------------------------------------------------------ process
@@ -93,7 +110,7 @@ def write_process_tsv(path, chroms, table, sstr, *, annotation=None, is_stranded
 
 
 def process(inBAM, inBed, outputPath, qGene="All", qChrom="All", maxIntronSize=0, annotationFile=None, aType="gene",
-            isStranded=False, strandedType=None, isbeta2Cryptic=False, ctx=None):
+            isStranded=False, strandedType=None, isbeta2Cryptic=False, ctx=None, read_filter=None):
     print("Processing")
     print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
     parsed_bed = None
@@ -115,10 +132,12 @@ def process(inBAM, inBed, outputPath, qGene="All", qChrom="All", maxIntronSize=0
     own = ctx is None
     ctx = ctx or api.Context(0)
     try:
+        _with_filter(ctx, read_filter)
         with open(inBed) as fh:
             chroms, table, sstr = process_table(ctx, inBAM, fh, annotation=annotation, qchrom=qChrom, qgene=qGene,
                                                 max_intron=maxIntronSize, is_stranded=isStranded, stranded_type=strandedType,
                                                 beta2_cryptic=isbeta2Cryptic, parsed_bed=parsed_bed)
+        _report_filter(ctx, inBAM, read_filter)
     finally:
         if own:
             ctx.close()
@@ -129,7 +148,7 @@ def process(inBAM, inBed, outputPath, qGene="All", qChrom="All", maxIntronSize=0
 
 # ------------------------------------------------------------------------------------------------ without regtools
 def junctions(inBAM, outBed, minAnchor=8, minIntron=70, maxIntron=500000, isStranded=False, strandedType=None, strandFromXS=False,
-              ctx=None):
+              ctx=None, read_filter=None):
     """The `regtools junctions extract -a -m -M` step on the GPU: the junction table of every header reference, written as
     BED12 in regtools' layout (chromStart / chromEnd from the longest anchors).  Strands: with strandFromXS the record's XS tag
     ('?' without one; include/spliser_b200.h, SPL_FLAG_XS_STRAND), else '?' unstranded, else the strand check_strand derives
@@ -139,7 +158,8 @@ def junctions(inBAM, outBed, minAnchor=8, minIntron=70, maxIntron=500000, isStra
     own = ctx is None
     ctx = ctx or api.Context(0)
     try:
-        junc = ctx.extract_junctions_bam(inBAM, chroms, flags, minAnchor, minIntron, maxIntron)
+        junc = _with_filter(ctx, read_filter).extract_junctions_bam(inBAM, chroms, flags, minAnchor, minIntron, maxIntron)
+        _report_filter(ctx, inBAM, read_filter)
     finally:
         if own:
             ctx.close()
@@ -157,7 +177,8 @@ def _strand_column(junc):
 
 
 def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, annotationFile=None, aType="gene", isStranded=False,
-               strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False, ctx=None):
+               strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False, ctx=None,
+               read_filter=None):
     """`junctions` + `process -b` in one GPU call that ingests the BAM once (spl_process_bam_extract).  The chromosome list is
     the annotation's names, then the header's references not among them in header order: the relative order `process` gets
     from a BED12 written by `junctions`, so the .SpliSER.tsv is the same byte for byte.  strandFromXS: the table's strands come
@@ -182,6 +203,7 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
     ctx = ctx or api.Context(0)
     sample = None
     try:
+        _with_filter(ctx, read_filter)
         extract = functools.partial(ctx.process_bam_extract, inBAM)
         if auto:
             chroms = _chrom_list(annotation, inBAM)
@@ -194,10 +216,13 @@ def processBam(inBAM, outputPath, qGene="All", qChrom="All", maxIntronSize=0, an
                 votes = sample.infer_strand(chroms, genes)
             except api.SampleMemoryError:
                 votes = ctx.infer_strand_bam(inBAM, chroms, genes)
+            _report_filter(ctx, inBAM, read_filter)
             isStranded, strandedType = _verdict_flags(votes, inBAM)
             print("Stranded Analysis {}".format(strandedType) if isStranded else "Unstranded Analysis")
         _process_bam_sample(extract, inBAM, outputPath + ".SpliSER.tsv", annotation, bounds, qChrom, maxIntronSize, isStranded,
                             strandedType, isbeta2Cryptic, minAnchor, minIntron, maxIntron, strandFromXS)
+        if not auto:
+            _report_filter(ctx, inBAM, read_filter)
     finally:
         if sample is not None:
             sample.close()
@@ -255,7 +280,7 @@ def _verdict_flags(votes, what):
     return (False, None) if verdict == "unstranded" else (True, verdict)
 
 
-def inferStrandedness(inBAM, annotationFile=None, ctx=None):
+def inferStrandedness(inBAM, annotationFile=None, ctx=None, read_filter=None):
     """The library's protocol from the BAM (one vote per record; include/spliser_b200.h, spl_gene_strands, states the rule): the
     reference strand from every gene of the annotation, or from the aligner's XS tag without one.  Prints the counts, f, the
     thresholds and the verdict as the flags to pass; returns (verdict, StrandVotes) and raises StrandednessError when it is
@@ -265,7 +290,8 @@ def inferStrandedness(inBAM, annotationFile=None, ctx=None):
     own = ctx is None
     ctx = ctx or api.Context(0)
     try:
-        votes = ctx.infer_strand_bam(inBAM, chroms, genes)
+        votes = _with_filter(ctx, read_filter).infer_strand_bam(inBAM, chroms, genes)
+        _report_filter(ctx, inBAM, read_filter)
     finally:
         if own:
             ctx.close()
@@ -386,7 +412,7 @@ def _merge_recount_write(titles, tsv_paths, outputPath, qGene, isStranded, isbet
 
 
 def combineShallow(samplesFile, outputPath, qGene="All", isStranded=False, minSamples=0, minReads=10, minSSE=0.0, strandedType=None,
-                   isbeta2Cryptic=False, ctx=None, records_by_bam=None, devices=None, context_factory=None):
+                   isbeta2Cryptic=False, ctx=None, records_by_bam=None, devices=None, context_factory=None, read_filter=None):
     """combineShallow (S:920-1167): `combine` for many shallow samples.  The same lock-step merge and the same re-count of the
     sites a sample lacks (checkBam at S:1145 -> one spl_recount call per sample), with three filters on which positions are
     kept at all -- a position needs at least `minSamples` samples showing it with alpha + beta1 + beta2Simple >= `minReads`
@@ -396,11 +422,11 @@ def combineShallow(samplesFile, outputPath, qGene="All", isStranded=False, minSa
     whatever its region or strand (S:1158-1160).  Unlike `combine`, a samples-file line without exactly three columns is
     skipped silently (S:930-935)."""
     return combine(samplesFile, outputPath, qGene, isStranded, strandedType, isbeta2Cryptic, ctx, records_by_bam, devices,
-                   context_factory, _shallow=(minSamples, minReads, minSSE))
+                   context_factory, _shallow=(minSamples, minReads, minSSE), read_filter=read_filter)
 
 
 def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType="fr", isbeta2Cryptic=False, ctx=None,
-            records_by_bam=None, devices=None, context_factory=None, _shallow=None):
+            records_by_bam=None, devices=None, context_factory=None, _shallow=None, read_filter=None):
     """combine (S:742-917).  The native merge driver (csrc/host_text.cpp) parses the sample tables and replays the
     lock-step merge, collecting per sample the sites it lacks together with the partner / competitor / strand context
     gathered from lower-indexed samples only (the reference's order dependence, SURVEY.md F7); one spl_recount call
@@ -409,7 +435,8 @@ def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType
     The re-count shards by sample (SURVEY.md 8(e)): with `devices` = several CUDA ordinals, one context per device runs on
     its own host thread and takes the samples dist.samples_of(rank, n_devices, n_samples); a sample's result depends on
     nothing but its own BAM and gap list, so the host only collects the count arrays.  `ctx` (one existing context) takes
-    precedence; `context_factory(device)` replaces api.Context (tests)."""
+    precedence; `context_factory(device)` replaces api.Context (tests).  read_filter (api.ReadFilter) applies to every
+    context the re-count uses."""
     print("Combining samples...")
     titles, bed_paths, bam_paths = _read_samples_file(samplesFile, _shallow is not None)
     flags = api.mode_flags(isStranded, strandedType, False, combine=True)
@@ -417,7 +444,9 @@ def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType
     def recount(c, k, names, gaps):
         if records_by_bam is not None:
             return c.recount_records(records_by_bam(bam_paths[k], names), len(names), gaps, flags)
-        return c.recount_bam(bam_paths[k], names, gaps, flags)
+        got = c.recount_bam(bam_paths[k], names, gaps, flags)
+        _report_filter(c, bam_paths[k], read_filter)
+        return got
     make = context_factory or api.Context
     devs = [0] if not devices else list(devices)
     n_ranks = 1 if ctx is not None else len(devs)
@@ -425,9 +454,9 @@ def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType
 
     def rank_ctx(rank):                             # one context per device, made when its rank first needs it
         if ctx is not None:
-            return ctx
+            return _with_filter(ctx, read_filter)
         made.append(make(devs[rank]))
-        return made[-1]
+        return _with_filter(made[-1], read_filter)
     try:
         _merge_recount_write(titles, bed_paths, outputPath, qGene, isStranded, isbeta2Cryptic, _shallow, n_ranks, rank_ctx, recount)
     finally:
@@ -437,7 +466,7 @@ def combine(samplesFile, outputPath, qGene="All", isStranded=False, strandedType
 
 def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene="All", isStranded=False, strandedType=None,
                isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False, shallow=False, minSamples=0,
-               minReads=10, minSSE=0.0, devices=None, context_factory=None):
+               minReads=10, minSSE=0.0, devices=None, context_factory=None, read_filter=None):
     """`processBam` for every sample of a samples file, then `combine` (or, with shallow, `combineShallow -m -r -e`) over them,
     reading every BAM once.  Column 2 of the samples file is where the sample's .SpliSER.tsv is written: the file `processBam -B
     <column 3>` writes with the same -A / --isStranded -s / --beta2Cryptic / --minAnchor --minIntron --maxIntron / --strandFromXS
@@ -451,7 +480,9 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
 
     isStranded with strandedType 'auto': every rank loads its samples and votes on each (inferStrandedness's rule) before any
     extraction; the verdict is taken on the pooled votes and is refused (StrandednessError, nothing written) when it is undecided
-    or when a sample's own decided verdict differs from it.  The run is then the one the verdict's flags give."""
+    or when a sample's own decided verdict differs from it.  The run is then the one the verdict's flags give.
+
+    read_filter (api.ReadFilter) applies to every rank's context: the samples are loaded, voted on and counted under it."""
     print("Combining samples from their BAMs...")
     titles, tsv_paths, bam_paths = _read_samples_file(samplesFile, shallow)
     n = len(titles)
@@ -475,7 +506,7 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
         mine = samples_of(rank, n_ranks, n)
         if not mine:
             return
-        ctxs[rank] = c = make(devs[rank])
+        ctxs[rank] = c = _with_filter(make(devs[rank]), read_filter)
         for k in mine:
             genes = None
             if auto:
@@ -483,6 +514,7 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
                 genes = api.gene_strands(annotation, chroms) if annotation is not None else None
             try:
                 resident[k] = c.load_bam(bam_paths[k], xs=strandFromXS or (auto and genes is None))
+                _report_filter(c, bam_paths[k], read_filter)
             except api.SampleMemoryError:
                 pass
             if not auto:
@@ -491,6 +523,8 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
                 votes[k] = resident[k].infer_strand(chroms, genes)
             else:
                 votes[k] = c.infer_strand_bam(bam_paths[k], chroms, genes)
+            if resident[k] is None:                 # the path route's first ingest of the BAM
+                _report_filter(c, bam_paths[k], read_filter)
 
     def extract_rank(rank):
         for k in samples_of(rank, n_ranks, n):
@@ -499,7 +533,7 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
     def recount(c, k, names, gaps):
         s, resident[k] = resident[k], None
         if s is None:
-            return c.recount_bam(bam_paths[k], names, gaps, flags)
+            return c.recount_bam(bam_paths[k], names, gaps, flags)     # the same BAM and filter again: no second report
         with s:
             return s.recount(names, gaps, flags)
     try:
@@ -534,6 +568,33 @@ def _pooled_verdict(titles, votes):
 
 
 # ------------------------------------------------------------------------------------------------ main
+def _mapq_value(x):
+    v = int(x, 0)
+    if not 0 <= v <= 255:
+        raise argparse.ArgumentTypeError("MAPQ must be in 0..255, got %s" % x)
+    return v
+
+
+def _flag_value(x):
+    v = int(x, 0)
+    if not 0 <= v <= 0xFFFF:
+        raise argparse.ArgumentTypeError("FLAG bits must be in 0..0xFFFF, got %s" % x)
+    return v
+
+
+def _add_read_filter_options(p):
+    """samtools view's -q / -F / -f under long names only (the short letters stay free for the reference's options)."""
+    p.add_argument("--minMAPQ", dest="minMAPQ", default=0, type=_mapq_value, metavar="N",
+                   help="keep records with MAPQ >= N (samtools -q; 255, unavailable, passes)")
+    p.add_argument("--excludeFlags", dest="excludeFlags", default=0, type=_flag_value, metavar="F",
+                   help="drop records with any of these FLAG bits (samtools -F), e.g. 0x904")
+    p.add_argument("--requireFlags", dest="requireFlags", default=0, type=_flag_value, metavar="F",
+                   help="keep records with all of these FLAG bits (samtools -f), e.g. 0x2")
+
+
+READ_COMMANDS = ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam", "inferStrandedness")
+
+
 def main(argv=None):
     print("\nSpliSER " + VERSION + "\n")
     start = timeit.default_timer()
@@ -623,8 +684,15 @@ def main(argv=None):
     inf.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
     inf.add_argument("-A", "--annotationFile", dest="annotationFile", required=False,
                      help="reference strands from the genes of this GFF / GTF (default: from the aligner's XS tag)")
+    for name, sp in sub.choices.items():
+        if name in READ_COMMANDS:
+            _add_read_filter_options(sp)
     kwargs = vars(parser.parse_args(argv))          # --strandFromXS is only passed on when given (SUPPRESS)
     command = kwargs.pop("command")
+    if command in READ_COMMANDS:
+        rf = api.ReadFilter(kwargs.pop("minMAPQ"), kwargs.pop("excludeFlags"), kwargs.pop("requireFlags"))
+        if not rf.is_none:
+            kwargs["read_filter"] = rf
     if command in ("combine", "combineShallow", "combineBam"):
         kwargs["devices"] = list(range(max(1, kwargs.pop("n_gpus") or 1)))
     if command in ("process", "processBam") and kwargs.get("qGene") != "All" and (kwargs.get("annotationFile") is None or kwargs.get("maxIntronSize") is None):

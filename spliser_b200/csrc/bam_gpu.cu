@@ -17,7 +17,9 @@
 //                      round-robin by the lanes: POS, FLAG, chromosome and CIGAR (k_bam_fill<true>: and the XS strand, from
 //                      a walk of the record's aux fields by the same lane)
 //   k_bam_segments     chromosome boundaries of the record arrays (a coordinate-sorted BAM has one segment per reference)
-// Kept records follow the host reader: mapped to a caller chromosome and with at least one CIGAR operator (bam_io.cpp).
+// Kept records follow the host reader: mapped to a caller chromosome, with at least one CIGAR operator (bam_io.cpp), and
+// through the read filter (read_filter.h; the rule is in include/spliser_b200.h, spl_read_filter).  The counting walk counts
+// the records the filter drops per member; k_bam_fill follows the walk's kept-offset list and needs no filter of its own.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -30,6 +32,7 @@
 #include "bam_gpu.h"
 #include "device_types.h"
 #include "inflate.h"
+#include "read_filter.h"
 
 namespace spl {
 
@@ -55,7 +58,7 @@ __device__ __forceinline__ uint32_t ld32u(const uint8_t* __restrict__ u, uint64_
 }
 
 // fixed part of a BAM record at offset o, read as 9 aligned words
-struct RecHdr { uint32_t bs, l_name, n_cig, flag; int32_t refid, pos, l_seq, next_ref, next_pos; };
+struct RecHdr { uint32_t bs, l_name, mapq, n_cig, flag; int32_t refid, pos, l_seq, next_ref, next_pos; };
 __device__ __forceinline__ RecHdr read_hdr(const uint8_t* __restrict__ u, uint64_t o) {
     const uint32_t* w = reinterpret_cast<const uint32_t*>(u + (o & ~3ull));
     const uint32_t sh = (uint32_t)(o & 3ull) * 8u;
@@ -66,7 +69,9 @@ __device__ __forceinline__ RecHdr read_hdr(const uint8_t* __restrict__ u, uint64
     h.bs = __funnelshift_r(a[0], a[1], sh);
     h.refid = (int32_t)__funnelshift_r(a[1], a[2], sh);
     h.pos = (int32_t)__funnelshift_r(a[2], a[3], sh);
-    h.l_name = __funnelshift_r(a[3], a[4], sh) & 0xffu;
+    const uint32_t bmn = __funnelshift_r(a[3], a[4], sh);              // bin_mq_nl: l_read_name, MAPQ, bin
+    h.l_name = bmn & 0xffu;
+    h.mapq = (bmn >> 8) & 0xffu;
     const uint32_t cf = __funnelshift_r(a[4], a[5], sh);
     h.n_cig = cf & 0xffffu; h.flag = cf >> 16;
     h.l_seq = (int32_t)__funnelshift_r(a[5], a[6], sh);
@@ -113,7 +118,7 @@ __global__ void __launch_bounds__(256) k_bam_first(const uint8_t* __restrict__ u
     if (lane == 0) first[m] = found;
 }
 
-struct WalkOut { uint64_t land; uint32_t n_rec, n_cig, flags, pad; };
+struct WalkOut { uint64_t land; uint32_t n_rec, n_cig, flags, n_drop; };   // n_drop: records the read filter dropped
 constexpr uint32_t WALK_BAD = 1u, WALK_LONG_CIGAR = 2u;
 
 // slot of member m's first kept-record offset in the scratch list: a record is at least 36 bytes, so the records that
@@ -124,14 +129,14 @@ template <bool FILL>
 __global__ void __launch_bounds__(128) k_bam_walk(const uint8_t* __restrict__ u, const BgzfMember* __restrict__ mem, uint32_t n_mem, uint64_t total,
                                                   int32_t n_ref, const int32_t* __restrict__ refmap, const uint64_t* __restrict__ first,
                                                   WalkOut* __restrict__ wo, const uint64_t* __restrict__ rec_base, const uint64_t* __restrict__ cig_base,
-                                                  DevRecordArrays out, uint32_t* __restrict__ kept) {
+                                                  DevRecordArrays out, uint32_t* __restrict__ kept, ReadFilter rf) {
     const uint32_t m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= n_mem) return;
     uint64_t o = first[m];
     if (FILL) { if (rec_base[m] == ~0ull) return; }                      // member not on the verified chain
     if (o == ~0ull) { if (!FILL) wo[m] = WalkOut{~0ull, 0, 0, 0, 0}; return; }
     const uint64_t limit = mem[m].uoff + mem[m].isize;
-    uint32_t n_rec = 0, n_cig_tot = 0, flags = 0;
+    uint32_t n_rec = 0, n_cig_tot = 0, flags = 0, n_drop = 0;
     uint64_t ri = FILL ? rec_base[m] : 0, ci = FILL ? cig_base[m] : 0;
     while (o < limit) {
         uint64_t nx;
@@ -141,7 +146,9 @@ __global__ void __launch_bounds__(128) k_bam_walk(const uint8_t* __restrict__ u,
         // CIGARs of more than 65535 operators live in a CG tag (SAM spec 4.2.2): left to the host reader
         if (h.n_cig == 2 && ld32u(u, cig) == (((uint32_t)h.l_seq << 4) | 4u) && (ld32u(u, cig + 4) & 15u) == 3u) flags |= WALK_LONG_CIGAR;
         const int32_t chrom = h.refid >= 0 ? refmap[h.refid] : -1;
-        if (chrom >= 0 && h.n_cig > 0) {
+        if (chrom >= 0 && h.n_cig > 0 && !read_filter_keeps(rf, h.mapq, h.flag)) {
+            ++n_drop;
+        } else if (chrom >= 0 && h.n_cig > 0) {
             if (!FILL && kept) kept[list_base(mem[m], m) + n_rec] = (uint32_t)(o - mem[m].uoff);   // may exceed isize-1 never: o < limit
             if (FILL) {
                 out.pos[ri] = h.pos + 1;
@@ -154,7 +161,7 @@ __global__ void __launch_bounds__(128) k_bam_walk(const uint8_t* __restrict__ u,
         }
         o = nx;
     }
-    if (!FILL) wo[m] = WalkOut{o, n_rec, n_cig_tot, flags, 0};
+    if (!FILL) wo[m] = WalkOut{o, n_rec, n_cig_tot, flags, n_drop};
 }
 
 // second pass, one WARP per accepted member: the lanes take the kept records of the member round-robin from the offset list
@@ -223,7 +230,7 @@ __global__ void k_set_u32(uint32_t* p, uint32_t v) { *p = v; }
 
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream, bool comp_uploaded,
-                   bool want_xs, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
+                   bool want_xs, const ReadFilter& rf, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
     cudaStream_t st = (cudaStream_t)stream;
     const uint32_t n_mem = (uint32_t)members.size();
     cnt = BamGpuCounts{};
@@ -258,7 +265,7 @@ int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const
     { SPL_LAUNCH; k_bgzf_inflate<<<(n_mem + INF_WARPS - 1) / INF_WARPS, INF_WARPS * 32, 0, st>>>((const uint8_t*)mem.comp.p, d_mem, n_mem, (uint8_t*)mem.unc.p, d_err); }
     // ---- speculative record starts + counting walk
     { SPL_LAUNCH; k_bam_first<<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, total_u, n_ref, first_record, d_first); }
-    { SPL_LAUNCH; k_bam_walk<false><<<(n_mem + 127) / 128, 128, 0, st>>>(d_u, d_mem, n_mem, total_u, n_ref, d_refmap, d_first, d_wo, nullptr, nullptr, DevRecordArrays{}, d_kept); }
+    { SPL_LAUNCH; k_bam_walk<false><<<(n_mem + 127) / 128, 128, 0, st>>>(d_u, d_mem, n_mem, total_u, n_ref, d_refmap, d_first, d_wo, nullptr, nullptr, DevRecordArrays{}, d_kept, rf); }
     BG_CU(cudaGetLastError());
     std::vector<uint64_t> h_first(n_mem);
     std::vector<WalkOut> h_wo(n_mem);
@@ -270,7 +277,7 @@ int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const
     if (h_err[0]) { err = "BGZF inflate failed on the device (member " + std::to_string(h_err[0] - 1) + ")"; return BAMGPU_FALLBACK; }
     // ---- verify the chain: each accepted member's walk must land exactly on the next accepted member's candidate
     std::vector<uint64_t> rbase(n_mem, ~0ull), cbase(n_mem, ~0ull);
-    uint64_t expect = first_record, nrec = 0, ncig = 0;
+    uint64_t expect = first_record, nrec = 0, ncig = 0, ndrop = 0;
     uint32_t m = 0;
     while (expect < total_u) {
         while (m < n_mem && members[m].uoff + members[m].isize <= expect) ++m;      // member that holds `expect`
@@ -279,13 +286,13 @@ int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const
         if (h_wo[m].flags & WALK_BAD) { err = "implausible BAM record"; return BAMGPU_FALLBACK; }
         if (h_wo[m].flags & WALK_LONG_CIGAR) { err = "CG-tag CIGAR"; return BAMGPU_FALLBACK; }
         rbase[m] = nrec; cbase[m] = ncig;
-        nrec += h_wo[m].n_rec; ncig += h_wo[m].n_cig;
+        nrec += h_wo[m].n_rec; ncig += h_wo[m].n_cig; ndrop += h_wo[m].n_drop;
         expect = h_wo[m].land;
         ++m;
     }
     if (expect != total_u) { err = "truncated BAM (partial record at end of file)"; return BAMGPU_FALLBACK; }
     if (nrec >= (uint64_t)UINT32_MAX - 16 || ncig >= (uint64_t)UINT32_MAX - 16) { err = "more than 2^32 records or CIGAR operators"; return BAMGPU_FALLBACK; }
-    cnt.n_rec = nrec; cnt.n_cigar = ncig;
+    cnt.n_rec = nrec; cnt.n_cigar = ncig; cnt.n_dropped = ndrop;
     // ---- record arrays
     {
         size_t off = 0;

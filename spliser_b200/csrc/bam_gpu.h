@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "graph_build.h"   // GbBuf
+#include "read_filter.h"
 
 namespace spl {
 
@@ -29,6 +30,7 @@ struct BamGpuMem { GbBuf comp, unc, tab, rec, list; };
 
 struct BamGpuCounts {
     uint64_t n_rec = 0, n_cigar = 0;
+    uint64_t n_dropped = 0;  // records the keep rule keeps and the read filter drops
     std::vector<int32_t> seg_chrom;
     std::vector<int64_t> seg_off;
     double h2d_bytes = 0;
@@ -48,6 +50,6 @@ std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const cha
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream,
                    bool comp_uploaded /* mem.comp already holds the file image (copy queued on `stream`) */,
-                   bool want_xs /* fill out.xs */, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err);
+                   bool want_xs /* fill out.xs */, const ReadFilter& rf, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err);
 
 }  // namespace spl

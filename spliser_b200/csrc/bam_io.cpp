@@ -68,6 +68,13 @@ bool find_cg(const uint8_t* p, const uint8_t* end, const uint8_t*& data, uint32_
 
 }  // namespace
 
+bool read_filter_from(const spl_read_filter& f, ReadFilter& out, std::string& err) {
+    if (f.min_mapq < 0 || f.min_mapq > 255) { err = "read filter: MAPQ threshold " + std::to_string(f.min_mapq) + " outside 0..255"; return false; }
+    if (f.exclude_flags > 0xFFFFu || f.require_flags > 0xFFFFu) { err = "read filter: FLAG bits above 0xFFFF"; return false; }
+    out.min_mapq = (uint32_t)f.min_mapq; out.exclude = f.exclude_flags; out.require = f.require_flags;
+    return true;
+}
+
 std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, int32_t n_chrom, const char* const* chrom_names) {
     std::unordered_map<std::string, int32_t> names;
     for (int32_t c = 0; c < n_chrom; ++c)
@@ -81,7 +88,7 @@ std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, i
 }
 
 std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out, bool want_xs,
-                     std::vector<std::string>* header_order) {
+                     std::vector<std::string>* header_order, const ReadFilter& rf) {
     out = BamRecords();
     if (header_order) header_order->clear();
     const int fd = open(path, O_RDONLY);
@@ -195,7 +202,7 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             if ((size_t)(end - p) < 4 + (size_t)bs) break;
             const uint8_t* r = p + 4;
             const int32_t refid = rdi32(r), pos0 = rdi32(r + 4);
-            const uint32_t l_name = r[8];
+            const uint32_t l_name = r[8], mapq = r[9];
             uint32_t n_cig = rd16(r + 12);
             const uint16_t flag = rd16(r + 14);
             const int32_t l_seq = rdi32(r + 16);
@@ -213,6 +220,7 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             }
             const int32_t chrom = (refid >= 0 && (size_t)refid < refmap.size()) ? refmap[(size_t)refid] : -1;
             if (chrom < 0 || n_cig == 0) { out.n_skipped++; continue; }
+            if (!read_filter_keeps(rf, mapq, flag)) { out.n_filtered++; continue; }
             if (chrom != cur_chrom) {
                 out.seg_chrom.push_back(chrom);
                 out.seg_off.push_back((int64_t)out.pos.size());
@@ -351,7 +359,8 @@ bool deflate_block(const uint8_t* src, uint32_t n, std::vector<uint8_t>& dst) {
 }  // namespace
 
 std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
-                      const spl_records_view* rec, int n_threads, bool with_seq, const int64_t* aux_off, const uint8_t* aux) {
+                      const spl_records_view* rec, int n_threads, bool with_seq, const int64_t* aux_off, const uint8_t* aux,
+                      const uint8_t* mapq) {
     if (!path || !rec || n_ref < 0 || (aux_off && !aux)) return "bad argument";
     std::vector<uint8_t> u;
     u.reserve((size_t)rec->n_rec * (with_seq ? 300 : 40) + (size_t)rec->n_cigar * 4 + 4096);
@@ -384,12 +393,13 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
             const int64_t a0 = aux_off ? aux_off[i] : 0, a1 = aux_off ? aux_off[i + 1] : 0;
             if (a1 < a0 || a1 - a0 > (1 << 24)) return "write_bam: bad aux offsets";
             const uint32_t n_aux = (uint32_t)(a1 - a0);
+            const uint8_t mq = mapq ? mapq[i] : (uint8_t)255;
             if (!with_seq) {
                 wr32(u, 32 + 2 + n_cig * 4 + n_aux);
                 wr32(u, (uint32_t)ref);
                 wr32(u, (uint32_t)pos0);
                 u.push_back(2);                       // l_read_name
-                u.push_back(255);                     // mapq
+                u.push_back(mq);                      // mapq
                 wr16(u, (uint16_t)reg2bin(pos0, pos0 + (reflen ? reflen : 1)));
                 wr16(u, (uint16_t)n_cig);
                 wr16(u, rec->flag[i]);
@@ -413,7 +423,7 @@ std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_na
             wr32(u, (uint32_t)ref);
             wr32(u, (uint32_t)pos0);
             u.push_back((uint8_t)ln);
-            u.push_back(255);
+            u.push_back(mq);
             wr16(u, (uint16_t)reg2bin(pos0, pos0 + (reflen ? reflen : 1)));
             wr16(u, (uint16_t)n_cig);
             wr16(u, rec->flag[i]);
@@ -489,6 +499,13 @@ int spl_write_bam_aux(const char* path, int32_t n_ref, const char* const* ref_na
     return SPL_OK;
 }
 
+int spl_write_bam_mapq(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len, const spl_records_view* rec,
+                       const int64_t* aux_off, const uint8_t* aux, const uint8_t* mapq, int with_seq, int n_threads) {
+    const std::string e = spl::write_bam(path, n_ref, ref_names, ref_len, rec, n_threads, with_seq != 0, aux_off, aux, mapq);
+    if (!e.empty()) { fprintf(stderr, "spl_write_bam_mapq: %s\n", e.c_str()); return SPL_ERR_IO; }
+    return SPL_OK;
+}
+
 int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                   const spl_records_view* rec, int n_threads) {
     const std::string e = spl::write_bam(path, n_ref, ref_names, ref_len, rec, n_threads);
@@ -498,12 +515,12 @@ int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names,
 
 namespace {
 int read_bam_handle(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, bool want_xs, spl_records** out,
-                    char* err, int err_len) {
+                    char* err, int err_len, const spl::ReadFilter& rf = spl::ReadFilter{}) {
     if (!out || !path) return SPL_ERR_ARG;
     *out = nullptr;
     spl_records* h = new (std::nothrow) spl_records();
     if (!h) return SPL_ERR_NOMEM;
-    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r, want_xs);
+    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r, want_xs, nullptr, rf);
     if (!e.empty()) {
         if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
         delete h;
@@ -524,6 +541,26 @@ int spl_read_bam(const char* path, int32_t n_chrom, const char* const* chrom_nam
 int spl_read_bam_xs(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, spl_records** out,
                     char* err, int err_len) {
     return read_bam_handle(path, n_chrom, chrom_names, n_threads, true, out, err, err_len);
+}
+
+int spl_read_bam_filtered(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, const spl_read_filter* filter,
+                          int want_xs, spl_records** out, char* err, int err_len) {
+    spl::ReadFilter rf;
+    if (filter) {
+        std::string e;
+        if (!spl::read_filter_from(*filter, rf, e)) {
+            if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
+            return SPL_ERR_ARG;
+        }
+    }
+    return read_bam_handle(path, n_chrom, chrom_names, n_threads, want_xs != 0, out, err, err_len, rf);
+}
+
+int spl_records_filter_counts(const spl_records* r, int64_t counts[2]) {
+    if (!r || !counts) return SPL_ERR_ARG;
+    counts[0] = (int64_t)r->r.pos.size();
+    counts[1] = r->r.n_filtered;
+    return SPL_OK;
 }
 
 const spl_records_view* spl_records_get(const spl_records* r) { return r ? &r->v : nullptr; }

@@ -7,6 +7,7 @@
 #include <vector>
 
 #include "../../include/spliser_b200.h"
+#include "read_filter.h"
 
 namespace spl {
 
@@ -20,6 +21,7 @@ struct BamRecords {
     std::vector<int64_t> seg_off;    // n_seg+1
     int64_t n_total = 0;             // records in the file
     int64_t n_skipped = 0;           // unmapped / unknown reference / no CIGAR
+    int64_t n_filtered = 0;          // kept by the rule above, dropped by the read filter
     spl_records_view view() const;
 };
 
@@ -27,13 +29,18 @@ struct BamRecords {
 // name repeats there), else -1.  Every reader and the device-resident samples map references with this one rule.
 std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, int32_t n_chrom, const char* const* chrom_names);
 
+// The ABI's filter checked (MAPQ 0..255, flags <= 0xFFFF) and converted; false with the reason in err.
+bool read_filter_from(const spl_read_filter& f, ReadFilter& out, std::string& err);
+
 // Returns "" or an error message.  chrom_names maps BAM reference names to caller indices.  header_order != NULL: chrom_names
 // is ignored, every record keeps its header reference index (seg_chrom) and *header_order receives the reference names.
+// rf: the read filter, applied after the keep rule (and after a CG-tag CIGAR replaced the placeholder).
 std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out,
-                     bool want_xs = false, std::vector<std::string>* header_order = nullptr);
+                     bool want_xs = false, std::vector<std::string>* header_order = nullptr, const ReadFilter& rf = ReadFilter{});
 
 std::string write_bam(const char* path, int32_t n_ref, const char* const* ref_names, const int32_t* ref_len,
                       const spl_records_view* rec, int n_threads, bool with_seq = false,
-                      const int64_t* aux_off = nullptr /* [n_rec + 1], or NULL */, const uint8_t* aux = nullptr /* raw aux bytes */);
+                      const int64_t* aux_off = nullptr /* [n_rec + 1], or NULL */, const uint8_t* aux = nullptr /* raw aux bytes */,
+                      const uint8_t* mapq = nullptr /* [n_rec], or NULL = 255 */);
 
 }  // namespace spl

@@ -194,6 +194,9 @@ struct spl_ctx {
     int variant = SPL_VARIANT_FUSED;
     int loaded_variant = SPL_VARIANT_FUSED;
     double stats[SPL_NSTATS] = {0};
+    ReadFilter rf;                  // spl_set_read_filter; {0, 0, 0} = none
+    int64_t rf_counts[2] = {0, 0};  // kept / dropped by the filter in the last ingest (spl_last_read_filter)
+    bool from_bam = false;          // the records of the current call came from an ingest under rf (see refuse_records)
 
     // fused variant (count_fused.cu)
     DevBuf d_cpk;                                        // the columns of a compact upload (spl_process_compact)
@@ -1385,16 +1388,41 @@ int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const cha
     if (!e.empty()) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_IO, "%s", e.c_str()); }
     if (header_order) for (int32_t r = 0; r < n_ref; ++r) refmap[(size_t)r] = r;
     const int rc = bam_gpu_ingest(ctx->bgm, (const uint8_t*)ctx->h_file, fsz, members, total_u, first_record, n_ref, refmap, ctx->stream,
-                                  uploaded, want_xs, ctx->dev_rec, cnt, e);
+                                  uploaded, want_xs, ctx->rf, ctx->dev_rec, cnt, e);
     if (rc != BAMGPU_OK) cudaStreamSynchronize(ctx->stream);           // the pinned image may be re-used by the fallback / next call
     if (rc == BAMGPU_ERROR) return ctx->fail(SPL_ERR_CUDA, "%s", e.c_str());
     if (rc == BAMGPU_FALLBACK) { *fallback = true; return SPL_OK; }
+    ctx->rf_counts[0] = (int64_t)cnt.n_rec; ctx->rf_counts[1] = (int64_t)cnt.n_dropped;
     view = spl_records_view{};
     view.n_rec = (int64_t)cnt.n_rec; view.n_cigar = (int64_t)cnt.n_cigar;
     view.n_seg = (int32_t)cnt.seg_chrom.size();
     view.seg_chrom = cnt.seg_chrom.data(); view.seg_off = cnt.seg_off.data();
     return SPL_OK;
 }
+
+// The host reader under the context's read filter: the fallback of every ingest above
+std::string read_bam_ctx(spl_ctx* ctx, const char* path, int32_t n_chrom, const char* const* chrom_names, BamRecords& recs, bool want_xs = false,
+                         std::vector<std::string>* header_order = nullptr) {
+    std::string e = read_bam(path, n_chrom, chrom_names, ctx->n_threads, recs, want_xs, header_order, ctx->rf);
+    if (e.empty()) { ctx->rf_counts[0] = (int64_t)recs.pos.size(); ctx->rf_counts[1] = recs.n_filtered; }
+    return e;
+}
+
+// Host record arrays carry no MAPQ: a record-array entry point refuses to run while a read filter is set, unless its records
+// came from an ingest that applied it (the path entry points and the resident samples call these routines themselves)
+int refuse_records(spl_ctx* ctx, const char* fn) {
+    if (ctx->from_bam || read_filter_none(ctx->rf)) return SPL_OK;
+    return ctx->fail(SPL_ERR_ARG, "%s: host record arrays carry no MAPQ, so the context's read filter cannot be applied; "
+                     "remove it (spl_set_read_filter(ctx, NULL)) or pass the BAM path", fn);
+}
+
+// marks the records of one call as ingested under the context's filter
+struct FromBam {
+    spl_ctx* ctx;
+    bool saved;
+    explicit FromBam(spl_ctx* c) : ctx(c), saved(c->from_bam) { ctx->from_bam = true; }
+    ~FromBam() { ctx->from_bam = saved; }
+};
 
 }  // namespace
 
@@ -1512,6 +1540,21 @@ int spl_set_threads(spl_ctx* ctx, int n) {
     return SPL_OK;
 }
 
+int spl_set_read_filter(spl_ctx* ctx, const spl_read_filter* filter) {
+    if (!ctx) return SPL_ERR_ARG;
+    ReadFilter rf;
+    std::string e;
+    if (filter && !read_filter_from(*filter, rf, e)) return ctx->fail(SPL_ERR_ARG, "%s", e.c_str());
+    ctx->rf = rf;
+    return SPL_OK;
+}
+
+int spl_last_read_filter(const spl_ctx* ctx, int64_t counts[2]) {
+    if (!ctx || !counts) return SPL_ERR_ARG;
+    counts[0] = ctx->rf_counts[0]; counts[1] = ctx->rf_counts[1];
+    return SPL_OK;
+}
+
 int spl_last_stats(const spl_ctx* ctx, double* stats_out) {
     if (!ctx || !stats_out) return SPL_ERR_ARG;
     memcpy(stats_out, ctx->stats, sizeof ctx->stats);
@@ -1525,6 +1568,7 @@ int spl_process_records(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chr
     if (!out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (const int rr = refuse_records(ctx, "spl_process_records")) return rr;
     const double t0 = now_ms();
     int rc = load_common(ctx, rec, n_chrom, n_junc, j_chrom, j_left, j_right, j_score, j_strand, flags, true);
     if (rc) return drain_on_error(ctx, rc);
@@ -1554,6 +1598,7 @@ int spl_process_packed(spl_ctx* ctx, const spl_packed_view* pv, int32_t n_chrom,
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (!pv) return ctx->fail(SPL_ERR_ARG, "packed view is NULL");
+    if (const int rr = refuse_records(ctx, "spl_process_packed")) return rr;
     if (ctx->variant != SPL_VARIANT_FUSED) return ctx->fail(SPL_ERR_ARG, "the packed view is read by the fused variant only");
     if (pv->n_rec > 0 && (!pv->pos || !pv->flag8 || !pv->n_op || !pv->cig_index)) return ctx->fail(SPL_ERR_ARG, "NULL packed array");
     if (pv->n_cigar > 0 && !pv->cigar) return ctx->fail(SPL_ERR_ARG, "NULL cigar array");
@@ -1590,6 +1635,7 @@ int spl_process_compact(spl_ctx* ctx, const spl_compact_view* cv, int32_t n_chro
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (!cv) return ctx->fail(SPL_ERR_ARG, "compact view is NULL");
+    if (const int rr = refuse_records(ctx, "spl_process_compact")) return rr;
     if (ctx->variant != SPL_VARIANT_FUSED) return ctx->fail(SPL_ERR_ARG, "the compact view is read by the fused variant only");
     if (cv->n_rec < 0 || cv->n16 < 0 || cv->n32 < 0 || cv->n_wide < 0 || cv->n16 + cv->n32 != cv->n_cigar)
         return ctx->fail(SPL_ERR_ARG, "compact view: inconsistent sizes");
@@ -1655,6 +1701,7 @@ int spl_process(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
     if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
     const double t0 = now_ms();
     CU(cudaSetDevice(ctx->device));
+    FromBam from_bam(ctx);
     {   // BGZF inflate + record parse on the device; the host reader is the fallback for what that path does not cover
         BamGpuCounts cnt;
         spl_records_view dv{};
@@ -1674,7 +1721,7 @@ int spl_process(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs);
+    std::string e = read_bam_ctx(ctx, bam_path, n_chrom, chrom_names, recs);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
@@ -1778,6 +1825,7 @@ int spl_extract_junctions_records(spl_ctx* ctx, const spl_records_view* rec, int
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (flags & SPL_FLAG_XS_STRAND) return ctx->fail(SPL_ERR_ARG, "SPL_FLAG_XS_STRAND needs the strand column of spl_extract_junctions_records_xs");
+    if (const int rr = refuse_records(ctx, "spl_extract_junctions_records")) return rr;
     return extract_common(ctx, rec, nullptr, n_chrom, min_anchor, min_intron, max_intron, flags, out);
 }
 
@@ -1788,6 +1836,7 @@ int spl_extract_junctions_records_xs(spl_ctx* ctx, const spl_records_view* rec, 
     *out = nullptr;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (!xs && rec && rec->n_rec > 0) return ctx->fail(SPL_ERR_ARG, "xs is NULL");
+    if (const int rr = refuse_records(ctx, "spl_extract_junctions_records_xs")) return rr;
     return extract_common(ctx, rec, xs, n_chrom, min_anchor, min_intron, max_intron, flags, out);
 }
 
@@ -1819,7 +1868,7 @@ int spl_extract_junctions(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, c
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
+    std::string e = read_bam_ctx(ctx, bam_path, n_chrom, chrom_names, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
@@ -1849,6 +1898,7 @@ int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom,
     for (int32_t c = 0; c < n_chrom; ++c) if (!chrom_names[c]) return ctx->fail(SPL_ERR_ARG, "chromosome name %d is NULL", c);
     const double t0 = now_ms();
     CU(cudaSetDevice(ctx->device));
+    FromBam from_bam(ctx);
     {   // ingest exactly as spl_process chooses: BGZF inflate + record parse on the device, the host reader as the fallback
         BamGpuCounts cnt;
         spl_records_view dv{};
@@ -1868,7 +1918,7 @@ int spl_process_bam_extract(spl_ctx* ctx, const char* bam_path, int32_t n_chrom,
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
+    std::string e = read_bam_ctx(ctx, bam_path, n_chrom, chrom_names, recs, (flags & SPL_FLAG_XS_STRAND) != 0);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
@@ -1885,6 +1935,7 @@ int spl_recount_records(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chr
     if (!ctx) return SPL_ERR_ARG;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
     if (n_sites > 0 && (!beta1_out || !beta2simple_out)) return ctx->fail(SPL_ERR_ARG, "NULL output array");
+    if (const int rr = refuse_records(ctx, "spl_recount_records")) return rr;
     ctx->loaded = false;
     int rc = check_view(ctx, rec, n_chrom);
     if (rc) return rc;
@@ -1948,6 +1999,7 @@ int spl_recount(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
     if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
     const double t0 = now_ms();
     CU(cudaSetDevice(ctx->device));
+    FromBam from_bam(ctx);
     {
         BamGpuCounts cnt;
         spl_records_view dv{};
@@ -1967,7 +2019,7 @@ int spl_recount(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs);
+    std::string e = read_bam_ctx(ctx, bam_path, n_chrom, chrom_names, recs);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
@@ -1987,6 +2039,7 @@ struct spl_sample {
     DevRecordArrays rec{};                // pos / flag / cig_off / cigar (/ xs) inside mem; no per-record chromosome
     int64_t n_rec = 0, n_cigar = 0;
     std::vector<std::string> ref_names;   // the header's references, in header order
+    ReadFilter rf;                        // the read filter the records were ingested under
     std::vector<int32_t> seg_ref;         // header reference index of every segment
     std::vector<int64_t> seg_off;         // [n_seg + 1]
 };
@@ -2016,6 +2069,10 @@ int sample_reserve(spl_ctx* ctx, size_t bytes, void** p) {
 int check_sample(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names) {
     if (!s) return ctx->fail(SPL_ERR_ARG, "sample is NULL");
     if (s->ctx != ctx) return ctx->fail(SPL_ERR_ARG, "the sample was loaded by another context");
+    if (s->rf.min_mapq != ctx->rf.min_mapq || s->rf.exclude != ctx->rf.exclude || s->rf.require != ctx->rf.require)
+        return ctx->fail(SPL_ERR_ARG, "the sample was loaded under read filter (min MAPQ %u, exclude 0x%x, require 0x%x) and the context's is "
+                         "now (min MAPQ %u, exclude 0x%x, require 0x%x): load the sample again, or set its filter back",
+                         s->rf.min_mapq, s->rf.exclude, s->rf.require, ctx->rf.min_mapq, ctx->rf.exclude, ctx->rf.require);
     if (n_chrom < 0 || (n_chrom > 0 && !chrom_names)) return ctx->fail(SPL_ERR_ARG, "chrom_names is NULL");
     for (int32_t c = 0; c < n_chrom; ++c) if (!chrom_names[c]) return ctx->fail(SPL_ERR_ARG, "chromosome name %d is NULL", c);
     return SPL_OK;
@@ -2038,7 +2095,8 @@ struct SampleBinding {
     spl_ctx* ctx;
     DevRecordArrays saved;
     bool saved_dev;
-    SampleBinding(spl_ctx* c, const spl_sample* s) : ctx(c), saved(c->dev_rec), saved_dev(c->rec_on_device) {
+    FromBam from_bam;                     // the sample's records were ingested under its filter, which check_sample matched
+    SampleBinding(spl_ctx* c, const spl_sample* s) : ctx(c), saved(c->dev_rec), saved_dev(c->rec_on_device), from_bam(c) {
         ctx->dev_rec = s->rec;
         ctx->rec_on_device = true;
     }
@@ -2061,6 +2119,7 @@ int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_
     if (!s) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
     s->ctx = ctx;
     s->device = ctx->device;
+    s->rf = ctx->rf;
     // ingest exactly as spl_process chooses, every reference kept in header order
     BamGpuCounts cnt;
     spl_records_view dv{};
@@ -2069,7 +2128,7 @@ int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_
     if (rc) return rc;
     BamRecords recs;
     if (fallback) {
-        std::string e = read_bam(bam_path, 0, nullptr, ctx->n_threads, recs, want_xs, &s->ref_names);
+        std::string e = read_bam_ctx(ctx, bam_path, 0, nullptr, recs, want_xs, &s->ref_names);
         if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
         s->n_rec = (int64_t)recs.pos.size(); s->n_cigar = (int64_t)recs.cigar.size();
         s->seg_ref = recs.seg_chrom; s->seg_off = recs.seg_off;
@@ -2224,6 +2283,7 @@ int spl_infer_strand_records(spl_ctx* ctx, const spl_records_view* rec, const ui
                              const spl_gene_strands* genes, int64_t counts[3]) {
     if (!ctx) return SPL_ERR_ARG;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (const int rr = refuse_records(ctx, "spl_infer_strand_records")) return rr;
     const double t0 = now_ms();
     const int rc = infer_common(ctx, rec, xs, n_chrom, genes, counts);
     ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
@@ -2259,7 +2319,7 @@ int spl_infer_strand(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const 
         }
     }
     BamRecords recs;
-    std::string e = read_bam(bam_path, n_chrom, chrom_names, ctx->n_threads, recs, want_xs);
+    std::string e = read_bam_ctx(ctx, bam_path, n_chrom, chrom_names, recs, want_xs);
     if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
     const double t1 = now_ms();
     spl_records_view v = recs.view();
@@ -2305,6 +2365,7 @@ int spl_resident_load(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom
                       const int32_t* j_left, const int32_t* j_right, const int64_t* j_score, const uint8_t* j_strand, uint32_t flags) {
     if (!ctx) return SPL_ERR_ARG;
     if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (const int rr = refuse_records(ctx, "spl_resident_load")) return rr;
     int rc = load_common(ctx, rec, n_chrom, n_junc, j_chrom, j_left, j_right, j_score, j_strand, flags, false);
     if (rc) return drain_on_error(ctx, rc);
     CU(cudaStreamSynchronize(ctx->stream));
