@@ -308,6 +308,50 @@ int64_t spl_sample_n_records(const spl_sample* s);
 int64_t spl_sample_device_bytes(const spl_sample* s);
 void    spl_sample_free(spl_sample* s);
 
+/* ---- samples told apart by an aux tag --------------------------------------------------------------------------------------
+ * Several samples in one BAM (read groups RG:Z, cell-barcode clusters CB:Z, haplotypes HP:i), split into resident samples by
+ * one ingest.  A tag group table has a two-character tag (SAM spec: [A-Za-z][A-Za-z0-9]), 1 <= n_groups <= 65535 groups, and
+ * n_values distinct values, value v being blob[offsets[v] .. offsets[v + 1]) and mapped to group[v] (0 <= group[v] < n_groups;
+ * a group may have no value).  A value is a non-empty byte string of at most 255 bytes without NUL, TAB or newline.  A repeated
+ * value, a bad tag or an out-of-range group is SPL_ERR_ARG.
+ *
+ * A record's value: its aux fields are walked as for SPL_FLAG_XS_STRAND, and the FIRST field with the tag decides -- type Z: the
+ * bytes before the NUL; type A: the one character; types c C s S i I: the decimal text of the integer as samtools prints it
+ * ("1", "-3"); any other type (f, H, B), no such field, or a malformed field before it: no value.  Matching is exact byte
+ * equality.  Every record an ingest keeps (the keep rule, then the context's read filter) is in exactly one class: group g,
+ * "no value", or "value in no group"; the three counts add up to spl_last_read_filter's counts[0].
+ *
+ * Defining property: group g's sample holds exactly the kept records whose value maps to g, in BAM order, under the BAM's full
+ * header; every spl_sample_* call on it gives what the same call gives on the sample spl_sample_load_bam loads from a BAM of just
+ * those records (the XS column too, under SPL_FLAG_XS_STRAND).
+ *
+ * spl_sample_load_bam_groups ingests the BAM once (on the device, or the host reader as the fallback; the group of every record is
+ * found as it is parsed), sorts the records stably by group on the device and gathers every group's columns into its own slice
+ * of one device allocation, which the group samples share: it is freed when the last of them is.  The split makes one
+ * reservation under spl_sample_load_bam's residency rule (the kept records of every group plus the sort scratch must fit);
+ * SPL_ERR_NOMEM holds nothing.  The sort scratch is released before the call returns.  spl_sample_device_bytes of a group sample is its own slice; the slices add up to the allocation.
+ * out[n_groups] receives the samples in group order (a group without records is a valid, empty sample); counts[n_groups + 2]
+ * the records of every group, then "no value", then "value in no group".  flags: SPL_FLAG_XS_STRAND only.  spl_last_stats
+ * reports SPL_STAT_MS_DECODE, SPL_STAT_H2D_BYTES and SPL_STAT_BAM_DEVICE of the ingest as spl_sample_load_bam does.  No existing
+ * call changes.
+ *
+ * spl_read_bam_groups is the host reader with the grouping (the fallback's routine): spl_records_group gives the int32 group of
+ * every kept record (-1 no value, -2 value in no group). */
+typedef struct spl_tag_groups {
+    char tag[2];
+    int32_t n_groups;
+    int64_t n_values;
+    const uint8_t* blob;
+    const int64_t* offsets;       /* [n_values + 1], offsets[0] == 0 */
+    const int32_t* group;         /* [n_values] */
+} spl_tag_groups;
+int spl_sample_load_bam_groups(spl_ctx* ctx, const char* bam_path, uint32_t flags, const spl_tag_groups* groups,
+                               spl_sample** out /* [n_groups] */, int64_t* counts /* [n_groups + 2] */);
+/* The records a resident sample holds, copied back into host record arrays (spl_records_get; spl_records_xs for a sample loaded
+ * with SPL_FLAG_XS_STRAND): POS, FLAG, CIGAR offsets and operators in the sample's order, seg_chrom = the header reference
+ * index of every segment (spl_bam_reference_names order).  What a sample holds, for checks and tests. */
+int spl_sample_fetch_records(spl_ctx* ctx, const spl_sample* s, struct spl_records** out);
+
 /* ---- library strandedness ------------------------------------------------------------------------------------------------
  * Which protocol (`--isStranded -s fr`, `-s rf`, or unstranded) a library was made with, from its records: one vote per record.
  *   - records: those an ingest keeps -- mapped to a caller chromosome, with at least one CIGAR operator, and through the
@@ -599,6 +643,12 @@ int spl_read_bam_xs(const char* path, int32_t n_chrom, const char* const* chrom_
 int spl_read_bam_filtered(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
                           const spl_read_filter* filter, int want_xs, spl_records** out, char* err, int err_len);
 int spl_records_filter_counts(const spl_records* r, int64_t counts[2]);
+/* spl_read_bam_filtered with the tag group of every kept record (spl_tag_groups' rule; groups != NULL): spl_records_group.  A
+ * table that breaks the rule is SPL_ERR_ARG with the reason in err. */
+int spl_read_bam_groups(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads,
+                        const spl_read_filter* filter, int want_xs, const spl_tag_groups* groups, spl_records** out, char* err,
+                        int err_len);
+const int32_t* spl_records_group(const spl_records* r);   /* [n_rec]; NULL for a handle read without groups */
 const spl_records_view* spl_records_get(const spl_records* r);
 const uint8_t* spl_records_xs(const spl_records* r);      /* [n_rec] '+', '-' or '?'; NULL for a handle of spl_read_bam */
 void spl_records_free(spl_records* r);

@@ -6,7 +6,7 @@ SpliSER-compatible CLI and TSV writers.  Importing the package does not need a G
 Context does, and there is no CPU fallback.
 """
 from .api import (CompactRecords, Context, DeviceSample, Junctions, PackedRecords, ReadFilter, Records, SampleMemoryError,  # noqa: F401
-                  SiteTable, SpliserError, StrandVotes, mode_flags, FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names,
+                  SiteTable, SpliserError, StrandVotes, TagGroups, GroupedSamples, mode_flags, FLAG_COMBINE, FLAG_CRYPTIC, FLAG_RF, FLAG_STRANDED, bam_reference_names,
                   gene_strands, library_type)
 
 __version__ = "0.1.0"

@@ -65,6 +65,11 @@ class ReadFilterC(C.Structure):
     _fields_ = [("min_mapq", C.c_int32), ("exclude_flags", C.c_uint32), ("require_flags", C.c_uint32)]
 
 
+class TagGroupsC(C.Structure):
+    _fields_ = [("tag", C.c_char * 2), ("n_groups", C.c_int32), ("n_values", C.c_int64), ("blob", c_u8p), ("offsets", c_i64p),
+                ("group", c_i32p)]
+
+
 class SiteColumns(C.Structure):
     _fields_ = [("n_sites", C.c_int64), ("chrom", c_i32p), ("pos", c_i32p), ("first_line", c_i64p),
                 ("alpha", c_i64p), ("beta1", c_i64p), ("beta2simple", c_i64p), ("beta2cryptic", c_i64p),
@@ -115,6 +120,8 @@ SIGNATURES = {
     "spl_sample_n_records": (C.c_int64, [C.c_void_p]),
     "spl_sample_device_bytes": (C.c_int64, [C.c_void_p]),
     "spl_sample_free": (None, [C.c_void_p]),
+    "spl_sample_fetch_records": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "spl_sample_load_bam_groups": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint32, C.POINTER(TagGroupsC), C.POINTER(C.c_void_p), c_i64p]),
     "spl_infer_strand_records": (C.c_int, [C.c_void_p, C.POINTER(RecordsView), c_u8p, C.c_int32, C.POINTER(GeneStrandsView), c_i64p]),
     "spl_infer_strand": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, c_strp, C.POINTER(GeneStrandsView), c_i64p]),
     "spl_sample_infer_strand": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, c_strp, C.POINTER(GeneStrandsView), c_i64p]),
@@ -156,6 +163,9 @@ SIGNATURES = {
     "spl_read_bam_filtered": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(ReadFilterC), C.c_int, C.POINTER(C.c_void_p),
                                         C.c_char_p, C.c_int]),
     "spl_records_filter_counts": (C.c_int, [C.c_void_p, c_i64p]),
+    "spl_read_bam_groups": (C.c_int, [C.c_char_p, C.c_int32, c_strp, C.c_int, C.POINTER(ReadFilterC), C.c_int, C.POINTER(TagGroupsC),
+                                      C.POINTER(C.c_void_p), C.c_char_p, C.c_int]),
+    "spl_records_group": (c_i32p, [C.c_void_p]),
     "spl_records_get": (C.POINTER(RecordsView), [C.c_void_p]),
     "spl_records_xs": (c_u8p, [C.c_void_p]),
     "spl_records_free": (None, [C.c_void_p]),

@@ -113,7 +113,7 @@ class Records:
     """Alignment records as flat arrays grouped in chromosome segments (spl_records_view).  xs: optional strand of every record
     from its XS tag (uint8 '+', '-' or '?'), what extraction with FLAG_XS_STRAND reads."""
 
-    def __init__(self, pos, flag, cig_off, cigar, seg_chrom, seg_off, _owner=None, xs=None):
+    def __init__(self, pos, flag, cig_off, cigar, seg_chrom, seg_off, _owner=None, xs=None, group=None):
         self.pos = np.ascontiguousarray(pos, dtype=np.int32)
         self.flag = np.ascontiguousarray(flag, dtype=np.uint16)
         self.cig_off = np.ascontiguousarray(cig_off, dtype=np.uint32)
@@ -122,6 +122,7 @@ class Records:
         self.seg_off = np.ascontiguousarray(seg_off, dtype=np.int64)
         self._owner = _owner
         self.xs = None if xs is None else np.ascontiguousarray(xs, dtype=np.uint8)
+        self.group = None if group is None else np.ascontiguousarray(group, dtype=np.int32)   # read_bam(groups=): tag group per record
         if len(self.cig_off) != len(self.pos) + 1 or len(self.flag) != len(self.pos):
             raise ValueError("record arrays differ in length")
         if self.xs is not None and len(self.xs) != len(self.pos):
@@ -174,14 +175,23 @@ class Records:
         return cls(pos, flag, off, cig, seg_chrom, seg_off, xs=xs if xs else None)
 
     @classmethod
-    def from_bam(cls, path, chrom_names, threads=0, xs=False, read_filter: "ReadFilter" = None):
+    def from_bam(cls, path, chrom_names, threads=0, xs=False, read_filter: "ReadFilter" = None, groups: "TagGroups" = None):
         """xs: also read every record's strand from its XS tag (Records.xs).  read_filter: keep only the records it passes
-        (spl_read_bam_filtered, the reader a context falls back to); the result's filter_counts is then (kept, dropped)."""
+        (spl_read_bam_filtered, the reader a context falls back to); the result's filter_counts is then (kept, dropped).
+        groups: the tag group of every kept record in Records.group (spl_read_bam_groups: a group, -1 no value, -2 value in no
+        group)."""
         lib = L.load()
         names = (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
         h = C.c_void_p()
         err = C.create_string_buffer(512)
-        if read_filter is not None:
+        if groups is not None:
+            rf = read_filter._c() if read_filter is not None else None
+            tg = groups._c()
+            rc = lib.spl_read_bam_groups(str(path).encode(), len(chrom_names), names, threads, C.byref(rf) if rf is not None else None,
+                                         int(bool(xs)), C.byref(tg), C.byref(h), err, 512)
+            if rc == -1:
+                raise ValueError("spl_read_bam_groups(%s): %s" % (path, err.value.decode()))
+        elif read_filter is not None:
             rf = read_filter._c()
             rc = lib.spl_read_bam_filtered(str(path).encode(), len(chrom_names), names, threads, C.byref(rf), int(bool(xs)), C.byref(h),
                                            err, 512)
@@ -189,6 +199,11 @@ class Records:
             rc = (lib.spl_read_bam_xs if xs else lib.spl_read_bam)(str(path).encode(), len(chrom_names), names, threads, C.byref(h), err, 512)
         if rc != 0:
             raise IOError("spl_read_bam(%s): %s" % (path, err.value.decode()))
+        return cls._from_handle(lib, h, xs, groups is not None, read_filter is not None)
+
+    @classmethod
+    def _from_handle(cls, lib, h, xs, groups=False, filtered=False):
+        """Records copied out of a spl_records handle, which is freed."""
         try:
             v = lib.spl_records_get(h).contents
             n, nc, ns = v.n_rec, v.n_cigar, v.n_seg
@@ -199,8 +214,9 @@ class Records:
                       np.ctypeslib.as_array(v.cig_off, shape=(n + 1,)).astype(np.uint32, copy=True),
                       arr(v.cigar, nc, np.uint32), arr(v.seg_chrom, ns, np.int32),
                       np.ctypeslib.as_array(v.seg_off, shape=(ns + 1,)).astype(np.int64, copy=True),
-                      xs=arr(lib.spl_records_xs(h), n, np.uint8) if xs else None)
-            if read_filter is not None:
+                      xs=arr(lib.spl_records_xs(h), n, np.uint8) if xs else None,
+                      group=arr(lib.spl_records_group(h), n, np.int32) if groups else None)
+            if filtered:
                 fc = np.zeros(2, np.int64)
                 lib.spl_records_filter_counts(h, _ptr(fc, L.c_i64p))
                 out.filter_counts = (int(fc[0]), int(fc[1]))
@@ -597,15 +613,65 @@ def _names(chrom_names):
     return (C.c_char_p * max(1, len(chrom_names)))(*[c.encode() for c in chrom_names])
 
 
+class TagGroups:
+    """A tag group table (include/spliser_b200.h, spl_tag_groups, states the rule): records whose first `tag` aux field has
+    value values[i] belong to group groups[i] of n_groups.  Values are str or bytes (str is UTF-8 encoded); integer tags match
+    their decimal text ("1", "-3").  The library checks the table: a bad tag, a repeated value or an out-of-range group raises
+    ValueError when it is used."""
+
+    def __init__(self, tag, values, groups, n_groups):
+        self.tag = tag.encode() if isinstance(tag, str) else bytes(tag)
+        self.values = [v.encode() if isinstance(v, str) else bytes(v) for v in values]
+        self.groups = np.ascontiguousarray(groups, dtype=np.int32)
+        self.n_groups = int(n_groups)
+        if len(self.tag) != 2:
+            raise ValueError("tag must have two characters, got %r" % (tag,))
+        if len(self.groups) != len(self.values):
+            raise ValueError("one group per value")
+        self._off = np.zeros(len(self.values) + 1, np.int64)
+        self._off[1:] = np.cumsum([len(v) for v in self.values])
+        self._blob = np.frombuffer(b"".join(self.values) or b"\0", np.uint8).copy()
+
+    def _c(self):
+        t = L.TagGroupsC()
+        t.tag = self.tag
+        t.n_groups = self.n_groups
+        t.n_values = len(self.values)
+        t.blob = _ptr(self._blob, L.c_u8p)
+        t.offsets = _ptr(self._off, L.c_i64p)
+        t.group = _ptr(self.groups, L.c_i32p) if len(self.groups) else None
+        return t
+
+
+class GroupedSamples:
+    """The samples of one BAM split by a tag group table (Context.load_bam_groups): .samples holds a DeviceSample per group in
+    group order, .counts the records of every group, .no_value the kept records without a value, .unmatched those whose value
+    is in no group.  The samples share one device allocation, freed when the last of them is closed; close() closes them all."""
+
+    def __init__(self, samples, counts, no_value, unmatched):
+        self.samples, self.counts, self.no_value, self.unmatched = samples, counts, no_value, unmatched
+
+    def close(self):
+        for s in self.samples:
+            s.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+
 class DeviceSample:
     """One BAM's alignment records in device memory (Context.load_bam): the extraction + count of process_bam_extract and the
     re-count of recount_bam without reading the file again.  Calls go through the context that loaded it.  A context manager;
     close() frees the device memory.  read_filter: the context's read filter at the load (None = none); a call while the context
     has another one raises SpliserError, since the sample's records would not be the ones a path call reads."""
 
-    def __init__(self, ctx: "Context", h, read_filter: "ReadFilter" = None):
+    def __init__(self, ctx: "Context", h, read_filter: "ReadFilter" = None, xs=False):
         self._ctx, self._h = ctx, h
         self.read_filter = read_filter
+        self.xs = bool(xs)                          # loaded with the XS strand column
 
     @property
     def n_records(self) -> int:
@@ -629,6 +695,14 @@ class DeviceSample:
     def infer_strand(self, chrom_names, genes: "GeneStrands" = None) -> StrandVotes:
         """Context.infer_strand_bam of the loaded BAM.  The XS source (genes=None) needs a sample loaded with xs=True."""
         return self._ctx._infer(self._ctx._lib.spl_sample_infer_strand, self._h, chrom_names, genes)
+
+    def records(self) -> "Records":
+        """The records the sample holds, copied back (spl_sample_fetch_records): seg_chrom is the header reference index of every
+        segment (bam_reference_names order), xs is set for a sample loaded with xs=True."""
+        c = self._ctx
+        h = C.c_void_p()
+        c._check(c._lib.spl_sample_fetch_records(c._h, self._h, C.byref(h)), "spl_sample_fetch_records")
+        return Records._from_handle(c._lib, h, self.xs)
 
     def close(self):
         h, self._h = getattr(self, "_h", None), None
@@ -867,7 +941,25 @@ class Context:
         if rc == L.SPL_ERR_NOMEM:
             raise SampleMemoryError("spl_sample_load_bam(%s): %s" % (bam_path, self._lib.spl_last_error(self._h).decode()))
         self._check(rc, "spl_sample_load_bam")
-        return DeviceSample(self, h, self.read_filter)
+        return DeviceSample(self, h, self.read_filter, xs)
+
+    def load_bam_groups(self, bam_path, groups: TagGroups, xs=False) -> GroupedSamples:
+        """Ingests a BAM once and splits its kept records by the tag group table into one DeviceSample per group, which share one
+        device allocation (include/spliser_b200.h, spl_sample_load_bam_groups).  Raises SampleMemoryError when the split does
+        not fit next to this context's working memory, ValueError for a table that breaks the rule."""
+        G = groups.n_groups
+        hs = (C.c_void_p * max(1, G))()
+        counts = np.zeros(max(1, G) + 2, np.int64)
+        tg = groups._c()
+        rc = self._lib.spl_sample_load_bam_groups(self._h, str(bam_path).encode(), FLAG_XS_STRAND if xs else 0, C.byref(tg),
+                                                  C.cast(hs, C.POINTER(C.c_void_p)), _ptr(counts, L.c_i64p))
+        if rc == L.SPL_ERR_NOMEM:
+            raise SampleMemoryError("spl_sample_load_bam_groups(%s): %s" % (bam_path, self._lib.spl_last_error(self._h).decode()))
+        if rc == -1:
+            raise ValueError("spl_sample_load_bam_groups(%s): %s" % (bam_path, self._lib.spl_last_error(self._h).decode()))
+        self._check(rc, "spl_sample_load_bam_groups")
+        samples = [DeviceSample(self, C.c_void_p(hs[g]), self.read_filter, xs) for g in range(G)]
+        return GroupedSamples(samples, [int(x) for x in counts[:G]], int(counts[G]), int(counts[G + 1]))
 
     # ---- combine re-count ----------------------------------------------------------------------
     @staticmethod
@@ -914,10 +1006,10 @@ class Context:
         return self._take(h)
 
 
-def read_bam(path, chrom_names, threads=0, xs=False, read_filter: ReadFilter = None) -> Records:
+def read_bam(path, chrom_names, threads=0, xs=False, read_filter: ReadFilter = None, groups: "TagGroups" = None) -> Records:
     """The host BAM reader (no GPU): Records.from_bam, under read_filter when given (the result's filter_counts is then
-    (kept, dropped))."""
-    return Records.from_bam(path, chrom_names, threads=threads, xs=xs, read_filter=read_filter)
+    (kept, dropped)), with the tag group of every record in Records.group when groups is given."""
+    return Records.from_bam(path, chrom_names, threads=threads, xs=xs, read_filter=read_filter, groups=groups)
 
 
 def bam_reference_names(path):

@@ -9,8 +9,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libspliser_b200.so")
-SOURCES = ["kernels.cu", "count_fused.cu", "graph_build.cu", "bam_gpu.cu", "strand_votes.cu", "pipeline.cu", "site_graph.cpp", "bam_io.cpp", "host_text.cpp"]
-HEADERS = ["device_types.h", "dev_helpers.cuh", "graph_build.h", "bam_gpu.h", "inflate.h", "site_graph.h", "bam_io.h", "bam_aux.h", "read_filter.h", "junction_filter.h", "strand_votes.h", os.path.join("..", "..", "include", "spliser_b200.h")]
+SOURCES = ["kernels.cu", "count_fused.cu", "graph_build.cu", "bam_gpu.cu", "strand_votes.cu", "group_split.cu", "pipeline.cu", "site_graph.cpp", "bam_io.cpp", "host_text.cpp"]
+HEADERS = ["device_types.h", "dev_helpers.cuh", "graph_build.h", "bam_gpu.h", "inflate.h", "site_graph.h", "bam_io.h", "bam_aux.h", "read_filter.h", "junction_filter.h", "strand_votes.h", "tag_groups.h", "group_split.h", os.path.join("..", "..", "include", "spliser_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-Wall", "-shared"]
 

@@ -13,6 +13,8 @@ Without regtools (not a reference command; regtools' option letters):
                                           [--beta2Cryptic] [--minAnchor 8] [--minIntron 70] [--maxIntron 500000] [--strandFromXS]
                                           [--shallow [-m 0] [-r 10] [-e 0.0]] [--gpus N]
     python -m spliser_b200.cli inferStrandedness -B x.bam [-A genes.gff]
+    python -m spliser_b200.cli combineGroups -B x.bam --tag CB -G groups.tsv -o out [combineBam's -A -t -g --isStranded -s
+                                          --beta2Cryptic --minAnchor --minIntron --maxIntron --strandFromXS --shallow -m -r -e --gpus]
 Every command that reads a BAM also takes [--minMAPQ N] [--excludeFlags F] [--requireFlags F], samtools view's -q / -F / -f
 applied as the BAM is ingested (flags in decimal or 0x hex; include/spliser_b200.h, spl_read_filter, states the rule).
 `junctions` writes the junction BED12 that `regtools junctions extract` would feed `process` with; `processBam` is
@@ -22,7 +24,8 @@ with --isStranded -s.  `combineBam` is `processBam` for every sample of a sample
 `combine` (`combineShallow` with --shallow), with every BAM read once: the records stay in GPU memory for the re-count.
 `inferStrandedness` tells which of --isStranded -s fr, -s rf or an unstranded run fits the library (one vote per record,
 against the annotation's genes or the XS tag); `processBam` and `combineBam` take --isStranded -s auto to infer it over the
-same ingest and run with its verdict.
+same ingest and run with its verdict.  `combineGroups` is `combineBam` over the groups of one BAM that an aux tag tells apart
+(read groups, cell-barcode clusters, haplotypes), split on the GPU from one ingest instead of one BAM per group.
 
 What stays in Python is what the reference does in text: BED12 parsing and its filters (S:255-288), the
 annotation and gene lookup (S:50-173), the TSV writers (S:641-664, S:722-740) and the lock-step merge of
@@ -238,10 +241,11 @@ def _chrom_list(annotation, inBAM):
 
 
 def _process_bam_sample(extract, inBAM, tsv_path, annotation, bounds, qChrom, maxIntronSize, isStranded, strandedType, isbeta2Cryptic,
-                        minAnchor, minIntron, maxIntron, strandFromXS):
+                        minAnchor, minIntron, maxIntron, strandFromXS, chroms=None):
     """processBam after the annotation load.  extract(chrom_names, flags, min_anchor, min_intron, max_intron, qchrom=, gene_bounds=,
-    window_max_intron=) answers like Context.process_bam_extract of this BAM (or DeviceSample.process_extract of it loaded)."""
-    chroms = _chrom_list(annotation, inBAM)
+    window_max_intron=) answers like Context.process_bam_extract of this BAM (or DeviceSample.process_extract of it loaded).
+    chroms: _chrom_list(annotation, inBAM) when the caller has it already."""
+    chroms = _chrom_list(annotation, inBAM) if chroms is None else chroms
     flags = api.mode_flags(isStranded, strandedType, isbeta2Cryptic) | (api.FLAG_XS_STRAND if strandFromXS else 0)
     junc, table = extract(chroms, flags, minAnchor, minIntron, maxIntron, qchrom=qChrom, gene_bounds=bounds,
                           window_max_intron=int(maxIntronSize))
@@ -485,8 +489,26 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
     read_filter (api.ReadFilter) applies to every rank's context: the samples are loaded, voted on and counted under it."""
     print("Combining samples from their BAMs...")
     titles, tsv_paths, bam_paths = _read_samples_file(samplesFile, shallow)
-    n = len(titles)
     annotation = load_annotation(annotationFile, "All") if annotationFile is not None else None
+
+    def load(rank, c, k, xs):
+        try:
+            s = c.load_bam(bam_paths[k], xs=xs)
+        except api.SampleMemoryError:
+            return None
+        _report_filter(c, bam_paths[k], read_filter)
+        return s
+    _combine_resident(titles, tsv_paths, bam_paths, outputPath, annotation, qGene, isStranded, strandedType, isbeta2Cryptic, minAnchor,
+                      minIntron, maxIntron, strandFromXS, shallow, minSamples, minReads, minSSE, devices, context_factory, read_filter, load)
+
+
+def _combine_resident(titles, tsv_paths, bam_paths, outputPath, annotation, qGene, isStranded, strandedType, isbeta2Cryptic, minAnchor,
+                      minIntron, maxIntron, strandFromXS, shallow, minSamples, minReads, minSSE, devices, context_factory, read_filter,
+                      load):
+    """combineBam's orchestration over samples that are held in GPU memory: load(rank, ctx, k, xs) -> the DeviceSample of sample
+    k on that rank's context, or None for the path route (process_bam_extract / recount_bam on bam_paths[k]).  The samples of
+    rank r are dist.samples_of(r, n_ranks, n), asked for in order on the rank's host thread."""
+    n = len(titles)
     make = context_factory or api.Context
     devs = [0] if not devices else list(devices)
     n_ranks = len(devs)
@@ -495,12 +517,18 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
     auto = isStranded and strandedType == "auto"
     votes = [None] * n
     flags = None if auto else api.mode_flags(isStranded, strandedType, False, combine=True)
+    chrom_lists = {}
+
+    def chroms_of(k):                               # the header is read once per BAM (combineGroups: one BAM for every sample)
+        if bam_paths[k] not in chrom_lists:
+            chrom_lists[bam_paths[k]] = _chrom_list(annotation, bam_paths[k])
+        return chrom_lists[bam_paths[k]]
 
     def extract(rank, k):
         c = ctxs[rank]
         ex = resident[k].process_extract if resident[k] is not None else functools.partial(c.process_bam_extract, bam_paths[k])
         _process_bam_sample(ex, bam_paths[k], tsv_paths[k], annotation, None, "All", 0, isStranded, strandedType, isbeta2Cryptic,
-                            minAnchor, minIntron, maxIntron, strandFromXS)
+                            minAnchor, minIntron, maxIntron, strandFromXS, chroms_of(k))
 
     def process_rank(rank):
         mine = samples_of(rank, n_ranks, n)
@@ -510,13 +538,9 @@ def combineBam(samplesFile, outputPath, annotationFile=None, aType="gene", qGene
         for k in mine:
             genes = None
             if auto:
-                chroms = _chrom_list(annotation, bam_paths[k])
+                chroms = chroms_of(k)
                 genes = api.gene_strands(annotation, chroms) if annotation is not None else None
-            try:
-                resident[k] = c.load_bam(bam_paths[k], xs=strandFromXS or (auto and genes is None))
-                _report_filter(c, bam_paths[k], read_filter)
-            except api.SampleMemoryError:
-                pass
+            resident[k] = load(rank, c, k, strandFromXS or (auto and annotation is None))
             if not auto:
                 extract(rank, k)
             elif resident[k] is not None:
@@ -567,6 +591,94 @@ def _pooled_verdict(titles, votes):
     return _verdict_flags(pooled, "the pooled samples")
 
 
+# ------------------------------------------------------------------------------------------------ samples told apart by a tag
+class GroupsFileError(ValueError):
+    """A groups file (value <TAB> title per line) that cannot be read; the message names the line."""
+
+
+def _tag_value(x):
+    if len(x) != 2 or not (x[0].isascii() and x[0].isalpha()) or not (x[1].isascii() and x[1].isalnum()):
+        raise argparse.ArgumentTypeError("a tag is two characters, [A-Za-z][A-Za-z0-9], got %r" % x)
+    return x
+
+
+def read_groups_file(path):
+    """(values, group of every value, titles) of a groups file: lines `value <TAB> title`; many values may share a title (a
+    barcode -> cluster table).  The group order is the order in which titles first appear.  GroupsFileError names the line
+    that has not exactly two non-empty columns, has a value the library refuses (more than 255 bytes, NUL; TAB and newline cannot
+    occur), repeats a value, or has a title with '/', TAB or NUL."""
+    values, groups, titles, at, seen = [], [], [], {}, {}
+    with open(path, encoding="utf-8", newline="") as fh:
+        for ln, line in enumerate(fh, 1):
+            cols = line.rstrip("\r\n").split("\t")
+            if len(cols) != 2 or not cols[0] or not cols[1]:
+                raise GroupsFileError("%s line %d: not two tab-separated columns (value <TAB> title)" % (path, ln))
+            value, title = cols
+            if len(value.encode()) > 255 or "\0" in value:
+                raise GroupsFileError("%s line %d: value %r is longer than 255 bytes or contains NUL" % (path, ln, value))
+            if "/" in title or "\0" in title:
+                raise GroupsFileError("%s line %d: title %r contains '/', TAB or NUL" % (path, ln, title))
+            if value in seen:
+                raise GroupsFileError("%s line %d: value %r repeats line %d" % (path, ln, value, seen[value]))
+            seen[value] = ln
+            if title not in at:
+                at[title] = len(titles)
+                titles.append(title)
+            values.append(value)
+            groups.append(at[title])
+    if not titles:
+        raise GroupsFileError("%s: no groups" % path)
+    return values, groups, titles
+
+
+def _rank_table(tag, values, groups, mine):
+    """The tag group table of the groups `mine` (global indices, in order): their values, renumbered 0 .. len(mine) - 1."""
+    local = {g: i for i, g in enumerate(mine)}
+    keep = [(v, local[g]) for v, g in zip(values, groups) if g in local]
+    return api.TagGroups(tag, [v for v, _ in keep], [g for _, g in keep], len(mine))
+
+
+def combineGroups(inBAM, tag, groupsFile, outputPath, annotationFile=None, aType="gene", qGene="All", isStranded=False,
+                  strandedType=None, isbeta2Cryptic=False, minAnchor=8, minIntron=70, maxIntron=500000, strandFromXS=False,
+                  shallow=False, minSamples=0, minReads=10, minSSE=0.0, devices=None, context_factory=None, read_filter=None):
+    """The groups of one BAM told apart by an aux tag (read groups RG, cell-barcode clusters CB, haplotypes HP) as the samples of
+    combineBam: the BAM is ingested once per rank and split on the GPU (Context.load_bam_groups; include/spliser_b200.h,
+    spl_tag_groups, states the rule).  out.<title>.SpliSER.tsv is what processBam writes on a BAM of that group's records, and
+    out.combined.tsv what combineBam writes over those BAMs in group order, the order in which titles first appear in the groups
+    file.  With several devices rank r splits off the groups dist.samples_of(r, n_ranks, n_groups) only.  A split that does not
+    fit raises SampleMemoryError naming the bytes it needs; there is no path route for a group."""
+    print("Combining the groups of one BAM...")
+    values, groups, titles = read_groups_file(groupsFile)
+    n = len(titles)
+    tsv_paths = ["%s.%s.SpliSER.tsv" % (outputPath, t) for t in titles]
+    annotation = load_annotation(annotationFile, "All") if annotationFile is not None else None
+    n_ranks = len(devices) if devices else 1
+    splits, counts, no_value, kept = {}, [0] * n, [0], [0, 0]
+
+    def load(rank, c, k, xs):
+        if rank not in splits:
+            mine = samples_of(rank, n_ranks, n)
+            splits[rank] = (mine, c.load_bam_groups(inBAM, _rank_table(tag, values, groups, mine), xs=xs))
+            got = splits[rank][1]
+            for g, cnt in zip(mine, got.counts):
+                counts[g] = cnt
+            no_value[0] = got.no_value
+            kept[:] = c.last_read_filter()
+        mine, got = splits[rank]
+        return got.samples[mine.index(k)]
+    try:
+        _combine_resident(titles, tsv_paths, [inBAM] * n, outputPath, annotation, qGene, isStranded, strandedType, isbeta2Cryptic,
+                          minAnchor, minIntron, maxIntron, strandFromXS, shallow, minSamples, minReads, minSSE, devices, context_factory,
+                          read_filter, load)
+    finally:
+        for _, got in splits.values():
+            got.close()
+    print("Records per group ({}):\t{}\tno value {}\tvalue in no group {}".format(
+        tag, "\t".join("%s %d" % x for x in zip(titles, counts)), no_value[0], kept[0] - sum(counts) - no_value[0]))
+    if read_filter is not None:
+        print("Read filter {}:\tkept {}\tdropped {}".format(inBAM, *kept))
+
+
 # ------------------------------------------------------------------------------------------------ main
 def _mapq_value(x):
     v = int(x, 0)
@@ -592,7 +704,7 @@ def _add_read_filter_options(p):
                    help="keep records with all of these FLAG bits (samtools -f), e.g. 0x2")
 
 
-READ_COMMANDS = ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam", "inferStrandedness")
+READ_COMMANDS = ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam", "inferStrandedness", "combineGroups")
 
 
 def main(argv=None):
@@ -680,6 +792,29 @@ def main(argv=None):
     cb.add_argument("-e", "--minSSE", dest="minSSE", nargs="?", default=0.00, type=float)
     cb.add_argument("--gpus", dest="n_gpus", nargs="?", default=1, type=int,
                     help="hold and count the samples on this many GPUs (sharded by sample)")
+    cg = sub.add_parser("combineGroups", help="combineBam over the groups of one BAM told apart by an aux tag, with one ingest")
+    cg.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
+    cg.add_argument("--tag", dest="tag", required=True, type=_tag_value, help="the aux tag that tells the groups apart, e.g. RG, CB, HP")
+    cg.add_argument("-G", "--groupsFile", dest="groupsFile", required=True,
+                    help="value <TAB> title per line; values that share a title form one group, in the order titles first appear")
+    cg.add_argument("-o", "--outputPath", dest="outputPath", required=True)
+    cg.add_argument("-A", "--annotationFile", dest="annotationFile", required=False)
+    cg.add_argument("-t", "--annotationType", dest="aType", nargs="?", default="gene", type=str)
+    cg.add_argument("-g", "--gene", dest="qGene", nargs="?", default="All", type=str)
+    cg.add_argument("--isStranded", dest="isStranded", default=False, action="store_true")
+    cg.add_argument("-s", "--strandedType", dest="strandedType", nargs="?", type=str)
+    cg.add_argument("--beta2Cryptic", dest="isbeta2Cryptic", default=False, action="store_true")
+    cg.add_argument("--minAnchor", dest="minAnchor", default=8, type=int)
+    cg.add_argument("--minIntron", dest="minIntron", default=70, type=int)
+    cg.add_argument("--maxIntron", dest="maxIntron", default=500000, type=int)
+    cg.add_argument("--strandFromXS", dest="strandFromXS", default=False, action="store_true",
+                    help="junction strands from the aligner's XS tag; the count still follows --isStranded -s")
+    cg.add_argument("--shallow", dest="shallow", default=False, action="store_true", help="merge as combineShallow")
+    cg.add_argument("-m", "--minSamples", dest="minSamples", nargs="?", default=0, type=int)
+    cg.add_argument("-r", "--minReads", dest="minReads", nargs="?", default=10, type=int)
+    cg.add_argument("-e", "--minSSE", dest="minSSE", nargs="?", default=0.00, type=float)
+    cg.add_argument("--gpus", dest="n_gpus", nargs="?", default=1, type=int,
+                    help="split and count the groups on this many GPUs (sharded by group; each GPU ingests the BAM once)")
     inf = sub.add_parser("inferStrandedness", help="the library type (--isStranded -s fr|rf, or unstranded) from the BAM")
     inf.add_argument("-B", "--BAMFile", dest="inBAM", required=True)
     inf.add_argument("-A", "--annotationFile", dest="annotationFile", required=False,
@@ -693,13 +828,13 @@ def main(argv=None):
         rf = api.ReadFilter(kwargs.pop("minMAPQ"), kwargs.pop("excludeFlags"), kwargs.pop("requireFlags"))
         if not rf.is_none:
             kwargs["read_filter"] = rf
-    if command in ("combine", "combineShallow", "combineBam"):
+    if command in ("combine", "combineShallow", "combineBam", "combineGroups"):
         kwargs["devices"] = list(range(max(1, kwargs.pop("n_gpus") or 1)))
     if command in ("process", "processBam") and kwargs.get("qGene") != "All" and (kwargs.get("annotationFile") is None or kwargs.get("maxIntronSize") is None):
         parser.error("--gene requires --annotationFile and --maxIntronSize")                      # S:1350-1353
-    elif command == "combineBam" and kwargs.get("qGene") != "All" and kwargs.get("annotationFile") is None:
+    elif command in ("combineBam", "combineGroups") and kwargs.get("qGene") != "All" and kwargs.get("annotationFile") is None:
         parser.error("--gene requires --annotationFile (the Gene column comes from it)")
-    elif command in ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
+    elif command in ("process", "combine", "combineShallow", "junctions", "processBam", "combineBam", "combineGroups") and kwargs.get("isStranded") and kwargs.get("strandedType") is None:
         parser.error("--isStranded requires parameter --strandedType/-s as fr or rf")            # S:1354-1355
     elif command == "junctions" and kwargs.get("strandFromXS") and kwargs.get("isStranded"):
         parser.error("--strandFromXS and --isStranded name two strand sources for the junction table")
@@ -711,11 +846,16 @@ def main(argv=None):
         combineShallow(**kwargs)
     elif command == "junctions":
         junctions(**kwargs)
-    elif command in ("processBam", "combineBam", "inferStrandedness"):
+    elif command in ("processBam", "combineBam", "inferStrandedness", "combineGroups"):
         try:
-            {"processBam": processBam, "combineBam": combineBam, "inferStrandedness": inferStrandedness}[command](**kwargs)
-        except StrandednessError as e:
+            {"processBam": processBam, "combineBam": combineBam, "inferStrandedness": inferStrandedness,
+             "combineGroups": combineGroups}[command](**kwargs)
+        except (StrandednessError, GroupsFileError) as e:
             parser.error(str(e))
+        except api.SampleMemoryError as e:
+            if command != "combineGroups":
+                raise
+            parser.error("the groups do not fit in GPU memory: %s" % e)
     else:
         parser.error("command must be process, combine, combineShallow, junctions, processBam, combineBam or inferStrandedness "
                      "(output is unchanged Python in the reference)")

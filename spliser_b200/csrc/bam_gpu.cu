@@ -14,8 +14,9 @@
 //                      Any broken link (or a feature this path does not parse: CG-tag long CIGARs) -> the caller falls
 //                      back to the host reader (bam_io.cpp).
 //   k_bam_fill         one warp per accepted member: the kept records (offsets listed by the counting walk) are written out
-//                      round-robin by the lanes: POS, FLAG, chromosome and CIGAR (k_bam_fill<true>: and the XS strand, from
-//                      a walk of the record's aux fields by the same lane)
+//                      round-robin by the lanes: POS, FLAG, chromosome and CIGAR (k_bam_fill<true, *>: and the XS strand, from
+//                      a walk of the record's aux fields by the same lane; k_bam_fill<*, true>: and the record's tag group,
+//                      looked up in the tag group table by the same lane, tag_groups.h)
 //   k_bam_segments     chromosome boundaries of the record arrays (a coordinate-sorted BAM has one segment per reference)
 // Kept records follow the host reader: mapped to a caller chromosome, with at least one CIGAR operator (bam_io.cpp), and
 // through the read filter (read_filter.h; the rule is in include/spliser_b200.h, spl_read_filter).  The counting walk counts
@@ -33,6 +34,7 @@
 #include "device_types.h"
 #include "inflate.h"
 #include "read_filter.h"
+#include "tag_groups.h"
 
 namespace spl {
 
@@ -167,11 +169,12 @@ __global__ void __launch_bounds__(128) k_bam_walk(const uint8_t* __restrict__ u,
 // second pass, one WARP per accepted member: the lanes take the kept records of the member round-robin from the offset list
 // the counting walk left, so neighbouring lanes write neighbouring records (the per-thread walk wrote with a stride of
 // ~1,000 records between lanes)
-template <bool XS>
+template <bool XS, bool GRP>
 __global__ void __launch_bounds__(256) k_bam_fill(const uint8_t* __restrict__ u, const BgzfMember* __restrict__ mem, uint32_t n_mem,
                                                   const int32_t* __restrict__ refmap, const WalkOut* __restrict__ wo,
                                                   const uint64_t* __restrict__ rec_base, const uint64_t* __restrict__ cig_base,
-                                                  const uint32_t* __restrict__ kept, DevRecordArrays out) {
+                                                  const uint32_t* __restrict__ kept, DevRecordArrays out, int32_t* __restrict__ grp,
+                                                  TagTableView tags) {
     const uint32_t m = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (m >= n_mem || rec_base[m] == ~0ull) return;
@@ -198,9 +201,10 @@ __global__ void __launch_bounds__(256) k_bam_fill(const uint8_t* __restrict__ u,
             out.cig_off[ri] = (uint32_t)c0;
             const uint64_t cig = o + 36 + h.l_name;
             for (uint32_t q = 0; q < nc; ++q) out.cigar[c0 + q] = ld32u(u, cig + 4ull * q);
-            if (XS) {                                                  // aux fields: from the end of QUAL to the end of the record
+            if (XS || GRP) {                                           // aux fields: from the end of QUAL to the end of the record
                 const uint64_t aux = cig + 4ull * nc + ((uint64_t)h.l_seq + 1) / 2 + (uint64_t)h.l_seq;
-                out.xs[ri] = aux_xs_strand(u + aux, u + o + 4 + h.bs);  // aux <= the record end: the counting walk checked it
+                if (XS) out.xs[ri] = aux_xs_strand(u + aux, u + o + 4 + h.bs);   // aux <= the record end: the counting walk checked it
+                if (GRP) grp[ri] = tag_group_of(tags, u + aux, u + o + 4 + h.bs);
             }
         }
         ci += tot;
@@ -230,7 +234,7 @@ __global__ void k_set_u32(uint32_t* p, uint32_t v) { *p = v; }
 
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream, bool comp_uploaded,
-                   bool want_xs, const ReadFilter& rf, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
+                   bool want_xs, const ReadFilter& rf, const TagTableView* tags, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err) {
     cudaStream_t st = (cudaStream_t)stream;
     const uint32_t n_mem = (uint32_t)members.size();
     cnt = BamGpuCounts{};
@@ -299,18 +303,24 @@ int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const
         auto take = [&](size_t bytes) { off = (off + 255) & ~(size_t)255; const size_t o = off; off += bytes; return o; };
         const size_t o_pos = take((nrec + 4) * 4), o_flag = take((nrec + 4) * 2), o_off = take((nrec + 4) * 4), o_cig = take((ncig + 4) * 4),
                      o_chr = take((nrec + 4) * 4), o_sf = take(BAMGPU_MAX_SEG * 8), o_sc = take(BAMGPU_MAX_SEG * 4), o_ns = take(16),
-                     o_xs = want_xs ? take(nrec + 4) : 0;
+                     o_xs = want_xs ? take(nrec + 4) : 0, o_grp = tags ? take((nrec + 4) * 4) : 0;
         if (mem.rec.reserve(off + 256) != cudaSuccess) { cudaGetLastError(); err = "not enough device memory for the record arrays"; return BAMGPU_FALLBACK; }
         char* rb = (char*)mem.rec.p;
         out.pos = (int32_t*)(rb + o_pos); out.flag = (uint16_t*)(rb + o_flag); out.cig_off = (uint32_t*)(rb + o_off);
         out.cigar = (uint32_t*)(rb + o_cig); out.chrom = (int32_t*)(rb + o_chr);
         out.xs = want_xs ? (uint8_t*)(rb + o_xs) : nullptr;
+        int32_t* d_grp = tags ? (int32_t*)(rb + o_grp) : nullptr;
+        cnt.grp = d_grp;
         uint64_t* d_sf = (uint64_t*)(rb + o_sf); int32_t* d_sc = (int32_t*)(rb + o_sc); uint32_t* d_ns = (uint32_t*)(rb + o_ns);
         BG_CU(cudaMemcpyAsync(d_rbase, rbase.data(), (size_t)n_mem * 8, cudaMemcpyHostToDevice, st));
         BG_CU(cudaMemcpyAsync(d_cbase, cbase.data(), (size_t)n_mem * 8, cudaMemcpyHostToDevice, st));
         BG_CU(cudaMemsetAsync(d_ns, 0, 16, st));
-        if (want_xs) { SPL_LAUNCH; k_bam_fill<true><<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out); }
-        else { SPL_LAUNCH; k_bam_fill<false><<<(n_mem + 7) / 8, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out); }
+        const unsigned nb = (n_mem + 7) / 8;
+        const TagTableView tt = tags ? *tags : TagTableView{};
+        if (tags && want_xs) { SPL_LAUNCH; k_bam_fill<true, true><<<nb, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out, d_grp, tt); }
+        else if (tags) { SPL_LAUNCH; k_bam_fill<false, true><<<nb, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out, d_grp, tt); }
+        else if (want_xs) { SPL_LAUNCH; k_bam_fill<true, false><<<nb, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out, d_grp, tt); }
+        else { SPL_LAUNCH; k_bam_fill<false, false><<<nb, 256, 0, st>>>(d_u, d_mem, n_mem, d_refmap, d_wo, d_rbase, d_cbase, d_kept, out, d_grp, tt); }
         { SPL_LAUNCH; k_set_u32<<<1, 1, 0, st>>>(out.cig_off + nrec, (uint32_t)ncig); }
         if (nrec) { SPL_LAUNCH; k_bam_segments<<<(unsigned)((nrec + 255) / 256), 256, 0, st>>>(out.chrom, nrec, d_ns, d_sf, d_sc, BAMGPU_MAX_SEG); }
         BG_CU(cudaGetLastError());

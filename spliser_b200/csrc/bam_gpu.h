@@ -8,6 +8,7 @@
 
 #include "graph_build.h"   // GbBuf
 #include "read_filter.h"
+#include "tag_groups.h"
 
 namespace spl {
 
@@ -26,7 +27,7 @@ struct DevRecordArrays {     // what DevRecords points at, plus the chromosome o
     uint8_t* xs = nullptr;   // strand of every record from its XS tag ('+', '-', '?'; bam_aux.h), only when the ingest was asked for it
 };
 
-struct BamGpuMem { GbBuf comp, unc, tab, rec, list; };
+struct BamGpuMem { GbBuf comp, unc, tab, rec, list, tags; };
 
 struct BamGpuCounts {
     uint64_t n_rec = 0, n_cigar = 0;
@@ -34,6 +35,7 @@ struct BamGpuCounts {
     std::vector<int32_t> seg_chrom;
     std::vector<int64_t> seg_off;
     double h2d_bytes = 0;
+    int32_t* grp = nullptr;  // device: tag group of every record (tag_groups.h: a group, TAG_NO_VALUE or TAG_NO_GROUP), only with a table
 };
 
 constexpr uint32_t BAMGPU_MAX_SEG = 1u << 16;
@@ -50,6 +52,8 @@ std::string bam_scan(const uint8_t* file, size_t fsz, int32_t n_chrom, const cha
 int bam_gpu_ingest(BamGpuMem& mem, const uint8_t* file_pinned, size_t fsz, const std::vector<BgzfMember>& members, uint64_t total_u,
                    uint64_t first_record, int32_t n_ref, const std::vector<int32_t>& refmap, void* stream,
                    bool comp_uploaded /* mem.comp already holds the file image (copy queued on `stream`) */,
-                   bool want_xs /* fill out.xs */, const ReadFilter& rf, DevRecordArrays& out, BamGpuCounts& cnt, std::string& err);
+                   bool want_xs /* fill out.xs */, const ReadFilter& rf,
+                   const TagTableView* tags /* NULL, or a table in device memory: fill cnt.grp */, DevRecordArrays& out, BamGpuCounts& cnt,
+                   std::string& err);
 
 }  // namespace spl

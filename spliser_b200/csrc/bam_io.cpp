@@ -87,8 +87,60 @@ std::vector<int32_t> map_references(const std::vector<std::string>& ref_names, i
     return refmap;
 }
 
+TagTableView TagTableHost::view() const {
+    TagTableView v;
+    v.t0 = t0; v.t1 = t1; v.mask = mask;
+    v.slot = slot.data(); v.off = off.data(); v.blob = blob.data(); v.group = group.data();
+    return v;
+}
+
+std::string build_tag_table(const spl_tag_groups* g, TagTableHost& out) {
+    out = TagTableHost{};
+    if (!g) return "tag group table is NULL";
+    auto alpha = [](char c) { return (c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z'); };
+    auto alnum = [&](char c) { return alpha(c) || (c >= '0' && c <= '9'); };
+    if (!alpha(g->tag[0]) || !alnum(g->tag[1])) return "tag must match [A-Za-z][A-Za-z0-9]";
+    if (g->n_groups < 1 || g->n_groups > 65535) return "n_groups " + std::to_string(g->n_groups) + " outside 1..65535";
+    if (g->n_values < 0 || g->n_values > (int64_t)1 << 26) return "n_values " + std::to_string(g->n_values) + " outside 0..2^26";
+    const int64_t nv = g->n_values;
+    if (nv > 0 && (!g->offsets || !g->blob || !g->group)) return "the table's arrays are NULL";
+    if (nv > 0 && g->offsets[0] != 0) return "offsets[0] must be 0";
+    out.t0 = (uint8_t)g->tag[0]; out.t1 = (uint8_t)g->tag[1]; out.n_groups = g->n_groups;
+    uint32_t slots = 16;
+    while (slots < 2 * (uint64_t)nv) slots <<= 1;
+    out.mask = slots - 1;
+    out.slot.assign(slots, 0);
+    out.off.assign((size_t)nv + 1, 0);
+    out.group.assign((size_t)std::max<int64_t>(nv, 1), 0);
+    for (int64_t v = 0; v < nv; ++v) {
+        const int64_t a = g->offsets[v], b = g->offsets[v + 1];
+        if (b <= a) return "value " + std::to_string(v) + " is empty";
+        if (b - a > (int64_t)TAG_MAX_VALUE) return "value " + std::to_string(v) + " is longer than 255 bytes";
+        for (int64_t k = a; k < b; ++k) {
+            const uint8_t c = g->blob[k];
+            if (c == 0 || c == '\t' || c == '\n') return "value " + std::to_string(v) + " contains NUL, TAB or newline";
+        }
+        if (g->group[v] < 0 || g->group[v] >= g->n_groups) return "value " + std::to_string(v) + " maps to group " +
+                                                                 std::to_string(g->group[v]) + ", outside 0.." + std::to_string(g->n_groups - 1);
+        if (out.blob.size() + (size_t)(b - a) > (size_t)UINT32_MAX) return "the values add up to more than 2^32 - 1 bytes";
+        out.off[(size_t)v] = (uint32_t)out.blob.size();
+        out.blob.insert(out.blob.end(), g->blob + a, g->blob + b);
+        out.off[(size_t)v + 1] = (uint32_t)out.blob.size();
+        out.group[(size_t)v] = g->group[v];
+        const TagTableView t = out.view();
+        const uint8_t* p = out.blob.data() + out.off[(size_t)v];
+        const uint32_t n = (uint32_t)(b - a);
+        if (tag_lookup(t, p, n) != TAG_NO_GROUP) return "value " + std::to_string(v) + " repeats an earlier value";
+        uint32_t s = tag_hash(p, n) & out.mask;
+        while (out.slot[s]) s = (s + 1) & out.mask;
+        out.slot[s] = (uint32_t)v + 1;
+    }
+    if (out.blob.empty()) out.blob.push_back(0);
+    return "";
+}
+
 std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, BamRecords& out, bool want_xs,
-                     std::vector<std::string>* header_order, const ReadFilter& rf) {
+                     std::vector<std::string>* header_order, const ReadFilter& rf, const TagTableView* tags) {
     out = BamRecords();
     if (header_order) header_order->clear();
     const int fd = open(path, O_RDONLY);
@@ -229,6 +281,7 @@ std::string read_bam(const char* path, int32_t n_chrom, const char* const* chrom
             out.pos.push_back(pos0 + 1);
             out.flag.push_back(flag);
             if (want_xs) out.xs.push_back(aux ? aux_xs_strand(aux, r + bs) : (uint8_t)'?');
+            if (tags) out.grp.push_back(aux ? tag_group_of(*tags, aux, r + bs) : TAG_NO_VALUE);
             const size_t c0 = out.cigar.size();
             out.cigar.resize(c0 + n_cig);
             memcpy(out.cigar.data() + c0, cig, (size_t)n_cig * 4);   // BAM is little-endian, so is every host we build for
@@ -480,7 +533,17 @@ struct spl_records {
     spl::BamRecords r;
     spl_records_view v;
     bool has_xs = false;    // read by spl_read_bam_xs: r.xs holds one strand byte per record
+    bool has_grp = false;   // read by spl_read_bam_groups: r.grp holds the group of every record
 };
+
+spl_records* spl::records_handle(spl::BamRecords&& r, bool has_xs) {
+    spl_records* h = new (std::nothrow) spl_records();
+    if (!h) return nullptr;
+    h->r = std::move(r);
+    h->v = h->r.view();
+    h->has_xs = has_xs;
+    return h;
+}
 
 extern "C" {
 
@@ -515,12 +578,12 @@ int spl_write_bam(const char* path, int32_t n_ref, const char* const* ref_names,
 
 namespace {
 int read_bam_handle(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, bool want_xs, spl_records** out,
-                    char* err, int err_len, const spl::ReadFilter& rf = spl::ReadFilter{}) {
+                    char* err, int err_len, const spl::ReadFilter& rf = spl::ReadFilter{}, const spl::TagTableView* tags = nullptr) {
     if (!out || !path) return SPL_ERR_ARG;
     *out = nullptr;
     spl_records* h = new (std::nothrow) spl_records();
     if (!h) return SPL_ERR_NOMEM;
-    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r, want_xs, nullptr, rf);
+    const std::string e = spl::read_bam(path, n_chrom, chrom_names, n_threads, h->r, want_xs, nullptr, rf, tags);
     if (!e.empty()) {
         if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
         delete h;
@@ -528,6 +591,7 @@ int read_bam_handle(const char* path, int32_t n_chrom, const char* const* chrom_
     }
     h->v = h->r.view();
     h->has_xs = want_xs;
+    h->has_grp = tags != nullptr;
     *out = h;
     return SPL_OK;
 }
@@ -555,6 +619,22 @@ int spl_read_bam_filtered(const char* path, int32_t n_chrom, const char* const* 
     }
     return read_bam_handle(path, n_chrom, chrom_names, n_threads, want_xs != 0, out, err, err_len, rf);
 }
+
+int spl_read_bam_groups(const char* path, int32_t n_chrom, const char* const* chrom_names, int n_threads, const spl_read_filter* filter,
+                        int want_xs, const spl_tag_groups* groups, spl_records** out, char* err, int err_len) {
+    if (out) *out = nullptr;
+    spl::ReadFilter rf;
+    std::string e;
+    spl::TagTableHost t;
+    if ((filter && !spl::read_filter_from(*filter, rf, e)) || !(e = spl::build_tag_table(groups, t)).empty()) {
+        if (err && err_len > 0) snprintf(err, (size_t)err_len, "%s", e.c_str());
+        return SPL_ERR_ARG;
+    }
+    const spl::TagTableView tv = t.view();
+    return read_bam_handle(path, n_chrom, chrom_names, n_threads, want_xs != 0, out, err, err_len, rf, &tv);
+}
+
+const int32_t* spl_records_group(const spl_records* r) { return r && r->has_grp ? r->r.grp.data() : nullptr; }
 
 int spl_records_filter_counts(const spl_records* r, int64_t counts[2]) {
     if (!r || !counts) return SPL_ERR_ARG;

@@ -25,6 +25,7 @@
 #include "bam_io.h"
 #include "device_types.h"
 #include "graph_build.h"
+#include "group_split.h"
 #include "junction_filter.h"
 #include "site_graph.h"
 #include "strand_votes.h"
@@ -232,6 +233,8 @@ struct spl_ctx {
     size_t h_stage_bytes = 0;
     // device-side BAM ingest
     BamGpuMem bgm;
+    GroupSplitMem gsm;              // tag group split: the host reader's upload, the sort scratch, the tables (spl_sample_load_bam_groups;
+                                    // released when the split returns, so that the context holds none of it between calls)
     DevRecordArrays dev_rec{};
     bool rec_on_device = false;     // the next load takes its records from dev_rec (no host arrays, no upload)
     spl_result* pending = nullptr;  // result whose structure arrays are already on their way to the host (device-built graph)
@@ -1328,7 +1331,8 @@ int load_common(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int6
 // want_xs: ctx->dev_rec.xs receives the XS strand of every record as well.  header_order != NULL: chrom_names is ignored, every
 // record keeps its header reference index (no reference is dropped) and *header_order receives the reference names.
 int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const char* const* chrom_names, BamGpuCounts& cnt,
-                      spl_records_view& view, bool* fallback, bool want_xs = false, std::vector<std::string>* header_order = nullptr) {
+                      spl_records_view& view, bool* fallback, bool want_xs = false, std::vector<std::string>* header_order = nullptr,
+                      const TagTableHost* tags = nullptr) {
     *fallback = false;
     if (const char* f = std::getenv("SPLISER_HOST_BAM")) if (f[0] == '1') { *fallback = true; return SPL_OK; }
     const int fd = open(path, O_RDONLY);
@@ -1387,8 +1391,25 @@ int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const cha
                              header_order);
     if (!e.empty()) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_IO, "%s", e.c_str()); }
     if (header_order) for (int32_t r = 0; r < n_ref; ++r) refmap[(size_t)r] = r;
+    TagTableView d_tags;                                               // the tag group table in device memory
+    if (tags) {
+        const size_t b_slot = tags->slot.size() * 4, b_off = tags->off.size() * 4, b_grp = tags->group.size() * 4;
+        const size_t o_off = (b_slot + 255) & ~(size_t)255, o_grp = (o_off + b_off + 255) & ~(size_t)255, o_blob = (o_grp + b_grp + 255) & ~(size_t)255;
+        if (ctx->bgm.tags.reserve(o_blob + tags->blob.size() + 16) != cudaSuccess) {
+            cudaGetLastError(); cudaStreamSynchronize(ctx->stream);
+            return ctx->fail(SPL_ERR_NOMEM, "not enough device memory for the tag group table");
+        }
+        char* tb = (char*)ctx->bgm.tags.p;
+        CU(cudaMemcpyAsync(tb, tags->slot.data(), b_slot, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(tb + o_off, tags->off.data(), b_off, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(tb + o_grp, tags->group.data(), b_grp, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemcpyAsync(tb + o_blob, tags->blob.data(), tags->blob.size(), cudaMemcpyHostToDevice, ctx->stream));
+        d_tags = tags->view();
+        d_tags.slot = (const uint32_t*)tb; d_tags.off = (const uint32_t*)(tb + o_off);
+        d_tags.group = (const int32_t*)(tb + o_grp); d_tags.blob = (const uint8_t*)(tb + o_blob);
+    }
     const int rc = bam_gpu_ingest(ctx->bgm, (const uint8_t*)ctx->h_file, fsz, members, total_u, first_record, n_ref, refmap, ctx->stream,
-                                  uploaded, want_xs, ctx->rf, ctx->dev_rec, cnt, e);
+                                  uploaded, want_xs, ctx->rf, tags ? &d_tags : nullptr, ctx->dev_rec, cnt, e);
     if (rc != BAMGPU_OK) cudaStreamSynchronize(ctx->stream);           // the pinned image may be re-used by the fallback / next call
     if (rc == BAMGPU_ERROR) return ctx->fail(SPL_ERR_CUDA, "%s", e.c_str());
     if (rc == BAMGPU_FALLBACK) { *fallback = true; return SPL_OK; }
@@ -1402,8 +1423,8 @@ int ingest_bam_device(spl_ctx* ctx, const char* path, int32_t n_chrom, const cha
 
 // The host reader under the context's read filter: the fallback of every ingest above
 std::string read_bam_ctx(spl_ctx* ctx, const char* path, int32_t n_chrom, const char* const* chrom_names, BamRecords& recs, bool want_xs = false,
-                         std::vector<std::string>* header_order = nullptr) {
-    std::string e = read_bam(path, n_chrom, chrom_names, ctx->n_threads, recs, want_xs, header_order, ctx->rf);
+                         std::vector<std::string>* header_order = nullptr, const TagTableView* tags = nullptr) {
+    std::string e = read_bam(path, n_chrom, chrom_names, ctx->n_threads, recs, want_xs, header_order, ctx->rf, tags);
     if (e.empty()) { ctx->rf_counts[0] = (int64_t)recs.pos.size(); ctx->rf_counts[1] = recs.n_filtered; }
     return e;
 }
@@ -1497,6 +1518,7 @@ void spl_destroy(spl_ctx* ctx) {
         if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
         if (ctx->h_file) cudaFreeHost(ctx->h_file);
         ctx->bgm.comp.release(); ctx->bgm.unc.release(); ctx->bgm.tab.release(); ctx->bgm.rec.release(); ctx->bgm.list.release();
+        ctx->bgm.tags.release(); ctx->gsm.release();
         ctx->gbm.fin.release(); ctx->gbm.fin2.release(); ctx->gbm.work.release(); ctx->gbm.work2.release();
         ctx->jem.release();
         if (ctx->stream2) { cudaStreamSynchronize(ctx->stream2); cudaStreamDestroy(ctx->stream2); }
@@ -2031,11 +2053,30 @@ int spl_recount(spl_ctx* ctx, const char* bam_path, int32_t n_chrom, const char*
 }
 
 // ---- device-resident samples ----------------------------------------------------------------------------------------------
+namespace {
+std::atomic<int64_t> g_resident_bytes(0);          // what the samples of this process hold (SPLISER_SAMPLE_BUDGET_MB caps it)
+
+// One device allocation of resident samples: a sample of spl_sample_load_bam owns one, the group samples of one
+// spl_sample_load_bam_groups share one.  The last owner frees it and returns its bytes to the residency count.
+struct SampleBlock {
+    void* p = nullptr;
+    size_t bytes = 0;
+    int device = 0;
+    SampleBlock(void* p_, size_t b, int d) : p(p_), bytes(b), device(d) {}
+    ~SampleBlock() {
+        if (!p) return;
+        cudaSetDevice(device);
+        cudaFree(p);
+        g_resident_bytes -= (int64_t)bytes;
+    }
+};
+}  // namespace
+
 struct spl_sample {
     const spl_ctx* ctx = nullptr;         // the context that loaded it (compared, never dereferenced)
     int device = 0;
-    void* mem = nullptr;                  // the one device allocation that holds every column
-    size_t bytes = 0;
+    std::shared_ptr<SampleBlock> mem;     // the device allocation that holds every column (shared by the samples of one split)
+    size_t bytes = 0;                     // the sample's own slice of it
     DevRecordArrays rec{};                // pos / flag / cig_off / cigar (/ xs) inside mem; no per-record chromosome
     int64_t n_rec = 0, n_cigar = 0;
     std::vector<std::string> ref_names;   // the header's references, in header order
@@ -2045,7 +2086,6 @@ struct spl_sample {
 };
 
 namespace {
-std::atomic<int64_t> g_resident_bytes(0);          // what the samples of this process hold (SPLISER_SAMPLE_BUDGET_MB caps it)
 constexpr size_t SAMPLE_HEADROOM = (size_t)1 << 30;
 
 // Takes `bytes` of device memory for a sample under the residency policy of spl_sample_load_bam; SPL_ERR_NOMEM holds nothing.
@@ -2142,10 +2182,12 @@ int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_
     Carver c;
     const size_t o_pos = c.take<int32_t>(n + 4), o_flag = c.take<uint16_t>(n + 4), o_off = c.take<uint32_t>(n + 4),
                  o_cig = c.take<uint32_t>(nc + 4), o_xs = want_xs ? c.take<uint8_t>(n + 4) : 0;
-    rc = sample_reserve(ctx, c.off, &s->mem);
+    void* mp = nullptr;
+    rc = sample_reserve(ctx, c.off, &mp);
     if (rc) return rc;
+    s->mem = std::make_shared<SampleBlock>(mp, c.off, ctx->device);
     s->bytes = c.off;
-    char* m = (char*)s->mem;
+    char* m = (char*)mp;
     s->rec.pos = (int32_t*)(m + o_pos); s->rec.flag = (uint16_t*)(m + o_flag);
     s->rec.cig_off = (uint32_t*)(m + o_off); s->rec.cigar = (uint32_t*)(m + o_cig);
     s->rec.xs = want_xs ? (uint8_t*)(m + o_xs) : nullptr;
@@ -2178,6 +2220,164 @@ int spl_sample_load_bam(spl_ctx* ctx, const char* bam_path, uint32_t flags, spl_
     ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
     *out = s.release();
     return SPL_OK;
+}
+
+int spl_sample_load_bam_groups(spl_ctx* ctx, const char* bam_path, uint32_t flags, const spl_tag_groups* groups, spl_sample** out,
+                               int64_t* counts) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out || !counts) return ctx->fail(SPL_ERR_ARG, "out / counts is NULL");
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!bam_path) return ctx->fail(SPL_ERR_ARG, "bam_path is NULL");
+    if (flags & ~SPL_FLAG_XS_STRAND) return ctx->fail(SPL_ERR_ARG, "spl_sample_load_bam_groups takes SPL_FLAG_XS_STRAND only");
+    TagTableHost tags;
+    {
+        const std::string e = build_tag_table(groups, tags);
+        if (!e.empty()) return ctx->fail(SPL_ERR_ARG, "tag group table: %s", e.c_str());
+    }
+    const uint32_t G = (uint32_t)tags.n_groups;
+    for (uint32_t g = 0; g < G; ++g) out[g] = nullptr;
+    const bool want_xs = (flags & SPL_FLAG_XS_STRAND) != 0;
+    const double t0 = now_ms();
+    CU(cudaSetDevice(ctx->device));
+    reset_stats(ctx);
+    struct ReleaseScratch {                                            // on every return: cudaFree waits for the stream's work
+        GroupSplitMem& m;
+        ~ReleaseScratch() { m.release(); }
+    } release_scratch{ctx->gsm};
+    // ---- one ingest, every reference kept in header order, the group of every record found as it is parsed
+    std::vector<std::string> ref_names;
+    BamGpuCounts cnt;
+    spl_records_view dv{};
+    bool fallback = false;
+    int rc = ingest_bam_device(ctx, bam_path, 0, nullptr, cnt, dv, &fallback, want_xs, &ref_names, &tags);
+    if (rc) return rc;
+    DevRecordArrays in{};
+    const int32_t* grp = cnt.grp;
+    uint64_t n = 0;
+    double h2d = cnt.h2d_bytes;
+    if (!fallback) {
+        in = ctx->dev_rec;
+        n = cnt.n_rec;
+    } else {                                                           // the host reader's records and groups, uploaded once
+        BamRecords recs;
+        const TagTableView tv = tags.view();
+        std::string e = read_bam_ctx(ctx, bam_path, 0, nullptr, recs, want_xs, &ref_names, &tv);
+        if (!e.empty()) return ctx->fail(SPL_ERR_IO, "%s", e.c_str());
+        n = recs.pos.size();
+        const size_t nc = recs.cigar.size();
+        std::vector<int32_t> chrom(n);
+        for (size_t k = 0; k + 1 < recs.seg_off.size(); ++k)
+            std::fill(chrom.begin() + recs.seg_off[k], chrom.begin() + recs.seg_off[k + 1], recs.seg_chrom[k]);
+        Carver c;
+        const size_t o_pos = c.take<int32_t>(n + 4), o_flag = c.take<uint16_t>(n + 4), o_off = c.take<uint32_t>(n + 4),
+                     o_cig = c.take<uint32_t>(nc + 4), o_chr = c.take<int32_t>(n + 4), o_grp = c.take<int32_t>(n + 4),
+                     o_xs = want_xs ? c.take<uint8_t>(n + 4) : 0;
+        if (ctx->gsm.in.reserve(c.off + 256) != cudaSuccess) {
+            cudaGetLastError();
+            return ctx->fail(SPL_ERR_NOMEM, "the split of %s is not held: no device memory for the records (%zu bytes); use more GPUs", bam_path, c.off);
+        }
+        char* b = (char*)ctx->gsm.in.p;
+        in.pos = (int32_t*)(b + o_pos); in.flag = (uint16_t*)(b + o_flag); in.cig_off = (uint32_t*)(b + o_off);
+        in.cigar = (uint32_t*)(b + o_cig); in.chrom = (int32_t*)(b + o_chr);
+        int32_t* d_grp = (int32_t*)(b + o_grp);
+        grp = d_grp;
+        in.xs = want_xs ? (uint8_t*)(b + o_xs) : nullptr;
+        if (n) {
+            CU(cudaMemcpyAsync(in.pos, recs.pos.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaMemcpyAsync(in.flag, recs.flag.data(), n * 2, cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaMemcpyAsync(in.cigar, recs.cigar.data(), nc * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaMemcpyAsync(in.chrom, chrom.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CU(cudaMemcpyAsync(d_grp, recs.grp.data(), n * 4, cudaMemcpyHostToDevice, ctx->stream));
+            if (want_xs) CU(cudaMemcpyAsync(in.xs, recs.xs.data(), n, cudaMemcpyHostToDevice, ctx->stream));
+        }
+        CU(cudaMemcpyAsync(in.cig_off, recs.cig_off.data(), (n + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));                         // recs is freed at the end of this scope
+        h2d = (double)(n * 18 + 4 + nc * 4 + (want_xs ? n : 0));
+    }
+    const double t1 = now_ms();
+    // ---- stable sort by group, then one allocation with every group's columns in a slice of its own
+    GroupSort gs;
+    std::string e;
+    rc = group_sort(ctx->gsm, in, grp, n, (int32_t)G, ctx->stream, gs, e);
+    if (rc < 0) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_CUDA, "%s", e.c_str()); }
+    if (rc > 0) { cudaStreamSynchronize(ctx->stream); return ctx->fail(SPL_ERR_NOMEM, "the split of %s is not held: %s; use more GPUs", bam_path, e.c_str()); }
+    std::vector<GroupCols> cols(G);
+    std::vector<size_t> slice0(G + 1);
+    Carver c;
+    for (uint32_t g = 0; g < G; ++g) {
+        const size_t ng = (size_t)gs.n_rec[g], ncg = (size_t)gs.n_cig[g];
+        c.off = (c.off + 255) & ~(size_t)255;
+        slice0[g] = c.off;
+        GroupCols& q = cols[g];
+        q.pos = c.take<int32_t>(ng + 4); q.flag = c.take<uint16_t>(ng + 4); q.off = c.take<uint32_t>(ng + 4);
+        q.cig = c.take<uint32_t>(ncg + 4); q.xs = want_xs ? c.take<uint8_t>(ng + 4) : 0;
+        q.start = gs.g_start[g]; q.cig0 = gs.g_cig[g]; q.n = (uint32_t)ng; q.nc = (uint32_t)ncg;
+    }
+    c.off = (c.off + 255) & ~(size_t)255;
+    slice0[G] = c.off;
+    void* mp = nullptr;
+    rc = sample_reserve(ctx, c.off, &mp);
+    if (rc == SPL_ERR_NOMEM) {
+        const std::string why = spl_last_error(ctx);
+        return ctx->fail(SPL_ERR_NOMEM, "the split of %s needs %zu bytes of device memory for the kept records of its groups, which are "
+                         "not held (%s); use more GPUs (--gpus) so that each holds fewer groups", bam_path, c.off, why.c_str());
+    }
+    if (rc) return rc;
+    auto block = std::make_shared<SampleBlock>(mp, c.off, ctx->device);
+    rc = group_gather(ctx->gsm, in, gs, cols, (char*)mp, ctx->stream, e);
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);
+    if (rc || ce != cudaSuccess) {
+        cudaGetLastError();
+        return ctx->fail(SPL_ERR_CUDA, "the split of %s failed: %s", bam_path, rc ? e.c_str() : cudaGetErrorString(ce));
+    }
+    std::vector<std::unique_ptr<spl_sample>> made(G);
+    for (uint32_t g = 0; g < G; ++g) {
+        made[g].reset(new (std::nothrow) spl_sample());
+        if (!made[g]) return ctx->fail(SPL_ERR_NOMEM, "out of memory");
+        spl_sample& s = *made[g];
+        char* m = (char*)mp;
+        s.ctx = ctx; s.device = ctx->device; s.rf = ctx->rf;
+        s.mem = block; s.bytes = slice0[g + 1] - slice0[g];
+        s.rec.pos = (int32_t*)(m + cols[g].pos); s.rec.flag = (uint16_t*)(m + cols[g].flag);
+        s.rec.cig_off = (uint32_t*)(m + cols[g].off); s.rec.cigar = (uint32_t*)(m + cols[g].cig);
+        s.rec.xs = want_xs ? (uint8_t*)(m + cols[g].xs) : nullptr;
+        s.n_rec = gs.n_rec[g]; s.n_cigar = gs.n_cig[g];
+        s.ref_names = ref_names;
+        s.seg_ref = gs.seg_chrom[g]; s.seg_off = gs.seg_off[g];
+    }
+    for (uint32_t g = 0; g < G; ++g) { counts[g] = gs.n_rec[g]; out[g] = made[g].release(); }
+    counts[G] = (int64_t)gs.no_value; counts[G + 1] = (int64_t)gs.no_group;
+    ctx->stats[SPL_STAT_H2D_BYTES] = h2d;
+    ctx->stats[SPL_STAT_BAM_DEVICE] = fallback ? 0.0 : 1.0;
+    ctx->stats[SPL_STAT_MS_DECODE] = t1 - t0;
+    ctx->stats[SPL_STAT_MS_TOTAL] = now_ms() - t0;
+    return SPL_OK;
+}
+
+int spl_sample_fetch_records(spl_ctx* ctx, const spl_sample* s, spl_records** out) {
+    if (!ctx) return SPL_ERR_ARG;
+    if (!out) return ctx->fail(SPL_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx->stream) return ctx->fail(SPL_ERR_CUDA, "context has no CUDA device; libspliser_b200 has no CPU fallback");
+    if (!s) return ctx->fail(SPL_ERR_ARG, "sample is NULL");
+    if (s->ctx != ctx) return ctx->fail(SPL_ERR_ARG, "the sample was loaded by another context");
+    CU(cudaSetDevice(ctx->device));
+    const size_t n = (size_t)s->n_rec, nc = (size_t)s->n_cigar;
+    BamRecords r;
+    r.pos.resize(n); r.flag.resize(n); r.cig_off.resize(n + 1); r.cigar.resize(nc);
+    if (s->rec.xs) r.xs.resize(n);
+    if (n) {
+        CU(cudaMemcpyAsync(r.pos.data(), s->rec.pos, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(r.flag.data(), s->rec.flag, n * 2, cudaMemcpyDeviceToHost, ctx->stream));
+        if (s->rec.xs) CU(cudaMemcpyAsync(r.xs.data(), s->rec.xs, n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    if (nc) CU(cudaMemcpyAsync(r.cigar.data(), s->rec.cigar, nc * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaMemcpyAsync(r.cig_off.data(), s->rec.cig_off, (n + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    r.seg_chrom = s->seg_ref; r.seg_off = s->seg_off;
+    const bool xs = s->rec.xs != nullptr;
+    *out = records_handle(std::move(r), xs);
+    return *out ? SPL_OK : ctx->fail(SPL_ERR_NOMEM, "out of memory");
 }
 
 int spl_sample_process_extract(spl_ctx* ctx, const spl_sample* s, int32_t n_chrom, const char* const* chrom_names,
@@ -2352,13 +2552,7 @@ int64_t spl_sample_n_records(const spl_sample* s) { return s ? s->n_rec : 0; }
 int64_t spl_sample_device_bytes(const spl_sample* s) { return s ? (int64_t)s->bytes : 0; }
 
 void spl_sample_free(spl_sample* s) {
-    if (!s) return;
-    if (s->mem) {
-        cudaSetDevice(s->device);
-        cudaFree(s->mem);
-        g_resident_bytes -= (int64_t)s->bytes;
-    }
-    delete s;
+    delete s;                             // the last sample of an allocation frees it (SampleBlock)
 }
 
 int spl_resident_load(spl_ctx* ctx, const spl_records_view* rec, int32_t n_chrom, int64_t n_junc, const int32_t* j_chrom,
